@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — hybrid filtered top-k queries/sec on B200 (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg4] [--impl b200|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload cfg4] [--impl b200|reference] [--dump-outputs DIR]
 
 Default workload: BASELINE.json configs[3] in its weak form — 12.5M x 768-d rows PER GPU (N = 8 is the
 100M-row corpus), scope + time filter at 50 %, batch 1024 for the whole job, top-100.  At N = 1 it is the
@@ -24,6 +24,8 @@ the K timed steps last >= 0.5 s and the clock sampler sees them).
           (a row slice and a few queries of one batch), extrapolated linearly in rows, stated in `sample`.
 Multi-GPU (torchrun, one rank per GPU): rows are sharded over the ranks, candidates are exchanged by one
 NCCL all-gather per batch.  `--impl reference` times the CPU port alone (rank 0), same config/metric.
+--dump-outputs DIR writes what the timed path returned in its last step (see dump_outputs) so that two builds
+can be compared output for output; the inputs depend only on the arguments.
 """
 from __future__ import annotations
 
@@ -81,6 +83,7 @@ WORKLOADS = {
 BLOCK_ROWS = 125_000        # corpus generation granule: shard boundaries at 1/2/4/8 GPUs coincide with it
 N_QUERY_BATCHES = 8
 L2_BYTES = 126 << 20
+DUMP_BYTES = 64 << 20       # --dump-outputs: at most this much in all
 
 
 def peaks():
@@ -377,7 +380,20 @@ def run_api(ix, cfg, batches, flt, n_threads, n_calls, device, torch):
     return res
 
 
+def dump_outputs(out_dir, results):
+    """What the batches of one step returned to their caller, one row per query in stream order, as float64:
+    rows.npy [Q, limit] (row ids, exact below 2^53), scores.npy [Q, limit], counts.npy [Q].  Slots past a list's
+    count are zero.  The largest workload (cfg5: 4096 queries, top-20) writes about 1.3 MB."""
+    out = {k: np.concatenate([getattr(r, k) for r in results]).astype(np.float64) for k in ("rows", "scores", "counts")}
+    assert sum(v.nbytes for v in out.values()) <= DUMP_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v)
+    return sorted(out)
+
+
 def main():
+    sys.dont_write_bytecode = True      # the bench runs from the source tree (possibly read-only) and leaves nothing in it
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=20)
@@ -390,7 +406,13 @@ def main():
     ap.add_argument("--clock-period-ms", type=int, default=50, help="nvidia-smi sampling period during the timed region")
     ap.add_argument("--no-api", action="store_true", help="skip the e2e_api (VectorStoreService.search) section")
     ap.add_argument("--api-threads", type=int, default=16)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the results of the B200 path (--impl b200)")
     cfg = dict(WORKLOADS[args.workload])
     if "rows_per_gpu" in cfg:
         cfg["n"] = cfg["rows_per_gpu"] * max(1, args.gpus)
@@ -478,16 +500,18 @@ def main():
             dist.barrier()
         torch.cuda.synchronize(device)
 
-    def device_step(step_index):
+    def device_step(step_index, results=None):
         total, launches = 0.0, 0
         for k in range(bps):
             st = stage(step_index * bps + k)            # host staging + H2D: outside the timed events
             if world > 1:                               # ranks enter the batch together: otherwise the all-gather of the
                 torch.cuda.synchronize(device)          # faster rank waits for the other's host staging inside the events
                 dist.barrier()
-            ms_, _ = device_batch(st)
+            ms_, res_ = device_batch(st)
             total += ms_
             launches += ix.stats()["last_launches"]
+            if results is not None:
+                results.append(res_)
         return total, launches
 
     # ---- device-resident timing ("value") ----------------------------------------------------------
@@ -499,8 +523,9 @@ def main():
     t_begin = time.perf_counter()
     ms = np.zeros(args.steps)
     launches = 0
+    last_step = []
     for i in range(args.steps):
-        ms[i], l_ = device_step(args.warmup + i)
+        ms[i], l_ = device_step(args.warmup + i, last_step if i == args.steps - 1 else None)
         launches += l_
     barrier()
     t_end = time.perf_counter()
@@ -509,6 +534,10 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = t.cpu().numpy()
     clocks = sampler.stop(t_begin, t_end)
+    if args.dump_outputs and rank == 0:
+        names = dump_outputs(args.dump_outputs, last_step)
+        print(f"bench.py: last timed step ({len(last_step)} batch(es)) -> {args.dump_outputs}/{{{','.join(names)}}}.npy",
+              file=sys.stderr)
     total_ms = float(ms.sum())
     value = qps * args.steps / (total_ms / 1e3)
     dense_path = ix.stats()["last_dense_path"]

@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Generate tests/golden/voitta_cases.json by running the REFERENCE's own
-``voitta/services/vector_store.py`` (imported from /root/reference, unmodified) in the
-build container.
+``voitta/services/vector_store.py`` (unmodified, from the voitta-rag checkout that
+$VOITTA_REFERENCE_SRC names).
 
 ``qdrant_client`` is not installable here (no network), so it is replaced by a stub whose
 ``QdrantClient`` delegates to ``oracle.oracle.LocalCollection`` (the restatement of
@@ -12,13 +12,14 @@ reference wrote it: point construction (:233-317), ``_build_filter`` (:462-530),
 ``oracle.OracleVectorStore`` (tests/test_oracle_golden.py) and are replayed against the
 B200 backend (tests/test_gpu_golden.py).
 
-Run from the repo root:  python tests/golden/make_golden.py
-/root/reference is NOT needed at test time; only this script reads it.
+Run from the repo root:  VOITTA_REFERENCE_SRC=<voitta-rag>/src/voitta python tests/golden/make_golden.py
+The reference source is NOT needed at test time; only this script reads it.
 """
 from __future__ import annotations
 
 import importlib.util
 import json
+import os
 import sys
 import types
 import uuid
@@ -33,7 +34,6 @@ sys.path.insert(0, str(ROOT / "tests"))
 from oracle import oracle as O  # noqa: E402
 import _data  # noqa: E402
 
-REF = Path("/root/reference/src/voitta")
 DIM = 32
 N = 600
 
@@ -144,6 +144,12 @@ def real_qdrant_available() -> bool:
         return False
 
 
+def reference_src() -> Path | None:
+    """voitta-rag's ``src/voitta`` directory, named by $VOITTA_REFERENCE_SRC; None if unset or not a checkout."""
+    p = os.environ.get("VOITTA_REFERENCE_SRC")
+    return Path(p) if p and (Path(p) / "services" / "vector_store.py").is_file() else None
+
+
 def _install_real():
     """Route the reference's QdrantClient(host, port) to qdrant-client's local in-memory mode."""
     import qdrant_client
@@ -156,9 +162,12 @@ def _install_real():
 
 
 def load_reference_vector_store(dim: int, real: bool = False):
-    """Import /root/reference/src/voitta/services/vector_store.py without running the
+    """Import the reference's services/vector_store.py (``reference_src()``) without running the
     package __init__ files (they import sqlalchemy/fastmcp/... which are absent).  ``real``: over the real
     qdrant-client (local mode) instead of the stub that delegates to the oracle."""
+    REF = reference_src()
+    if REF is None:
+        raise RuntimeError("set VOITTA_REFERENCE_SRC to voitta-rag's src/voitta directory")
     if real:
         _install_real()
     else:
@@ -382,7 +391,7 @@ def main():
     out_dir = Path(__file__).resolve().parent
     with open(out_dir / "voitta_cases.json", "w") as f:
         json.dump({"generated_by": "tests/golden/make_golden.py",
-                   "reference": "voitta/services/vector_store.py (unmodified, /root/reference) over "
+                   "reference": "voitta/services/vector_store.py (unmodified) over "
                                 "oracle.LocalCollection standing in for qdrant-client",
                    "dim": DIM, "n": N, "ops": ops, "outs": outs}, f, indent=0)
     n_search = sum(1 for o in ops if o["op"] == "search")

@@ -48,12 +48,12 @@ def test_oracle_matches_reference_outputs(replayed):
 
 
 def test_real_qdrant_client_agrees_when_installed():
-    """The day qdrant-client is importable (a driver-provided baseline/_ref, or the package in the image) the golden
-    scenario is replayed through the reference over the REAL client and must match the committed outputs — that flips
-    the oracle's qdrant half from "parity unpinned" to pinned.  Not installed in this image: skipped, and said so."""
+    """Where qdrant-client is importable (installed, or under baseline/_ref) and $VOITTA_REFERENCE_SRC names voitta-rag's
+    src/voitta, the golden scenario is replayed through the reference over the REAL client and must match the committed
+    outputs — that pins the oracle's qdrant half.  Neither ships with this repository: without them, skipped, and said so."""
     import pytest
     from golden import make_golden as G
-    if not G.real_qdrant_available():
-        pytest.skip("qdrant-client is not installed (no network): the qdrant half of the oracle stays pinned only by the "
-                    "hand-derived vectors in tests/golden/known_answers.json")
+    if not G.real_qdrant_available() or G.reference_src() is None:
+        pytest.skip("needs qdrant-client and voitta-rag's source ($VOITTA_REFERENCE_SRC): the qdrant half of the oracle stays "
+                    "pinned only by the hand-derived vectors in tests/golden/known_answers.json")
     assert G.check_against_real_qdrant() > 40
