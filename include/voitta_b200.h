@@ -71,8 +71,10 @@ typedef struct vb_query_batch {
     const uint32_t* sp_term;      /* host [nnz] hashed term ids (sparse_embedding.py:29-39)   */
     const double*   sp_weight;    /* host [nnz] query values (IDF applied iff !apply_idf)     */
     int32_t         apply_idf;    /* 1: multiply by ln(1+(N-df+.5)/(df+.5)) using this index  */
-    uint32_t        n_filters;    /* distinct filters in the batch                            */
-    const vb_filter* filters;     /* host [n_filters]                                         */
+    uint32_t        n_filters;    /* filters passed, any number; one per query is fine        */
+    const vb_filter* filters;     /* host [n_filters]; ones no query uses are ignored, ones of
+                                     equal content (same ts_field, same range if it has one,
+                                     same scope words up to trailing zeros) are merged          */
     const int32_t*  filter_of;    /* host [B] index into filters, -1 = unfiltered; NULL = all -1 */
     uint32_t        limit;        /* results per query                                        */
     uint32_t        kprime;       /* per-branch over-fetch, voitta: 3*limit (vector_store.py:636) */

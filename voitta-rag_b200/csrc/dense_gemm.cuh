@@ -27,7 +27,27 @@
 #define VB_TILE_M 128u
 #define VB_BLOCK_K 64u
 #define VB_STAGE_BYTES (VB_TILE_M * VB_BLOCK_K * 2u)   // 16 KB
-#define VB_GEMM_MAX_FILTERS 256u
+#define VB_GEMM_MAX_FILTERS 256u       // mask words the epilogue caches per warp: one per filter of a query tile (<= 256 queries)
+
+// Mask mode 3 (more than 31 distinct filters in the batch): the filters each query tile uses, so that the epilogue's
+// per-warp mask-word cache is indexed by a tile-local id.  A tile holds at most 256 queries, hence at most 256 filters,
+// whatever the batch holds in all.  Built on the host with the batch (vb_api.cu prepare_batch), one set per tile size.
+// When all tiles of one launch use at most 256 filters between them, they share one list (n[t] carries
+// VB_FTAB_SHARED): K2T then loads the mask words once per corpus tile instead of once per (corpus tile, query tile).
+#define VB_FTAB_SHARED 0x80000000u
+struct VbFilterTiles {
+    const int32_t* loc = nullptr;    // [B] index of the query's filter in its tile's list, -1 = unfiltered
+    const uint32_t* n = nullptr;     // [tiles] filters listed per tile (| VB_FTAB_SHARED: the launch's tiles share the list)
+    const int32_t* ids = nullptr;    // [tiles][VB_GEMM_MAX_FILTERS] batch-wide filter id of each listed filter
+    uint32_t tile = 0;               // queries per tile (0: no tables)
+};
+
+// mode 3: this warp's mask word (32 rows) of every listed filter, lane l loading entries l, l + 32, ...
+__device__ __forceinline__ void vb_cache_mask_words(uint32_t* mw, const uint32_t* mask, const int32_t* tab, uint32_t nf,
+                                                    uint32_t mask_words, uint32_t word, uint32_t lane) {
+    for (uint32_t l = lane; l < nf; l += 32u)
+        mw[l] = word < mask_words ? mask[(size_t)tab[l] * mask_words + word] : 0u;
+}
 
 static std::string g_gemm_err;
 static const char* vb_gemm_last_error() { return g_gemm_err.c_str(); }
@@ -128,7 +148,9 @@ __device__ __forceinline__ float vb_pre_threshold(float tau, float qs) {
 struct VbGemmArgs {
     const float* inv_norm;
     const uint32_t* mask;      // [n_filters][mask_words] or nullptr
-    const int32_t* mask_of;    // [B_total] or nullptr
+    const int32_t* mask_of;    // [B_total] or nullptr; mask_mode 3: the tile-local ids (VbFilterTiles::loc)
+    const uint32_t* ftab_n;    // mask_mode 3: [1] filters listed for this sub-batch
+    const int32_t* ftab;       // mask_mode 3: [ftab_n[0]] their batch-wide ids
     const float* tau;          // [n_lists]
     const float* q_scale;      // [B_total] 1/|bf16(q)| (1 for the bf16x2 query)
     VbLists lists;
@@ -201,6 +223,7 @@ vb_dense_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_co
         qs_s[c] = qs;
         tau_s[c] = SPLIT ? t : vb_pre_threshold(t, qs);        // bf16x2 query: no scale, the hot compare is exact
         mof_s[c] = (live && a.mask_of) ? a.mask_of[a.q_begin + c] : -1;
+        VB_CHECK(MODE != 3 || mof_s[c] < (int32_t)(a.ftab_n[0] & ~VB_FTAB_SHARED));
     }
     vb_tcgen05_fence_before();
     __syncthreads();
@@ -212,6 +235,7 @@ vb_dense_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_co
     const uint32_t tile_begin = cmp ? 0u : a.tile_begin;
     const uint32_t row_end = cmp ? a.sel[0] : a.row_end;
     const uint32_t n_tiles = cmp ? (a.sel[0] + VB_TILE_M - 1u) / VB_TILE_M : a.tile_end - a.tile_begin;
+    const uint32_t n_tab = MODE == 3 ? a.ftab_n[0] & ~VB_FTAB_SHARED : 0u;
 
     if (warp == 0) {
         // ===== TMA producer =====
@@ -301,8 +325,7 @@ vb_dense_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_co
                     fbits |= ((__shfl_sync(0xffffffffu, w, f) >> lane) & 1u) << f;
             } else if (mode == 3u) {
                 __syncwarp();
-                for (uint32_t f = lane; f < a.n_filters; f += 32u)
-                    mw[f] = word < a.mask_words ? a.mask[(size_t)f * a.mask_words + word] : 0u;
+                vb_cache_mask_words(mw, a.mask, a.ftab, n_tab, a.mask_words, word, lane);
                 __syncwarp();
             }
             vb_mbar_wait(bar_tfull + 8u * acc, (it >> 1) & 1u);
@@ -411,7 +434,9 @@ vb_dense_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_co
 struct VbGemmTiledArgs {
     const float* inv_norm;
     const uint32_t* mask;      // [n_filters][mask_words] or nullptr
-    const int32_t* mask_of;    // [B_total] or nullptr
+    const int32_t* mask_of;    // [B_total] or nullptr; mask_mode 3: the tile-local ids (VbFilterTiles::loc)
+    const uint32_t* ftab_n;    // mask_mode 3: [query tiles of this launch] filters listed per tile
+    const int32_t* ftab;       // mask_mode 3: [query tiles of this launch][VB_GEMM_MAX_FILTERS] their batch-wide ids
     const float* tau;          // [n_lists]
     const float* q_scale;      // [B_total] 1/|bf16(q)|
     VbLists lists;
@@ -472,6 +497,7 @@ vb_dense_gemm_tiled_kernel(const __grid_constant__ CUtensorMap tmap_a, const __g
         qs_s[c] = qs;
         tau_s[c] = vb_pre_threshold(t, qs);
         mof_s[c] = (live && a.mask_of) ? a.mask_of[a.q_begin + c] : -1;
+        VB_CHECK(MODE != 3 || !live || mof_s[c] < (int32_t)(a.ftab_n[c / VB_TILE_N] & ~VB_FTAB_SHARED));
     }
     vb_tcgen05_fence_before();
     __syncthreads();
@@ -484,6 +510,7 @@ vb_dense_gemm_tiled_kernel(const __grid_constant__ CUtensorMap tmap_a, const __g
     const uint32_t row_end = cmp ? a.sel[0] : a.row_end;
     const uint32_t n_tiles = cmp ? (a.sel[0] + VB_TILE_M - 1u) / VB_TILE_M : a.tile_end - a.tile_begin;
     const uint32_t n_ntiles = (a.n_q + VB_TILE_N - 1u) / VB_TILE_N;
+    const bool tab_once = MODE == 3 && (a.ftab_n[0] & VB_FTAB_SHARED) != 0u;    // one list for all query tiles
 
     if (warp == 0) {
         // ===== TMA producer: per (corpus tile, query tile, K block) one corpus box + one query box =====
@@ -564,16 +591,21 @@ vb_dense_gemm_tiled_kernel(const __grid_constant__ CUtensorMap tmap_a, const __g
                 const uint32_t w = (lane < a.n_filters && word < a.mask_words) ? a.mask[(size_t)lane * a.mask_words + word] : 0u;
                 for (uint32_t f = 0; f < a.n_filters; ++f)
                     fbits |= ((__shfl_sync(0xffffffffu, w, f) >> lane) & 1u) << f;
-            } else if (mode == 3u) {
+            } else if (mode == 3u && tab_once) {
                 __syncwarp();
-                for (uint32_t f = lane; f < a.n_filters; f += 32u)
-                    mw[f] = word < a.mask_words ? a.mask[(size_t)f * a.mask_words + word] : 0u;
+                vb_cache_mask_words(mw, a.mask, a.ftab, a.ftab_n[0] & ~VB_FTAB_SHARED, a.mask_words, word, lane);
                 __syncwarp();
             }
             for (uint32_t j = 0; j < n_ntiles; ++j, ++it) {
                 const uint32_t acc = it & 1u;
                 const uint32_t qoff = j * VB_TILE_N;
                 const uint32_t ncol = min(VB_TILE_N, (a.n_q - qoff + 15u) & ~15u);
+                if (mode == 3u && !tab_once) {
+                    // this query tile's own list (loads issued before blocking on the accumulator); the warp's previous
+                    // tile has been fully read from mw (the __syncwarp that ends it)
+                    vb_cache_mask_words(mw, a.mask, a.ftab + (size_t)j * VB_GEMM_MAX_FILTERS, a.ftab_n[j], a.mask_words, word, lane);
+                    __syncwarp();
+                }
                 vb_mbar_wait(bar_tfull + 8u * acc, (it >> 1) & 1u);
                 vb_tcgen05_fence_after();
                 const uint32_t taddr = tmem_base + ((quad * 32u) << 16) + acc * VB_TILE_N;
@@ -770,6 +802,7 @@ struct VbGemmLaunch {
     uint32_t direct;
     VbGemmPlan plan;
     const int32_t* mask_of_host;   // host copy of mask_of (to pick the epilogue's mask mode)
+    VbFilterTiles ftab;            // mask mode 3: filter tables for this launcher's query tiles (K2: plan.sub, K2T: VB_TILE_N)
     // K2T over the compacted copy of the rows passing the batch's shared filter (dense_compact.cuh); sel == nullptr: off
     const uint32_t* sel = nullptr;
     const uint32_t* sel_ids = nullptr;
@@ -807,8 +840,8 @@ static int vb_encode_a3d(CUtensorMap* map, const void* base, uint64_t rows, uint
 
 static int vb_gemm_launch(const VbGemmLaunch& g, int* launches) {
     if (!g_encode_tiled) { g_gemm_err = "tensor-core path not configured"; return 1; }
-    if (g.mask && g.n_filters > VB_GEMM_MAX_FILTERS) { g_gemm_err = "more than 256 distinct filters in one batch"; return 1; }
     const uint32_t sub = g.plan.sub, mult = g.plan.split ? 2u : 1u;
+    if (g.mask && g.n_filters > 31u && g.ftab.tile != sub) { g_gemm_err = "filter tables were built for another sub-batch size"; return 1; }
     const uint32_t k_blocks = g.d_pad / VB_BLOCK_K;
     const uint32_t kbox = vb_gemm_kbox(g.d_pad);
     (void)k_blocks;
@@ -836,6 +869,9 @@ static int vb_gemm_launch(const VbGemmLaunch& g, int* launches) {
             if (uniform && g.mask_of_host[q0] < 0) { a.mask = nullptr; a.mask_of = nullptr; }
             else if (uniform) { a.mask_mode = 1; a.uniform_filter = g.mask_of_host[q0]; }
             else a.mask_mode = g.n_filters <= 31u ? 2 : 3;
+            if (a.mask_mode == 3u) {                // sub-batch s is tile s of the tables
+                a.mask_of = g.ftab.loc; a.ftab_n = g.ftab.n + q0 / sub; a.ftab = g.ftab.ids + (size_t)(q0 / sub) * VB_GEMM_MAX_FILTERS;
+            }
         }
         const uint32_t q_bytes = bn * g.d_pad * 2u;
         a.kbox = kbox;
@@ -878,7 +914,7 @@ static bool vb_gemm_tiled_supported(int d_pad) {
 // g.q_bf16 must hold the queries unsplit, row i = query i (vb_gemm_plan with split = 0).
 static int vb_gemm_tiled_launch(const VbGemmLaunch& g, int* launches) {
     if (!g_encode_tiled) { g_gemm_err = "tensor-core path not configured"; return 1; }
-    if (g.mask && g.n_filters > VB_GEMM_MAX_FILTERS) { g_gemm_err = "more than 256 distinct filters in one batch"; return 1; }
+    if (g.mask && g.n_filters > 31u && g.ftab.tile != VB_TILE_N) { g_gemm_err = "filter tables were built for another query tile"; return 1; }
     if (g.plan.split) { g_gemm_err = "tiled kernel needs the unsplit query layout"; return 1; }
     CUtensorMap tmap_a;
     if (vb_encode_2d(&tmap_a, g.rows, g.n_rows_total, g.d_pad, VB_TILE_M)) return 1;
@@ -903,6 +939,9 @@ static int vb_gemm_tiled_launch(const VbGemmLaunch& g, int* launches) {
             if (uniform && g.mask_of_host[q0] < 0) { a.mask = nullptr; a.mask_of = nullptr; }
             else if (uniform) { a.mask_mode = 1; a.uniform_filter = g.mask_of_host[q0]; }
             else a.mask_mode = g.n_filters <= 31u ? 2 : 3;
+            if (a.mask_mode == 3u) {                // q0 is a multiple of VB_TILED_MAX_Q: this launch holds tiles q0 / VB_TILE_N ...
+                a.mask_of = g.ftab.loc; a.ftab_n = g.ftab.n + q0 / VB_TILE_N; a.ftab = g.ftab.ids + (size_t)(q0 / VB_TILE_N) * VB_GEMM_MAX_FILTERS;
+            }
         }
         const bool use_sel = g.sel != nullptr && a.mask_mode == 1u && !g.direct;
         const size_t smem = 1024u + (size_t)stages * VB_TILED_STAGE_BYTES + VB_TILED_TAIL_BYTES;

@@ -113,6 +113,7 @@ struct Batch {
     uint32_t base_rows = 0;                    // rows covered by the inverted index when the batch was staged
     uint64_t ms_max_post = 0;                  // most postings any K3M query's terms hold (how many stages a search needs)
     const int32_t* d_maskof = nullptr;
+    VbFilterTiles ft_k2, ft_k2t;               // mask mode 3 (> 31 filters): filter tables per K2 sub-batch / per K2T query tile
     const int32_t* d_mode = nullptr;
     const VbFilterDev* d_filters = nullptr;
     uint32_t need_created = 0, need_modified = 0, need_scope = 0;
@@ -1021,6 +1022,77 @@ static int validate_batch(const vb_index* h, const vb_query_batch* q) {
     return 0;
 }
 
+// Filter content as the mask kernel sees it: scope words past scope_words read as 0, the range only counts with a field.
+struct FilterKey {
+    const vb_filter* f;
+    uint32_t words;            // scope words up to the last non-zero one
+};
+struct FilterKeyHash {
+    size_t operator()(const FilterKey& k) const {
+        uint64_t x = 0x9E3779B97F4A7C15ull ^ (uint64_t)(k.f->scope_bits != nullptr) ^ ((uint64_t)(uint32_t)k.f->ts_field << 1);
+        auto mix = [&](uint64_t v) { x = (x ^ v) * 0xBF58476D1CE4E5B9ull; x ^= x >> 31; };
+        if (k.f->ts_field != VB_TS_NONE) { mix((uint64_t)k.f->ts_lo); mix((uint64_t)k.f->ts_hi); }
+        for (uint32_t w = 0; w < k.words; ++w) mix(k.f->scope_bits[w]);
+        return (size_t)x;
+    }
+};
+struct FilterKeyEq {
+    bool operator()(const FilterKey& a, const FilterKey& b) const {
+        const vb_filter &x = *a.f, &y = *b.f;
+        if (x.ts_field != y.ts_field || (x.scope_bits == nullptr) != (y.scope_bits == nullptr) || a.words != b.words) return false;
+        if (x.ts_field != VB_TS_NONE && (x.ts_lo != y.ts_lo || x.ts_hi != y.ts_hi)) return false;
+        return a.words == 0 || memcmp(x.scope_bits, y.scope_bits, (size_t)a.words * 4) == 0;
+    }
+};
+static FilterKey filter_key(const vb_filter* f) {
+    uint32_t w = f->scope_bits ? f->scope_words : 0u;
+    while (w > 0 && f->scope_bits[w - 1] == 0u) --w;
+    return FilterKey{f, w};
+}
+
+// Mask mode 3 tables for query tiles of `tile` queries: the distinct filters each tile uses (<= tile <= 256) and each
+// query's index into its tile's list.  The tiles of one launch (`group` queries) share the launch's list when it holds
+// at most 256 filters (VB_FTAB_SHARED).  Laid out at `off` of the staged argument block (host hp, device dp).
+static size_t filter_tiles_bytes(uint32_t B, uint32_t tile) {
+    const size_t tiles = (B + tile - 1) / tile;
+    return (size_t)B * 4 + align_up(tiles * 4, 16) + tiles * VB_GEMM_MAX_FILTERS * 4;
+}
+static VbFilterTiles build_filter_tiles(const std::vector<int32_t>& mask_of, uint32_t n_filters, uint32_t tile, uint32_t group,
+                                        unsigned char* hp, const unsigned char* dp, size_t off) {
+    const uint32_t B = (uint32_t)mask_of.size(), tiles = (B + tile - 1) / tile;
+    int32_t* loc = reinterpret_cast<int32_t*>(hp + off);
+    uint32_t* cnt = reinterpret_cast<uint32_t*>(hp + off + (size_t)B * 4);
+    int32_t* ids = reinterpret_cast<int32_t*>(hp + off + (size_t)B * 4 + align_up((size_t)tiles * 4, 16));
+    std::vector<int32_t> local(n_filters, -1);                 // batch-wide id -> index in the current list
+    std::vector<int32_t> list;
+    // queries [q0, q1) on one list: tiles [t0, t1) get it (flag set: the tiles of a launch share it)
+    auto make_list = [&](uint32_t q0, uint32_t q1) {
+        list.clear();
+        for (uint32_t i = q0; i < q1; ++i) {
+            const int32_t f = mask_of[i];
+            if (f >= 0 && local[f] < 0) { local[f] = (int32_t)list.size(); list.push_back(f); }
+            loc[i] = f >= 0 ? local[f] : -1;
+        }
+        for (int32_t f : list) local[f] = -1;
+    };
+    for (uint32_t g0 = 0; g0 < B; g0 += group) {
+        const uint32_t g1 = std::min(B, g0 + group);
+        make_list(g0, g1);
+        const bool shared = list.size() <= VB_GEMM_MAX_FILTERS;
+        for (uint32_t t = g0 / tile; t < (g1 + tile - 1) / tile; ++t) {
+            if (!shared) make_list(t * tile, std::min(B, (t + 1) * tile));
+            std::copy(list.begin(), list.end(), ids + (size_t)t * VB_GEMM_MAX_FILTERS);
+            cnt[t] = (uint32_t)list.size() | (shared ? VB_FTAB_SHARED : 0u);
+        }
+    }
+    VbFilterTiles ft;
+    ft.loc = reinterpret_cast<const int32_t*>(dp + off);
+    ft.n = reinterpret_cast<const uint32_t*>(dp + off + (size_t)B * 4);
+    ft.ids = reinterpret_cast<const int32_t*>(dp + off + (size_t)B * 4 + align_up((size_t)tiles * 4, 16));
+    ft.tile = tile;
+    return ft;
+}
+
 // Upload the batch, evaluate the filters, initialise the candidate lists.
 static int prepare_batch(vb_index* h, const vb_query_batch* q, Batch& b, bool need_corpus) {
     b = Batch();
@@ -1119,26 +1191,38 @@ static int prepare_batch(vb_index* h, const vb_query_batch* q, Batch& b, bool ne
     }
     b.n_qterms = (uint32_t)weight.size();
 
-    // ---- filters ----
+    // ---- filters: the ones no query uses are dropped, the ones with equal content merged, so that every consumer
+    // (mask kernel, mask mode, row selection) sees distinct, used filters: at most B + 1 of them ----
     const bool tombstones = h->n_live < h->n_rows;
     std::vector<int32_t> mask_of(b.B, -1);
-    std::vector<vb_filter> flt(q->filters, q->filters + q->n_filters);
+    std::vector<vb_filter> flt;
+    std::vector<int32_t> merged_as(q->n_filters, -2);          // caller's filter -> index in flt (-1: no clause, -2: not seen)
+    std::unordered_map<FilterKey, int32_t, FilterKeyHash, FilterKeyEq> by_content;
+    const vb_filter alive_only{nullptr, 0, VB_TS_NONE, 0, 0};
+    auto merge = [&](const vb_filter* x) -> int32_t {
+        auto it = by_content.emplace(filter_key(x), (int32_t)flt.size());
+        if (it.second) flt.push_back(*x);
+        return it.first->second;
+    };
     bool any_filter = false;
     for (uint32_t i = 0; i < b.B; ++i) {
         int32_t f = q->filter_of ? q->filter_of[i] : -1;
         if (f >= 0) {
-            const vb_filter& x = flt[f];
-            if (x.scope_bits == nullptr && x.ts_field == VB_TS_NONE && !tombstones) f = -1;   // filter with no clause
+            if (merged_as[f] == -2) {
+                const vb_filter& x = q->filters[f];
+                merged_as[f] = (x.scope_bits == nullptr && x.ts_field == VB_TS_NONE && !tombstones) ? -1 : merge(&x);   // no clause
+            }
+            f = merged_as[f];
         }
         mask_of[i] = f;
         any_filter |= f >= 0;
     }
     if (tombstones) {   // unfiltered queries still need the alive bits
-        int32_t alive_only = -1;
+        int32_t alive_id = -1;
         for (uint32_t i = 0; i < b.B; ++i)
             if (mask_of[i] < 0) {
-                if (alive_only < 0) { alive_only = (int32_t)flt.size(); flt.push_back(vb_filter{nullptr, 0, VB_TS_NONE, 0, 0}); }
-                mask_of[i] = alive_only;
+                if (alive_id < 0) alive_id = merge(&alive_only);
+                mask_of[i] = alive_id;
             }
         any_filter = true;
     }
@@ -1192,6 +1276,11 @@ static int prepare_batch(vb_index* h, const vb_query_batch* q, Batch& b, bool ne
     std::vector<size_t> o_bits(b.n_filters, 0);
     for (uint32_t f = 0; f < b.n_filters; ++f)
         if (flt[f].scope_bits) o_bits[f] = ar.take((size_t)flt[f].scope_words * 4);
+    // mask mode 3 tables: K2T tiles of VB_TILE_N queries, resident-K2 sub-batches as vb_gemm_plan cuts them
+    const bool ftabs = b.n_filters > 31u && vb_gemm_supported(h->d_pad, b.B);
+    const uint32_t k2_sub = ftabs ? vb_gemm_plan((uint32_t)h->d_pad, b.B, (int)h->opt_k2_precision).sub : 0u;
+    const size_t o_ft2t = ftabs ? ar.take(filter_tiles_bytes(b.B, VB_TILE_N)) : 0;
+    const size_t o_ft2 = ftabs ? ar.take(filter_tiles_bytes(b.B, k2_sub)) : 0;
     TRY(host_reserve(h->h_args_s[h->cur], ar.off));
     TRY(dev_reserve(h, h->args, ar.off, false));
     unsigned char* hp = h->h_args_s[h->cur].as<unsigned char>();
@@ -1230,6 +1319,10 @@ static int prepare_batch(vb_index* h, const vb_query_batch* q, Batch& b, bool ne
     b.base_rows = (uint32_t)h->base_rows;
     b.gen = h->write_gen;
     memcpy(hp + o_mo, mask_of.data(), (size_t)b.B * 4);
+    if (ftabs) {
+        b.ft_k2t = build_filter_tiles(mask_of, b.n_filters, VB_TILE_N, VB_TILED_MAX_Q, hp, dp, o_ft2t);
+        b.ft_k2 = build_filter_tiles(mask_of, b.n_filters, k2_sub, k2_sub, hp, dp, o_ft2);
+    }
     memcpy(hp + o_md, b.mode.data(), (size_t)b.B * 4);
     VbFilterDev* hf = reinterpret_cast<VbFilterDev*>(hp + o_fl);
     for (uint32_t f = 0; f < b.n_filters; ++f) {
@@ -1451,7 +1544,12 @@ static int run_branches(vb_index* h, const Batch& b, bool safe, int phase = 0) {
     // K0 filter masks
     if (b.use_mask && phase != 2) {
         prof_begin(h, PH_MASK);
-        TRY(dev_reserve(h, h->mask, (size_t)b.n_filters * b.mask_words * 4, false));
+        const size_t mask_bytes = (size_t)b.n_filters * b.mask_words * 4;
+        if (dev_reserve(h, h->mask, mask_bytes, false) != 0) {
+            cudaGetLastError();
+            return vb_fail("filter masks of %u distinct filters over %u rows need %zu bytes of device memory: %s",
+                           b.n_filters, n, mask_bytes, g_err.c_str());
+        }
         vb_mask_kernel<<<grid_for((uint64_t)b.mask_words * 32, 256, h->sm_count * 8), 256, 0, h->stream>>>(
             h->scope_id.as<uint32_t>(), h->created.as<int64_t>(), h->modified.as<int64_t>(), h->alive.as<uint32_t>(), n,
             b.d_filters, b.n_filters, b.mask_words, b.need_created, b.need_modified, b.need_scope, h->mask.as<uint32_t>());
@@ -1615,6 +1713,7 @@ static int run_branches(vb_index* h, const Batch& b, bool safe, int phase = 0) {
             g.n_rows_total = n; g.row_begin = r0; g.row_end = r1; g.row_base = (uint32_t)h->row_base;
             g.d_pad = (uint32_t)h->d_pad; g.n_queries = b.B; g.sm_count = h->sm_count; g.stream = sd;
             g.direct = direct; g.plan = plan; g.mask_of_host = b.mask_of_host.data();
+            g.ftab = tiled ? b.ft_k2t : b.ft_k2;
             if (zsel) {                                          // K2T walks the compacted copy when the device-side decision says so
                 g.sel = h->sel_meta.as<uint32_t>() + zsel->meta_off; g.sel_ids = h->sel_ids.as<uint32_t>() + zsel->row_off;
                 g.sel_inv_norm = h->sel_inv.as<float>() + zsel->row_off;

@@ -798,14 +798,38 @@ class VectorStoreService:
         date_end: int | None = None,
         date_field: str | None = None,
         fusion: str | None = None,
+        filters: list[dict | None] | None = None,
     ) -> list[list[StoredChunk]]:
-        """Additive: ``search`` for B queries sharing one filter, in one device pass."""
+        """Additive: ``search`` for B queries in one device pass.
+
+        By default the B queries share one filter, built from the folder and date arguments.  ``filters`` gives each
+        query its own instead: a list of B entries, each None (unfiltered) or a dict of ``_build_filter`` keyword
+        arguments (``folder_filter``, ``include_folders``, ``exclude_folders``, ``exclude_index_folders``,
+        ``date_start``, ``date_end``, ``date_field``, ``scope_key``).  Queries whose filters have equal content share
+        one device mask.  Giving ``filters`` together with any of the shared filter arguments is a ValueError."""
         index = self.client
         coll = self._coll
-        search_filter = self._build_filter(
-            folder_filter, include_folders, exclude_folders, exclude_index_folders,
-            date_start=date_start, date_end=date_end, date_field=date_field)
         B = len(query_embeddings)
+        if filters is None:
+            search_filter = self._build_filter(
+                folder_filter, include_folders, exclude_folders, exclude_index_folders,
+                date_start=date_start, date_end=date_end, date_field=date_field)
+            flts = [search_filter] if search_filter is not None else None
+            filter_of = np.zeros(B, np.int32) if search_filter is not None else None
+        else:
+            shared = (folder_filter, include_folders, exclude_folders, exclude_index_folders, date_start, date_end, date_field)
+            if any(a is not None for a in shared):
+                raise ValueError("give either per-query filters or the shared filter arguments, not both")
+            if len(filters) != B:
+                raise ValueError(f"filters must have one entry per query: {len(filters)} for {B} queries")
+            flts, fo = [], np.full(B, -1, np.int32)
+            for i, kw in enumerate(filters):
+                f = None if kw is None else self._build_filter(**kw)
+                if f is not None:
+                    fo[i] = len(flts)
+                    flts.append(f)
+            filter_of = fo if flts else None
+            flts = flts or None
         if _is_device_tensor(query_embeddings):
             # tensor hand-off (SURVEY 8 f-4): the embedding model's output (embedding.py:76-86) stays on the GPU
             q = query_embeddings
@@ -828,9 +852,7 @@ class VectorStoreService:
             if coll.n_live == 0:
                 return [[] for _ in range(B)]
             res = index.search_batch(
-                q, sparse if any_sparse else None,
-                filters=[search_filter] if search_filter is not None else None,
-                filter_of=np.zeros(B, np.int32) if search_filter is not None else None,
+                q, sparse if any_sparse else None, filters=flts, filter_of=filter_of,
                 limit=limit, kprime=limit * 3 if any_sparse else limit,
                 fusion=(fusion or self.fusion) if any_sparse else "dense", sparse_weight=sparse_weight)
             return [self._rows_to_chunks(coll, res.hits(i)) for i in range(B)]
