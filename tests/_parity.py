@@ -5,8 +5,28 @@ scores fall within a stated relative tolerance of a tie.  ``assert_same_ranking`
 exactly that: positions whose reference scores are within ``rel_tol`` of each other form a tie
 cluster; within a cluster any order is accepted; the last cluster may exchange members with
 items that fell just below the cut-off (they are checked by score instead).
+
+The sparse branch is bit-exact, so it is held to more: ``assert_same_list`` requires the very same
+(row, score) sequence, scores equal bit for bit — the total order (score desc, row asc) decides
+every tie, including the ones at the k'-th position.
 """
 from __future__ import annotations
+
+import struct
+
+
+def _bits(x) -> bytes:
+    return struct.pack("<d", float(x))
+
+
+def assert_same_list(got, want, what=""):
+    """got / want: sequences of (row, score).  Identical rows in identical order, scores bit-equal."""
+    got = [(int(g[0]), float(g[1])) for g in got]
+    want = [(int(w[0]), float(w[1])) for w in want]
+    for i, (g, w) in enumerate(zip(got, want)):
+        assert g[0] == w[0] and _bits(g[1]) == _bits(w[1]), \
+            f"{what}: rank {i}: got {g} want {w}\n got={got[max(0, i - 3):i + 4]}\nwant={want[max(0, i - 3):i + 4]}"
+    assert len(got) == len(want), f"{what}: length {len(got)} != {len(want)}\n got={got[-4:]}\nwant={want[-4:]}"
 
 
 def _close(a: float, b: float, rel_tol: float, abs_tol: float) -> bool:

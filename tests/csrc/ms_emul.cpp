@@ -17,6 +17,7 @@ extern "C" int ms_emul_segment(
     uint32_t* out_rows, float* out_scores, uint32_t max_out, uint64_t* stats /* [4]: essential postings, units, n_ess, lookups-unused */)
 {
     if (nt == 0 || nt > VB_MS_MAX_TERMS) return -1;
+    tau = vb_ms_exact_tau(tau);                                 // K3M runs under the next float below the list's tau
     // ---- plan (vb_ms_plan_kernel) ----
     VbMsPlanShared s;
     for (uint32_t j = 0; j < nt; ++j)

@@ -11,7 +11,7 @@ import pytest
 
 import _data
 import _coded
-from _parity import assert_same_ranking, assert_topk_valid
+from _parity import assert_same_list, assert_same_ranking, assert_topk_valid
 from oracle import oracle as O
 from oracle import oracle_c
 
@@ -79,7 +79,7 @@ def check(got, want, B, tol, what):
         assert_same_ranking(gd, wd, rel_tol=tol, abs_tol=tol, what=f"{what} dense q{i}")
         gs = got.branch(i, "sparse")
         ws = [(int(want["sparse_rows"][i, j]), float(want["sparse_scores"][i, j])) for j in range(want["sparse_counts"][i])]
-        assert_same_ranking(gs, ws, rel_tol=0.0, what=f"{what} sparse q{i}")      # fp64 ordered sums: bit-equal
+        assert_same_list(gs, ws, what=f"{what} sparse q{i}")      # fp64 ordered sums: bit-equal
         gf = got.hits(i)
         wf = [(int(want["rows"][i, j]), float(want["scores"][i, j])) for j in range(want["counts"][i])]
         assert_same_ranking(gf, wf, rel_tol=10 * tol, abs_tol=10 * tol, what=f"{what} fused q{i}")
@@ -185,7 +185,7 @@ def test_per_query_filters_in_one_batch(world):
             wd = [(int(want["dense_rows"][i, j]), float(want["dense_scores"][i, j])) for j in range(want["dense_counts"][i])]
             assert_same_ranking(got.branch(i, "dense"), wd, rel_tol=tol, abs_tol=tol, what=f"path{path} q{i}")
             ws = [(int(want["sparse_rows"][i, j]), float(want["sparse_scores"][i, j])) for j in range(want["sparse_counts"][i])]
-            assert_same_ranking(got.branch(i, "sparse"), ws, rel_tol=0.0, what=f"path{path} sparse q{i}")
+            assert_same_list(got.branch(i, "sparse"), ws, what=f"path{path} sparse q{i}")
     world["ix"].set_option("dense_path", 0)
 
 
@@ -438,7 +438,7 @@ def test_large_batch_hybrid_against_oracle():
             wd = [(int(want["dense_rows"][i, j]), float(want["dense_scores"][i, j])) for j in range(want["dense_counts"][i])]
             assert_same_ranking(got.branch(i, "dense"), wd, rel_tol=2e-5, abs_tol=2e-5, what=f"dense q{i}")
             ws = [(int(want["sparse_rows"][i, j]), float(want["sparse_scores"][i, j])) for j in range(want["sparse_counts"][i])]
-            assert_same_ranking(got.branch(i, "sparse"), ws, rel_tol=0.0, what=f"sparse q{i}")
+            assert_same_list(got.branch(i, "sparse"), ws, what=f"sparse q{i}")
             fusion_bit_exact(got, i, 10, fusion, 0.1)
     # MaxScore pruning forced on: identical sparse lists (bit for bit) and fused results
     base = ix.search_batch(Q, SP, [engine.Filter(*flt)], fo, limit=10, fusion="rrf", branches=True)
@@ -462,7 +462,7 @@ def test_large_batch_hybrid_against_oracle():
     wantm = cc.search_batch(Q, SPm, [flt], fo, limit=10, fusion=2)
     for i in range(B):
         ws = [(int(wantm["sparse_rows"][i, j]), float(wantm["sparse_scores"][i, j])) for j in range(wantm["sparse_counts"][i])]
-        assert_same_ranking(gotm.branch(i, "sparse"), ws, rel_tol=0.0, what=f"mixed-sign sparse q{i}")
+        assert_same_list(gotm.branch(i, "sparse"), ws, what=f"mixed-sign sparse q{i}")
     # the pipelined stream API returns the same answers as the one-call API
     packed = [ix.pack(Q[j:j + 16], SP[j:j + 16], [engine.Filter(*flt)], np.zeros(16, np.int32), limit=10, fusion="rrf")
               for j in range(0, B, 16)]
@@ -694,7 +694,7 @@ def test_sparse_relaxed_mode_stress(seed):
                 want = cc.search_batch(Q, SP, fl, fo, limit=20, fusion=2, apply_idf=apply_idf)
                 for i in range(B):
                     ws = [(int(want["sparse_rows"][i, j]), float(want["sparse_scores"][i, j])) for j in range(want["sparse_counts"][i])]
-                    assert_same_ranking(got.branch(i, "sparse"), ws, rel_tol=0.0, what=f"stress nt={nts[i]} idf={apply_idf} filter={fl is not None}")
+                    assert_same_list(got.branch(i, "sparse"), ws, what=f"stress nt={nts[i]} idf={apply_idf} filter={fl is not None}")
         assert ix.stats()["overflow_reruns"] <= 8
     finally:
         ix.close()
@@ -729,7 +729,7 @@ def test_k3m_equals_k3_and_oracle(world):
             want = world["cc"].search_batch(Q, SP, None if flt is None else [flt], fo, limit=20, kprime=60, fusion=2)
             for i in range(B):
                 ws = [(int(want["sparse_rows"][i, j]), float(want["sparse_scores"][i, j])) for j in range(want["sparse_counts"][i])]
-                assert_same_ranking(base.branch(i, "sparse"), ws, rel_tol=0.0, what=f"k3m f{fi} q{i}")
+                assert_same_list(base.branch(i, "sparse"), ws, what=f"k3m f{fi} q{i}")
     finally:
         for k, v in {"sparse_ms": 1, "ms_chunk": 0, "ms_budget": 100, "seg_ratio": 0, "seg_first": 2048, "safe_mode": 0, "sparse_dense": 1}.items():
             ix.set_option(k, v)
@@ -884,7 +884,7 @@ def test_query_tiled_gemm_at_model_dimensions_against_oracle(dim):
             wd = [(int(want["dense_rows"][j, t]), float(want["dense_scores"][j, t])) for t in range(want["dense_counts"][j])]
             assert_same_ranking(got.branch(i, "dense"), wd, rel_tol=1e-3, abs_tol=1e-3, what=f"K2T d{dim} {name} dense q{i}")
             ws = [(int(want["sparse_rows"][j, t]), float(want["sparse_scores"][j, t])) for t in range(want["sparse_counts"][j])]
-            assert_same_ranking(got.branch(i, "sparse"), ws, rel_tol=0.0, what=f"K2T d{dim} {name} sparse q{i}")
+            assert_same_list(got.branch(i, "sparse"), ws, what=f"K2T d{dim} {name} sparse q{i}")
             fusion_bit_exact(got, i, limit, "rrf", 0.1)
         for i in range(0, B, 37):                     # properties for queries the oracle did not score
             rows = [r for r, _ in got.branch(i, "dense")]
@@ -957,7 +957,7 @@ def test_k3h_long_queries_equal_k3_and_oracle(world):
             want = world["cc"].search_batch(Q, SP, None if flt is None else [flt], fo, limit=20, kprime=60, fusion=2)
             for i in range(B):
                 ws = [(int(want["sparse_rows"][i, j]), float(want["sparse_scores"][i, j])) for j in range(want["sparse_counts"][i])]
-                assert_same_ranking(base.branch(i, "sparse"), ws, rel_tol=0.0, what=f"k3h f{fi} q{i}")
+                assert_same_list(base.branch(i, "sparse"), ws, what=f"k3h f{fi} q{i}")
     finally:
         for k, v in {"sparse_mh": 0, "ms_max_terms": 16, "safe_mode": 0, "seg_ratio": 0, "ms_staged": 1, "sparse_dense": 1}.items():
             ix.set_option(k, v)

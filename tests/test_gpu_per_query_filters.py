@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 
 import _data
-from _parity import assert_same_ranking
+from _parity import assert_same_list, assert_same_ranking
 from oracle import oracle as O
 from oracle import oracle_c
 
@@ -88,7 +88,7 @@ def check_batch(w, got, fl, fo, what, limit=100):
         wd = [(int(want["dense_rows"][j, t]), float(want["dense_scores"][j, t])) for t in range(want["dense_counts"][j])]
         assert_same_ranking(got.branch(i, "dense"), wd, rel_tol=1e-3, abs_tol=1e-3, what=f"{what} dense q{i}")
         ws = [(int(want["sparse_rows"][j, t]), float(want["sparse_scores"][j, t])) for t in range(want["sparse_counts"][j])]
-        assert_same_ranking(got.branch(i, "sparse"), ws, rel_tol=0.0, what=f"{what} sparse q{i}")
+        assert_same_list(got.branch(i, "sparse"), ws, what=f"{what} sparse q{i}")
         fusion_bit_exact(got, i, limit)
     n_pass = {}
     for i in range(B):

@@ -36,12 +36,8 @@ def emul(tmp_path_factory):
     return lib
 
 
-@pytest.fixture(scope="module")
-def index():
-    """Inverted index, dense columns and forward CSR of a small corpus, as the library builds them."""
-    corpus = _data.make_corpus(seed=11, n=9000, dim=8, vocab=300)
-    coded = _coded.code_corpus(corpus)
-    indptr, terms, vals = coded["csr"]
+def _index_of(indptr, terms, vals, corpus=None):
+    """Inverted index, dense columns and forward CSR of a corpus, as the library builds them."""
     n = len(indptr) - 1
     rows = np.repeat(np.arange(n, dtype=np.uint32), np.diff(indptr))
     order = np.lexsort((rows, terms))
@@ -77,6 +73,46 @@ def index():
                 post_val=np.ascontiguousarray(post_val), uniq=uniq, ptr=ptr, df=df, maxval=maxval, hv=hv, stride=stride, hof=hof)
 
 
+@pytest.fixture(scope="module")
+def index():
+    """A small BM25-style corpus: random document lengths, so exact score ties are rare."""
+    corpus = _data.make_corpus(seed=11, n=9000, dim=8, vocab=300)
+    coded = _coded.code_corpus(corpus)
+    return _index_of(*coded["csr"], corpus=corpus)
+
+
+TIE_A, TIE_B = 1000, 2000
+
+
+@pytest.fixture(scope="module")
+def ties_index():
+    """A corpus where most scores tie: term A on the odd rows, term B on the even rows (equal df, so a query [A, B]
+    weighs them equally), values from {0.5, 0.75, 1.0, 1.25}, one extra non-query term per row, and every 37th row
+    with a query-term value of 0.0 (score 0, still a candidate: it overlaps the query).  The postings of A and B
+    interleave in row order, so a stage that walks them in position order meets tied rows out of row order."""
+    n = 6000
+    rng = np.random.RandomState(17)
+    val = rng.choice(np.float32([0.5, 0.75, 1.0, 1.25]), size=n)
+    val[::37] = 0.0
+    extra = 3000 + rng.randint(0, 50, size=n)
+    indptr = np.arange(0, 2 * n + 1, 2, dtype=np.int64)
+    terms = np.empty(2 * n, np.uint32)
+    vals = np.empty(2 * n, np.float32)
+    terms[0::2] = np.where(np.arange(n) % 2 == 1, TIE_A, TIE_B)
+    vals[0::2] = val
+    terms[1::2] = extra
+    vals[1::2] = rng.choice(np.float32([0.5, 1.0]), size=n)
+    return _index_of(indptr, terms, vals)
+
+
+def _tie_query(ix, extra_term=None):
+    """[A, B] (plus optionally one extra term) with the IDF weights of the index: A and B weigh exactly the same."""
+    n = ix["n"]
+    dfm = {int(t): int(d) for t, d in zip(ix["uniq"], ix["df"])}
+    q_idx = sorted([TIE_A, TIE_B] + ([extra_term] if extra_term is not None else []))
+    return q_idx, [math.log((n - dfm[t] + 0.5) / (dfm[t] + 0.5) + 1.0) for t in q_idx]
+
+
 def _reference(ix, q_idx, q_w, r0, r1, mask_bits, tau):
     out = {}
     for r in range(r0, r1):
@@ -84,7 +120,7 @@ def _reference(ix, q_idx, q_w, r0, r1, mask_bits, tau):
             continue
         a, b = ix["indptr"][r], ix["indptr"][r + 1]
         s = oracle.sparse_dot_product(q_idx, q_w, ix["terms"][a:b].tolist(), [float(x) for x in ix["vals"][a:b]])
-        if s is not None and np.float32(s) > np.float32(tau):
+        if s is not None and np.float32(s) >= np.float32(tau):
             out[r] = np.float32(s)
     return out
 
@@ -134,25 +170,42 @@ def _query(ix, seed, nnz):
     return q_idx, w
 
 
-@pytest.mark.parametrize("seed", range(6))
-@pytest.mark.parametrize("masked", [False, True])
-def test_candidates_match_oracle(emul, index, seed, masked):
-    ix = index
+def _check_candidates(emul, ix, q_idx, w, mask_bits):
+    """Every threshold, segment, chunk, budget and lookup kind: the candidates are the rows whose score reaches tau (a
+    row that equals tau may still win its tie on the row id), with the oracle's score bits."""
     n = ix["n"]
-    q_idx, w = _query(ix, 100 + seed, (3, 12) if seed % 2 == 0 else (10, 40))
-    rng = np.random.RandomState(seed)
-    mask_bits = rng.randint(0, 2 ** 32, size=(n + 31) // 32, dtype=np.uint64).astype(np.uint32) if masked else None
     full = _reference(ix, q_idx, w, 0, n, mask_bits, -np.inf)
     ranked = sorted(full.values(), reverse=True)
     taus = [-np.inf, 0.0, float(ranked[min(len(ranked) - 1, 30)]), float(ranked[min(len(ranked) - 1, 300)]), float(ranked[0])]
     for tau in taus:
         for (r0, r1) in ((0, n), (2048, n), (2048, 6144)):
-            want = {r: s for r, s in full.items() if r0 <= r < r1 and s > np.float32(tau)}
+            want = {r: s for r, s in full.items() if r0 <= r < r1 and s >= np.float32(tau)}
             for chunk, budget, tabs, heavy in ((512, 100, True, True), (2048, 20, False, True), (512, 100, True, False)):
                 got, stats = _run(emul, ix, q_idx, w, r0, r1, mask_bits, np.float32(tau), chunk, budget, tabs, heavy)
                 assert got.keys() == want.keys(), (tau, r0, r1, chunk, sorted(set(got) ^ set(want))[:10])
                 bad = [r for r in want if got[r].tobytes() != want[r].tobytes()]
                 assert not bad, f"score bits differ for rows {bad[:5]}"
+
+
+@pytest.mark.parametrize("seed", range(6))
+@pytest.mark.parametrize("masked", [False, True])
+def test_candidates_match_oracle(emul, index, seed, masked):
+    ix = index
+    q_idx, w = _query(ix, 100 + seed, (3, 12) if seed % 2 == 0 else (10, 40))
+    rng = np.random.RandomState(seed)
+    mask_bits = rng.randint(0, 2 ** 32, size=(ix["n"] + 31) // 32, dtype=np.uint64).astype(np.uint32) if masked else None
+    _check_candidates(emul, ix, q_idx, w, mask_bits)
+
+
+@pytest.mark.parametrize("extra", [None, 3007])
+@pytest.mark.parametrize("masked", [False, True])
+def test_candidates_match_oracle_on_ties(emul, ties_index, extra, masked):
+    ix = ties_index
+    q_idx, w = _tie_query(ix, extra)
+    assert w[q_idx.index(TIE_A)] == w[q_idx.index(TIE_B)]
+    rng = np.random.RandomState(3)
+    mask_bits = rng.randint(0, 2 ** 32, size=(ix["n"] + 31) // 32, dtype=np.uint64).astype(np.uint32) if masked else None
+    _check_candidates(emul, ix, q_idx, w, mask_bits)
 
 
 def test_pruning_skips_most_postings(emul, index):
@@ -202,35 +255,32 @@ def test_stress_values(emul, index):
         full = _reference(ix, q_idx, w, 0, n, None, -np.inf)
         ranked = sorted(full.values(), reverse=True)
         for tau in (-np.inf, float(ranked[min(len(ranked) - 1, 50)])):
-            want = {r: s for r, s in full.items() if s > np.float32(tau)}
+            want = {r: s for r, s in full.items() if s >= np.float32(tau)}
             got, _ = _run(emul, ix, q_idx, w, 0, n, None, np.float32(tau), 512, 100)
             assert got.keys() == want.keys()
             assert all(got[r].tobytes() == want[r].tobytes() for r in want)
 
 
-@pytest.mark.parametrize("seed", range(5))
-def test_stages_score_every_row_once_and_reach_the_exact_top_k(emul, index, seed):
+def _check_stages(emul, ix, q_idx, w, mask_bits, ks, first=16):
     """The staged flow of a search: stage 0 scores the first postings (position order) with no threshold, each later
-    stage 32x more under the threshold the earlier stages produced.  No row may be reported twice across stages and
-    the top-k of everything reported must be the oracle's top-k, scores bit for bit."""
-    ix = index
+    stage 32x more under the threshold the earlier stages produced (the k-th best score so far); stage 0 takes
+    first * k postings.  No row may be
+    reported twice across stages and the top-k of everything reported must be the oracle's top-k in the order
+    (score desc, row asc), scores bit for bit."""
     n = ix["n"]
-    q_idx, w = _query(ix, 700 + seed, (3, 12) if seed % 2 else (12, 40))
-    rng = np.random.RandomState(seed)
-    mask_bits = rng.randint(0, 2 ** 32, size=(n + 31) // 32, dtype=np.uint64).astype(np.uint32) if seed % 2 else None
     full = _reference(ix, q_idx, w, 0, n, mask_bits, -np.inf)
-    for k in (5, 30):
+    dfm = {int(t): int(d) for t, d in zip(ix["uniq"], ix["df"])}
+    total = sum(dfm.get(t, 0) for t in q_idx)
+    for k in ks:
         best = {}
         tau = np.float32(-np.inf)
-        lo, hi = 0, 16 * k
-        dfm = {int(t): int(d) for t, d in zip(ix["uniq"], ix["df"])}
-        total = sum(dfm.get(t, 0) for t in q_idx)
+        lo, hi = 0, first * k
         n_stage = 0
         while lo < total:
             got, _ = _run(emul, ix, q_idx, w, 0, n, mask_bits, tau, 512, 100, stage=(lo, hi))
             for r, s_ in got.items():
                 assert r not in best, f"row {r} scored in two stages"
-                assert s_ > tau
+                assert s_ >= tau
                 best[r] = s_
             ranked = sorted(best.values(), reverse=True)
             if len(ranked) >= k:
@@ -240,8 +290,33 @@ def test_stages_score_every_row_once_and_reach_the_exact_top_k(emul, index, seed
         assert n_stage >= 2
         want = sorted(((s_, -r) for r, s_ in full.items()), reverse=True)[:k]
         have = sorted(((s_, -r) for r, s_ in best.items()), reverse=True)[:k]
-        assert [(float(a), b) for a, b in have] == [(float(a), b) for a, b in want]
+        assert [(float(a), -b) for a, b in have] == [(float(a), -b) for a, b in want], f"top {k}: (score, row)"
         assert all(best[-b].tobytes() == full[-b].tobytes() for _, b in want)
+
+
+@pytest.mark.parametrize("seed", range(5))
+def test_stages_score_every_row_once_and_reach_the_exact_top_k(emul, index, seed):
+    ix = index
+    q_idx, w = _query(ix, 700 + seed, (3, 12) if seed % 2 else (12, 40))
+    rng = np.random.RandomState(seed)
+    mask_bits = rng.randint(0, 2 ** 32, size=(ix["n"] + 31) // 32, dtype=np.uint64).astype(np.uint32) if seed % 2 else None
+    _check_stages(emul, ix, q_idx, w, mask_bits, (5, 30))
+
+
+@pytest.mark.parametrize("extra", [None, 3007])
+@pytest.mark.parametrize("masked", [False, True])
+def test_stages_keep_the_ties_at_the_cut_off(emul, ties_index, extra, masked):
+    """On the tie-heavy corpus a later stage meets rows that EQUAL the threshold but have a lower id than the current
+    k-th row: they belong in the top k.  Cut-offs inside tie groups (5, 30, 300) and among the score-0 rows."""
+    ix = ties_index
+    q_idx, w = _tie_query(ix, extra)
+    rng = np.random.RandomState(4)
+    mask_bits = rng.randint(0, 2 ** 32, size=(ix["n"] + 31) // 32, dtype=np.uint64).astype(np.uint32) if masked else None
+    _check_stages(emul, ix, q_idx, w, mask_bits, (5, 30, 300))
+    full = _reference(ix, q_idx, w, 0, ix["n"], mask_bits, -np.inf)
+    k0 = sum(1 for s_ in full.values() if s_ > 0) + 3
+    assert k0 < len(full)
+    _check_stages(emul, ix, q_idx, w, mask_bits, (k0,), first=1)
 
 
 @pytest.mark.parametrize("seed", range(5))

@@ -4,7 +4,7 @@ import pytest
 
 import _data
 import _coded
-from _parity import assert_same_ranking
+from _parity import assert_same_list, assert_same_ranking
 from oracle import oracle as O
 from oracle import oracle_c
 
@@ -61,7 +61,7 @@ def test_c_oracle_matches_python_oracle(setup, case, fusion):
         gs = [(int(out["sparse_rows"][i, j]), out["sparse_scores"][i, j]) for j in range(out["sparse_counts"][i])]
         assert_same_ranking(gd, [(p.row, p.score) for p in d], rel_tol=2e-6, abs_tol=1e-7, what=f"dense q{i}")
         # sparse scores: identical arithmetic (f64 accumulate in index order) -> bit-equal
-        assert_same_ranking(gs, [(p.row, p.score) for p in s], rel_tol=0.0, what=f"sparse q{i}")
+        assert_same_list(gs, [(p.row, p.score) for p in s], what=f"sparse q{i}")
 
 
 def test_dense_only_and_df(setup):

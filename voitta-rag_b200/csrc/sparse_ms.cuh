@@ -284,6 +284,14 @@ VB_HD uint32_t vb_mh_shift(uint64_t essential_postings, uint32_t seg_rows) {
 
 VB_HD double vb_ms_tau_lo(double tau_d) { return tau_d > 0.0 ? tau_d * (1.0 - 1e-9) : tau_d * (1.0 + 1e-9); }
 
+// K3M keeps a row whose score EQUALS the list's threshold: the stages visit rows in posting order (descending ub), not
+// in row order, so a row that ties with the k'-th best can arrive after it and still win the tie on its lower row id;
+// the compaction then picks by key.  So a K3M launch runs under the next float below the list's tau (the rule of
+// vb_tau_import_kernel): the plan's partition, the bound tests (tau_lo) and the exact compare all derive from it —
+// lowering the exact compare alone is not enough, the fp32 rounding of a tied row's score may lie above its fp64
+// sum by more than tau_lo's margin.  Every row is still scored once; the cost is an append per tied row.
+VB_HD float vb_ms_exact_tau(float tau) { return nextafterf(tau, -INFINITY); }
+
 #ifdef __CUDACC__
 #include "common.cuh"
 
@@ -349,7 +357,8 @@ vb_ms_plan_kernel(const VbMsPlanArgs a)
     const bool active = cls != 0u && ((a.classes >> (cls - 1u)) & 1u);
     __shared__ unsigned long long s_ess_post;
     if (j == 0) s_ess_post = 0ull;
-    const double tau_d = (double)a.tau[a.n_queries + q];
+    const float tau_f = a.tau[a.n_queries + q];
+    const double tau_d = (double)(cls == 1u ? vb_ms_exact_tau(tau_f) : tau_f);     // K3M: ties kept (vb_ms_exact_tau)
     if (active) {
         if (j < nt) vb_ms_plan_load(s, j, a.post_row, a.term_tab, a.q_plo[t_lo + j], a.q_phi[t_lo + j], a.q_tab[t_lo + j], a.q_shift[t_lo + j],
                                     a.n_rows, a.seg_row0, a.seg_row1, a.q_ub[t_lo + j]);
@@ -520,7 +529,7 @@ vb_ms_score_kernel(const VbMsArgs a)
         c.w = s_w; c.suf = s_suf; c.hidx = s_hidx; c.tab = s_tab; c.shift = s_shift; c.plo = s_plo; c.phi = s_phi;
         c.nt = nt; c.n_ess = qi.n_ess; c.tau_lo = qi.tau_lo;
         c.delta = (double)(4u * nt) * 1.1102230246251565e-16;
-        c.tau = a.tau[list];
+        c.tau = vb_ms_exact_tau(a.tau[list]);                           // (the plan derived tau_lo from the same value)
         __syncthreads();
         // U postings per thread per step: their (row, value) loads and filter words are issued together
         for (uint32_t pb = p0 + tid; pb < p1; pb += VB_MS_U * VB_MS_THREADS) {
