@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define VB_ABI_VERSION 3
+#define VB_ABI_VERSION 4
 #define VB_TS_MISSING INT64_MIN
 #define VB_MAX_KPRIME 1024          /* limit*3 <= 1024 */
 #define VB_MAX_QUERY_TERMS 256      /* non-zeros per sparse query */
@@ -183,17 +183,6 @@ int vb_merge_fuse(vb_index* h, const vb_query_batch* q, uint32_t n_shards,
  *   vb_fetch     D2H of the results, stream sync, decode; *overflowed = 1 asks for a safe-mode re-run
  *                (vb_set_option "safe_mode"). */
 int vb_stage(vb_index* h, const vb_query_batch* q, int32_t want_branches, int32_t need_corpus);
-/* Threshold exchange of the row-sharded flow (optional; between vb_stage and vb_run_local):
- *   vb_run_local_begin  set-up + the first row segment of both branches;
- *   vb_tau_export       copy the per-list thresholds (float [2*B]: score of the list's current k'-th best,
- *                       -inf while it holds fewer) to a device buffer — the caller all-reduces it with MAX over
- *                       the shards: a row scoring below ANY shard's k'-th best cannot be in the global top-k';
- *   vb_tau_import       raise this shard's thresholds to (just below) the reduced ones;
- * vb_run_local then continues with the remaining segments.  Results are unchanged; shards stop collecting
- * candidates that could only lose at the merge. */
-int vb_run_local_begin(vb_index* h);
-int vb_tau_export(vb_index* h, float* tau_dev);
-int vb_tau_import(vb_index* h, const float* tau_dev);
 int vb_run_local(vb_index* h, uint64_t* cand_dev);
 int vb_run_fuse(vb_index* h, uint32_t n_shards, const uint64_t* gathered_dev);
 int vb_fetch(vb_index* h, vb_result* out, int32_t* overflowed);

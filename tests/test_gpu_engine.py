@@ -283,7 +283,7 @@ def test_dimensions_and_padding(dim):
     ix.close()
 
 
-def test_two_shards_merge_equals_single_index(world):
+def test_two_shards_merged_and_staged_equal_single_index(world):
     """Row-sharded search (SURVEY §8e) emulated on one GPU: two indexes with row offsets, global
     IDF from summed df, candidates concatenated as an all-gather would, merged and fused.  Must be
     bit-identical to the single-index answer."""
@@ -322,29 +322,22 @@ def test_two_shards_merge_equals_single_index(world):
             assert np.array_equal(getattr(merged, name), getattr(single, name)), (fusion, name)
         # idf computed by numpy here vs libm in the library may differ in the last bit of a weight
         np.testing.assert_allclose(merged.sparse_scores, single.sparse_scores, rtol=1e-6)
-        # the same with the threshold exchange of the sharded flow (all-reduce MAX emulated with torch.maximum):
-        # shards keep fewer candidates, the merged answer is identical
-        taus = []
+        # the same through the staged calls the sharded flow makes (ShardedIndex._enqueue):
+        # stage -> run_local -> all-gather (emulated by torch.cat) -> run_fuse -> fetch
+        for buf in bufs:
+            buf.zero_()
+        torch.cuda.synchronize()
         staged = []
-        for sh_ix in (a, b):
-            staged.append(sh_ix.stage(Q, SPW, gf, fo, limit=limit, kprime=k, fusion=fusion, apply_idf=False, branches=True))
-            sh_ix.run_local_begin()
-            t = torch.zeros(2 * len(qs), dtype=torch.float32, device="cuda")
-            sh_ix.tau_export(t.data_ptr())
-            taus.append(t)
-        torch.cuda.synchronize()
-        tmax = torch.maximum(taus[0], taus[1])
-        torch.cuda.synchronize()
         for sh_ix, buf in zip((a, b), bufs):
-            sh_ix.tau_import(tmax.data_ptr())
+            staged.append(sh_ix.stage(Q, SPW, gf, fo, limit=limit, kprime=k, fusion=fusion, apply_idf=False, branches=True))
             sh_ix.run_local(buf.data_ptr())
         torch.cuda.synchronize()
         gathered2 = torch.cat(bufs)
         a.run_fuse(2, gathered2.data_ptr())
-        shared = a.fetch(staged[0])
+        via_stage = a.fetch(staged[0])
         for name in ("rows", "counts", "dense_rows", "dense_scores", "dense_counts", "sparse_rows", "sparse_counts"):
-            assert np.array_equal(getattr(shared, name), getattr(merged, name)), ("threshold exchange", fusion, name)
-        assert np.array_equal(shared.sparse_scores, merged.sparse_scores)
+            assert np.array_equal(getattr(via_stage, name), getattr(merged, name)), ("staged", fusion, name)
+        assert np.array_equal(via_stage.sparse_scores, merged.sparse_scores)
         np.testing.assert_allclose(merged.scores, single.scores, rtol=1e-6, atol=1e-9)
     a.close(); b.close()
 

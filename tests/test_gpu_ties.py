@@ -271,10 +271,10 @@ def test_tie_flood_overflows_and_stays_exact():
         ix.close()
 
 
-def test_ties_across_two_shards(tw):
+def test_ties_across_two_shards_merged_and_staged(tw):
     """Rows 0..SHARD-1 and SHARD.. on two indexes: shard 0 holds many rows that tie with shard 1's k'-th best.  The
-    merged answer equals the single index's and the oracle's, without and with the threshold exchange (which must
-    import the next float below the best k'-th, or shard 0 drops its tied rows of lower global id)."""
+    merged answer equals the single index's and the oracle's, both through search_local + merge_fuse and through the
+    staged calls of the sharded flow (stage -> run_local -> run_fuse -> fetch)."""
     import torch
     eng = tw["engine"]
     ip, tm, vl = tw["csr"]
@@ -304,23 +304,17 @@ def test_ties_across_two_shards(tw):
             b.search_local(bufs[1].data_ptr(), Q, SPW, gf, fo, limit=limit, kprime=k, fusion=fusion)
             torch.cuda.synchronize()
             merged = a.merge_fuse(torch.cat(bufs).data_ptr(), 2, Q, SPW, limit=limit, kprime=k, fusion=fusion, branches=True)
-            staged, taus = [], []
-            for sh in (a, b):
-                staged.append(sh.stage(Q, SPW, gf, fo, limit=limit, kprime=k, fusion=fusion, apply_idf=False, branches=True))
-                sh.run_local_begin()
-                t = torch.zeros(2 * B, dtype=torch.float32, device="cuda")
-                sh.tau_export(t.data_ptr())
-                taus.append(t)
+            for buf in bufs:
+                buf.zero_()
             torch.cuda.synchronize()
-            tmax = torch.maximum(taus[0], taus[1])
-            torch.cuda.synchronize()
+            staged = []
             for sh, buf in zip((a, b), bufs):
-                sh.tau_import(tmax.data_ptr())
+                staged.append(sh.stage(Q, SPW, gf, fo, limit=limit, kprime=k, fusion=fusion, apply_idf=False, branches=True))
                 sh.run_local(buf.data_ptr())
             torch.cuda.synchronize()
             a.run_fuse(2, torch.cat(bufs).data_ptr())
-            exchanged = a.fetch(staged[0])
-            for name, res in (("merged", merged), ("threshold exchange", exchanged)):
+            via_stage = a.fetch(staged[0])
+            for name, res in (("merged", merged), ("staged", via_stage)):
                 for i in range(B):
                     ws = [(int(want["sparse_rows"][i, j]), float(want["sparse_scores"][i, j])) for j in range(want["sparse_counts"][i])]
                     assert_same_list(res.branch(i, "sparse"), ws, what=f"{name} {fusion} sparse q{i}")

@@ -111,7 +111,6 @@ def _worker(rank, world, port, ret):
         cuts = [0, 1100, n]
         shard = FakeShardIndex(coded, cuts[rank], cuts[rank + 1])
         sh = ShardedIndex(shard, rank, world, device=torch.device("cpu"))
-        sh.share_thresholds = True                              # the test double expects the threshold exchange
         t, df = shard.directory()
         sh.finalize(t, df, shard.n)
         Q = np.stack([q for q, _ in queries])
@@ -144,7 +143,7 @@ def _worker(rank, world, port, ret):
         dist.destroy_process_group()
 
 
-def test_two_rank_gloo_sharded_batch_with_per_query_filters():
+def test_two_rank_gloo_single_collective_batch_with_per_query_filters():
     s = socket.socket(); s.bind(("127.0.0.1", 0)); port = s.getsockname()[1]; s.close()
     mgr = mp.Manager()
     ret = mgr.dict()

@@ -1,7 +1,7 @@
 """world_size-2 test of the row-sharded host logic (voitta_rag_b200.sharded) on CPU with the gloo
 backend: global IDF exchange, candidate all-gather, merge-then-fuse.  The per-shard engine is a
 test double backed by the C oracle; the GPU version of the same flow is
-tests/test_gpu_engine.py::test_two_shards_merge_equals_single_index."""
+tests/test_gpu_engine.py::test_two_shards_merged_and_staged_equal_single_index."""
 import ctypes
 import socket
 
@@ -47,24 +47,7 @@ class FakeShardIndex:
         self.st = dict(q=queries, sp=sparse, fl=filters, fo=filter_of, limit=limit, k=kprime, fusion=fusion, w=sparse_weight)
         return "staged"
 
-    # threshold exchange hooks (the double has no thresholds: it exports -inf and ignores the import, which
-    # exercises the collective of ShardedIndex._enqueue on CPU)
-    def run_local_begin(self):
-        self.began = True
-
-    def tau_export(self, ptr):
-        n = 2 * len(self.st["q"])
-        a = np.full(n, -np.inf, np.float32)
-        ctypes.memmove(ptr, a.ctypes.data, a.nbytes)
-
-    def tau_import(self, ptr):
-        n = 2 * len(self.st["q"])
-        got = np.ctypeslib.as_array((ctypes.c_float * n).from_address(ptr))
-        assert np.all(np.isneginf(got))
-        self.imported = True
-
     def run_local(self, ptr):
-        assert getattr(self, "began", False) and getattr(self, "imported", False)
         st = self.st
         fl = None if not st["fl"] else [(f.scope_bits, f.ts_field, f.ts_lo, f.ts_hi) for f in st["fl"]]
         out = self.cc.search_batch(st["q"], st["sp"], fl, st["fo"], st["limit"], st["k"], 1 if st["sp"] is not None else 0,
@@ -120,7 +103,6 @@ def _worker(rank, world, port, ret):
         cuts = [0, 1100, n]
         shard = FakeShardIndex(coded, cuts[rank], cuts[rank + 1])
         sh = ShardedIndex(shard, rank, world, device=torch.device("cpu"))
-        sh.share_thresholds = True                              # exercise the optional threshold all-reduce too
         t, df = shard.directory()
         sh.finalize(t, df, shard.n)
         assert sh.n_live_g == n
@@ -144,7 +126,7 @@ def _worker(rank, world, port, ret):
         dist.destroy_process_group()
 
 
-def test_two_rank_gloo_sharded_search():
+def test_two_rank_gloo_single_collective_search():
     s = socket.socket(); s.bind(("127.0.0.1", 0)); port = s.getsockname()[1]; s.close()
     mgr = mp.Manager()
     ret = mgr.dict()

@@ -286,8 +286,8 @@ VB_HD double vb_ms_tau_lo(double tau_d) { return tau_d > 0.0 ? tau_d * (1.0 - 1e
 
 // K3M keeps a row whose score EQUALS the list's threshold: the stages visit rows in posting order (descending ub), not
 // in row order, so a row that ties with the k'-th best can arrive after it and still win the tie on its lower row id;
-// the compaction then picks by key.  So a K3M launch runs under the next float below the list's tau (the rule of
-// vb_tau_import_kernel): the plan's partition, the bound tests (tau_lo) and the exact compare all derive from it —
+// the compaction then picks by key.  So a K3M launch runs under the next float below the list's tau: the plan's
+// partition, the bound tests (tau_lo) and the exact compare all derive from it —
 // lowering the exact compare alone is not enough, the fp32 rounding of a tied row's score may lie above its fp64
 // sum by more than tau_lo's margin.  Every row is still scored once; the cost is an append per tied row.
 VB_HD float vb_ms_exact_tau(float tau) { return nextafterf(tau, -INFINITY); }

@@ -226,8 +226,8 @@ vb_compact_kernel(VbLists L, float* __restrict__ tau, uint32_t* __restrict__ ove
     for (uint32_t i = threadIdx.x; i < keep; i += VB_COMPACT_THREADS) gkeys[i] = s_sel[i];
     if (threadIdx.x < VB_SUB) L.cnt[(size_t)list * VB_SUB + threadIdx.x] = threadIdx.x == 0 ? keep : 0u;   // the list now lives in sub-range 0
     if (threadIdx.x == 0) {
-        // never below the threshold the segment ran with: another shard's k'-th best may have been imported
-        // (vb_tau_import), and then this list can legitimately hold fewer than k' entries
+        // never below the threshold the segment ran with: a threshold is only ever raised (DESIGN §3), so a list
+        // that holds fewer than k' entries keeps the one it has
         tau[list] = fmaxf(tau[list], (keep >= k) ? vb_key_score(s_sel[k - 1]) : -INFINITY);
     }
 }

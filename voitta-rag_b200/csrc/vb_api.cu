@@ -78,7 +78,7 @@ static size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 struct Batch {
     uint32_t B = 0, k = 0, limit = 0, n_lists = 0, n_qterms = 0, nt_max = 1, n_filters = 0, mask_words = 0, n_blocks = 0;
-    bool any_sparse = false, use_mask = false, any_heavy = false, begun = false;
+    bool any_sparse = false, use_mask = false, any_heavy = false;
     bool any_ms = false, any_old = false, any_mh = false;   // some sparse query goes to K3M / stays on K3 / goes to K3H
     uint32_t n_old = 0;                        // sparse queries that stay on K3 in every segment
     uint32_t n_dir = 0;                        // sparse queries K3 scores in the direct segment when K3M runs in stages (K3 + K3H ones)
@@ -1478,9 +1478,7 @@ static int launch_scan(vb_index* h, const Batch& b, const VbLists& L, uint32_t r
 
 // Score both branches of this shard and leave the exact, sorted top-k' of every list in
 // cand[list][0..cnt).  `safe`: fixed small segments that can never overflow a list.
-// phase 0: everything; 1: set-up + first segment only; 2: the remaining segments (after phase 1, with the
-// thresholds possibly raised in between by vb_tau_import — the multi-GPU layer's threshold exchange)
-static int run_branches(vb_index* h, const Batch& b, bool safe, int phase = 0) {
+static int run_branches(vb_index* h, const Batch& b, bool safe) {
     const uint32_t n = (uint32_t)h->n_rows;
     // segment schedule (boundaries are multiples of VB_ROWS_PER_BLOCK)
     std::vector<uint32_t> bounds{0};
@@ -1526,23 +1524,21 @@ static int run_branches(vb_index* h, const Batch& b, bool safe, int phase = 0) {
     // a first segment: K1F scans in one pass, K3M in posting stages
     const bool k3_direct = do_sparse && (!ms_staged || b.n_dir > 0);
     const uint32_t direct_rows = (bounds[1] <= h->cand_cap && (!k1f || k3_direct)) ? bounds[1] : 0u;
-    if (phase != 2) TRY(init_lists(h, b, direct_rows));
+    TRY(init_lists(h, b, direct_rows));
     // list set-up + query prep (fp32 unit queries for K1, packed bf16 operand for K2) in ONE launch
     TRY(dev_reserve(h, h->q_hat, (size_t)b.B * h->d_pad * 4, false));
     TRY(dev_reserve(h, h->q_bf16, (size_t)(2 * ((size_t)b.B + 256)) * h->d_pad * 2, false));
     TRY(dev_reserve(h, h->q_scale, (size_t)b.B * 4, false));
-    if (phase != 2) {
-        VbListInit li{};
-        li.tau = b.tau; li.cnt = b.cnt; li.overflow = b.overflow; li.gtau = b.gtau; li.n = b.n_lists; li.cnt0 = direct_rows;
-        li.no_direct = ms_staged ? b.d_qms : nullptr; li.n_queries = b.B; li.dense_direct = k1f ? 0u : 1u;
-        vb_prep_query_kernel<<<b.B, 128, 0, h->stream>>>(b.d_q, (uint32_t)h->dim, (uint32_t)h->d_pad, b.B, plan.sub, plan.split,
-                                                         h->q_hat.as<float>(), h->q_bf16.as<__nv_bfloat16>(), h->q_scale.as<float>(),
-                                                         reinterpret_cast<uint32_t*>(h->out.as<unsigned char>() + b.o_bad), li);
-        CKK("vb_prep_query_kernel");
-        ++h->stats.last_launches;
-    }
+    VbListInit li{};
+    li.tau = b.tau; li.cnt = b.cnt; li.overflow = b.overflow; li.gtau = b.gtau; li.n = b.n_lists; li.cnt0 = direct_rows;
+    li.no_direct = ms_staged ? b.d_qms : nullptr; li.n_queries = b.B; li.dense_direct = k1f ? 0u : 1u;
+    vb_prep_query_kernel<<<b.B, 128, 0, h->stream>>>(b.d_q, (uint32_t)h->dim, (uint32_t)h->d_pad, b.B, plan.sub, plan.split,
+                                                     h->q_hat.as<float>(), h->q_bf16.as<__nv_bfloat16>(), h->q_scale.as<float>(),
+                                                     reinterpret_cast<uint32_t*>(h->out.as<unsigned char>() + b.o_bad), li);
+    CKK("vb_prep_query_kernel");
+    ++h->stats.last_launches;
     // K0 filter masks
-    if (b.use_mask && phase != 2) {
+    if (b.use_mask) {
         prof_begin(h, PH_MASK);
         const size_t mask_bytes = (size_t)b.n_filters * b.mask_words * 4;
         if (dev_reserve(h, h->mask, mask_bytes, false) != 0) {
@@ -1585,7 +1581,7 @@ static int run_branches(vb_index* h, const Batch& b, bool safe, int phase = 0) {
         else T = 0.245 * ((b.B + plan.sub - 1) / plan.sub);
         sel_pct = (uint32_t)(95.0 * T / (T + 0.49));
     }
-    if (path == 2 && !k1f && b.use_mask && sel_pct > 0 && !h->sel_no_memory && h->d_pad <= 1024 && phase != 1) {
+    if (path == 2 && !k1f && b.use_mask && sel_pct > 0 && !h->sel_no_memory && h->d_pad <= 1024) {
         bool uniform = b.mask_of_host[0] >= 0;
         for (uint32_t i = 1; uniform && i < b.B; ++i) uniform = b.mask_of_host[i] == b.mask_of_host[0];
         size_t rows_total = 0, meta_total = 0;
@@ -1871,7 +1867,7 @@ static int run_branches(vb_index* h, const Batch& b, bool safe, int phase = 0) {
             TRY(dev_reserve(h, h->ms_counters, 64, false));
         }
     }
-    if (do_sparse && phase != 2) {                              // sparse slice tables (sparse chain)
+    if (do_sparse) {                                            // sparse slice tables (sparse chain)
         const int pi = prof_begin(h, PH_SPARSE, ss);
         const uint64_t total = (uint64_t)b.n_qterms * (fine_blocks + 1);
         if (fine_blocks) {
@@ -1882,20 +1878,18 @@ static int run_branches(vb_index* h, const Batch& b, bool safe, int phase = 0) {
         if (ms_on || mh_on) CK(cudaMemsetAsync(h->ms_counters.p, 0, 64, ss));
         prof_end(h, pi, ss);
     }
-    // K3M stages (normal mode): stage 0 in phases 0 and 1, the rest in phases 0 and 2
-    auto ms_stages = [&](bool first, bool rest) -> int {
+    // K3M stages (normal mode)
+    auto ms_stages = [&]() -> int {
         // stage 0 scores its postings with no threshold (every lookup of every posting): just enough of them to fill a
         // list twice over after filters and ownership
         const uint64_t p0 = std::max<uint64_t>(ms_chunk, std::min<uint64_t>(align_up((size_t)8 * b.k, ms_chunk), h->cand_cap / 4));
         uint64_t lo = 0, hi = p0;
-        for (uint32_t st = 0; lo < b.ms_max_post; ++st) {
+        while (lo < b.ms_max_post) {
             const bool last = hi >= b.ms_max_post;
-            if (st == 0 ? first : rest) {
-                const int pi = prof_begin(h, PH_SPARSE | (last ? PH_BIG : 0), ss);
-                TRY(ms_launch(0u, nb, lo, last ? ~0ull : hi, 1u));
-                prof_end(h, pi, ss);
-                TRY(sparse_compact(L.sub_cap));
-            }
+            const int pi = prof_begin(h, PH_SPARSE | (last ? PH_BIG : 0), ss);
+            TRY(ms_launch(0u, nb, lo, last ? ~0ull : hi, 1u));
+            prof_end(h, pi, ss);
+            TRY(sparse_compact(L.sub_cap));
             lo = hi;
             // a stage appends ~ratio * k' candidates per list at worst (rows are visited best-first, usually far fewer)
             const uint64_t ratio = h->opt_ms_stage_ratio > 0 ? (uint64_t)std::max<int64_t>(2, h->opt_ms_stage_ratio)
@@ -1906,30 +1900,28 @@ static int run_branches(vb_index* h, const Batch& b, bool safe, int phase = 0) {
     };
     // enqueue the two chains interleaved so that neither stream starves on the host side
     const size_t n_seg = bounds.size() - 1;
-    const size_t s_begin = phase == 2 ? 1 : 0, s_end = phase == 1 ? 1 : n_seg;
     size_t big_seg = 0;
     for (size_t s = 1; s < n_seg; ++s) if (bounds[s + 1] - bounds[s] > bounds[big_seg + 1] - bounds[big_seg]) big_seg = s;
     // Order on the sparse stream: K3's direct first segment (fixed slots, counted by the list set-up) and its
     // compaction come BEFORE the K3M stages — a stage's compaction runs over every sparse list and would turn a
     // still-unwritten direct block into an empty list.
-    if (k1f && phase != 1) TRY(dense_single_pass());
-    for (size_t s = s_begin; s < s_end; ++s) {
+    if (k1f) TRY(dense_single_pass());
+    for (size_t s = 0; s < n_seg; ++s) {
         const uint32_t direct = (s == 0 && direct_rows) ? 1u : 0u;
         const bool big = s == big_seg;                          // the segment with the most rows: the roofline's launch
         if (big && !k1f) h->stats.last_big_rows = bounds[s + 1] - bounds[s];
         TRY(dense_segment(bounds[s], bounds[s + 1], direct, big));
         TRY(sparse_segment(bounds[s], bounds[s + 1], direct, big));
         if (s == 0 && ms_staged) {
-            TRY(ms_stages(true, phase != 1));
-            if (two_streams && h->opt_dense_wait_sparse && phase != 1) {
+            TRY(ms_stages());
+            if (two_streams && h->opt_dense_wait_sparse) {
                 if (!h->ev_sp_done) CK(cudaEventCreateWithFlags(&h->ev_sp_done, cudaEventDisableTiming));
                 CK(cudaEventRecord(h->ev_sp_done, ss));
                 sp_done_recorded = true;
             }
         }
     }
-    if (phase == 2 && ms_staged) TRY(ms_stages(false, true));
-    if (do_delta && phase != 1) {
+    if (do_delta) {
         // K3D: the rows appended since the index was built, straight from the forward CSR.  One launch (a few
         // thousand rows against thresholds the indexed rows have already established); the safe mode cuts it into
         // pieces a list cannot overflow on.
@@ -2086,54 +2078,6 @@ extern "C" int vb_stage(vb_index* h, const vb_query_batch* q, int32_t want_branc
     return 0;
 }
 
-__global__ void vb_tau_import_kernel(float* __restrict__ tau, const float* __restrict__ shared, uint32_t n) {
-    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) {
-        // a row that merely EQUALS another shard's k'-th best can still win its tie at the merge (the order is
-        // score desc, global row asc), so the imported threshold is the next float below it
-        const float g = shared[i];
-        const float lowered = (g > -INFINITY && g < INFINITY) ? nextafterf(g, -INFINITY) : -INFINITY;
-        tau[i] = fmaxf(tau[i], lowered);
-    }
-}
-
-extern "C" int vb_run_local_begin(vb_index* h) {
-    if (!h) return vb_fail("vb_run_local_begin: NULL index");
-    std::lock_guard<std::recursive_mutex> lk(h->mu);
-    Batch& b = h->staged_s[h->cur];
-    if (!b.valid) return vb_fail("vb_run_local_begin: no staged batch");
-    if (b.need_corpus && b.n_rows != (uint32_t)h->n_rows) return vb_fail("vb_run_local_begin: the index changed since vb_stage; stage the batch again");
-    CK(cudaSetDevice(h->device));
-    h->stats.last_launches = 0;
-    CK(cudaEventRecord(h->ev0s[h->cur], h->stream));
-    if (h->n_rows == 0) TRY(empty_lists(h, b));
-    else TRY(run_branches(h, b, h->staged_safe, 1));
-    b.begun = true;
-    return 0;
-}
-
-extern "C" int vb_tau_export(vb_index* h, float* tau_dev) {
-    if (!h || !tau_dev) return vb_fail("vb_tau_export: NULL argument");
-    std::lock_guard<std::recursive_mutex> lk(h->mu);
-    const Batch& b = h->staged_s[h->cur];
-    if (!b.valid || !b.begun) return vb_fail("vb_tau_export: call vb_run_local_begin first");
-    CK(cudaSetDevice(h->device));
-    CK(cudaMemcpyAsync(tau_dev, b.tau, (size_t)b.n_lists * 4, cudaMemcpyDeviceToDevice, h->stream));
-    return 0;
-}
-
-extern "C" int vb_tau_import(vb_index* h, const float* tau_dev) {
-    if (!h || !tau_dev) return vb_fail("vb_tau_import: NULL argument");
-    std::lock_guard<std::recursive_mutex> lk(h->mu);
-    const Batch& b = h->staged_s[h->cur];
-    if (!b.valid || !b.begun) return vb_fail("vb_tau_import: call vb_run_local_begin first");
-    CK(cudaSetDevice(h->device));
-    vb_tau_import_kernel<<<(b.n_lists + 255) / 256, 256, 0, h->stream>>>(b.tau, tau_dev, b.n_lists);
-    CKK("vb_tau_import_kernel");
-    ++h->stats.last_launches;
-    return 0;
-}
-
 extern "C" int vb_run_local(vb_index* h, uint64_t* cand_dev) {
     if (!h) return vb_fail("vb_run_local: NULL index");
     std::lock_guard<std::recursive_mutex> lk(h->mu);
@@ -2141,17 +2085,12 @@ extern "C" int vb_run_local(vb_index* h, uint64_t* cand_dev) {
     if (h->staged_s[h->cur].need_corpus && (h->staged_s[h->cur].n_rows != (uint32_t)h->n_rows || h->staged_s[h->cur].gen != h->write_gen))
         return vb_fail("vb_run_local: the index changed since vb_stage; stage the batch again");
     CK(cudaSetDevice(h->device));
-    if (h->staged_s[h->cur].begun) {                            // first segment done by vb_run_local_begin
-        h->staged_s[h->cur].begun = false;
-        if (h->n_rows != 0) TRY(run_branches(h, h->staged_s[h->cur], h->staged_safe, 2));
+    h->stats.last_launches = 0;
+    CK(cudaEventRecord(h->ev0s[h->cur], h->stream));
+    if (h->n_rows == 0) {
+        TRY(empty_lists(h, h->staged_s[h->cur]));
     } else {
-        h->stats.last_launches = 0;
-        CK(cudaEventRecord(h->ev0s[h->cur], h->stream));
-        if (h->n_rows == 0) {
-            TRY(empty_lists(h, h->staged_s[h->cur]));
-        } else {
-            TRY(run_branches(h, h->staged_s[h->cur], h->staged_safe));
-        }
+        TRY(run_branches(h, h->staged_s[h->cur], h->staged_safe));
     }
     if (cand_dev) {
         vb_export_kernel<<<h->staged_s[h->cur].n_lists, 128, 0, h->stream>>>(h->cand.as<uint64_t>(), h->staged_s[h->cur].cnt, h->cand_cap, h->staged_s[h->cur].k, cand_dev, h->staged_s[h->cur].overflow, h->staged_s[h->cur].n_lists);

@@ -71,12 +71,11 @@ class _Stats(C.Structure):
 
 
 # every symbol include/voitta_b200.h declares
-ABI_VERSION = 3          # include/voitta_b200.h VB_ABI_VERSION
+ABI_VERSION = 4          # include/voitta_b200.h VB_ABI_VERSION
 
 EXPORTS = ["vb_abi_version", "vb_last_error", "vb_create", "vb_destroy", "vb_upsert", "vb_upsert_dev",
            "vb_delete_rows", "vb_optimize", "vb_term_stats", "vb_search", "vb_search_local", "vb_merge_fuse",
            "vb_stage", "vb_run_local", "vb_run_fuse", "vb_fetch", "vb_stage_dev", "vb_search_dev",
-           "vb_run_local_begin", "vb_tau_export", "vb_tau_import",
            "vb_set_option", "vb_get_stats", "vb_get_timeline", "vb_sync", "vb_save", "vb_load"]
 
 _lib = None
@@ -117,9 +116,6 @@ def load_library():
     lib.vb_get_stats.argtypes = [vp, C.POINTER(_Stats)]
     lib.vb_sync.argtypes = [vp]
     lib.vb_get_timeline.argtypes = [vp, vp, C.c_uint32, C.POINTER(C.c_uint32)]
-    lib.vb_run_local_begin.argtypes = [vp]
-    lib.vb_tau_export.argtypes = [vp, vp]
-    lib.vb_tau_import.argtypes = [vp, vp]
     lib.vb_save.argtypes = [vp, C.c_char_p]
     lib.vb_load.argtypes = [C.c_char_p, C.c_int32, C.POINTER(vp)]
     _lib = lib
@@ -540,17 +536,6 @@ class Index:
         else:
             self._check(self._lib.vb_stage(self._h, C.byref(packed.c), int(want), int(need_corpus)))
         return packed.result
-
-    def run_local_begin(self) -> None:
-        """Set-up + first row segment of the staged batch (threshold exchange of the sharded flow)."""
-        self._check(self._lib.vb_run_local_begin(self._h))
-
-    def tau_export(self, tau_dev_ptr: int) -> None:
-        """Per-list thresholds (float32 [2*B]) -> device buffer, to be all-reduced with MAX over the shards."""
-        self._check(self._lib.vb_tau_export(self._h, _vp(tau_dev_ptr)))
-
-    def tau_import(self, tau_dev_ptr: int) -> None:
-        self._check(self._lib.vb_tau_import(self._h, _vp(tau_dev_ptr)))
 
     def run_local(self, cand_dev_ptr: int | None = None) -> None:
         self._check(self._lib.vb_run_local(self._h, _vp(cand_dev_ptr)))

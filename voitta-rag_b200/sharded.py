@@ -6,9 +6,8 @@ replicated.  Each rank computes the exact top-k' of both branches over its shard
 (``vb_search_local``); the exchange step of the path is an all-gather of those candidates
 (``[2][B][k']`` packed u64 per rank — NCCL over NVLink on GPUs, gloo in the CPU tests); every rank
 then merges n_shards*k' -> k' per branch and only THEN fuses (min-max and ranks are global
-properties; fusing per shard would be wrong) — ``vb_merge_fuse``.  One optional, tiny collective precedes
-it: an all-reduce(MAX) of the per-list thresholds after the first row segment (``share_thresholds``), which
-lets every shard skip rows that could only lose at the merge; results are unchanged.
+properties; fusing per shard would be wrong) — ``vb_merge_fuse``.  That all-gather is the one collective
+of a batch.
 
 IDF needs global statistics (N = live points, df per term).  They are host-owned: ``finalize()``
 all-gathers each shard's (term, df) directory once and keeps the summed table, so the per-query
@@ -17,7 +16,6 @@ weights are computed identically on every rank without a per-query collective.
 from __future__ import annotations
 
 import math
-import os
 
 import numpy as np
 import torch
@@ -35,10 +33,6 @@ class ShardedIndex:
         self.n_live_g = 0
         self._bufs: dict = {}
         self._idf_cache: dict = {}
-        # optional all-reduce(MAX) of the list thresholds after the first row segment (see _enqueue).  Off by
-        # default: on B200 + NVLink the extra collective (~45 us) costs more than the skipped candidates save at
-        # cfg2's shard sizes (measured at 2 and 8 GPUs); VB200_SHARE_TAU=1 enables it (skewed shards).
-        self.share_thresholds = os.environ.get("VB200_SHARE_TAU", "0") == "1"
         # one CUDA stream carries the library's kernels AND the collective, so they are ordered
         # without host synchronisation
         self.stream = None
@@ -127,15 +121,6 @@ class ShardedIndex:
         b = self._bufs.get(name)
         if b is None or b.numel() < numel:
             b = torch.zeros(numel, dtype=torch.int64, device=self.device)
-            if b.is_cuda:
-                torch.cuda.synchronize(self.device)
-            self._bufs[name] = b
-        return b[:numel]
-
-    def _buf_f32(self, name, numel):
-        b = self._bufs.get(name)
-        if b is None or b.numel() < numel:
-            b = torch.zeros(numel, dtype=torch.float32, device=self.device)
             if b.is_cuda:
                 torch.cuda.synchronize(self.device)
             self._bufs[name] = b
@@ -231,15 +216,6 @@ class ShardedIndex:
         local = self._buf("local", words)
         gathered = self._buf("gathered", words * self.world)
         with self._stream_ctx():
-            if self.world > 1 and self.share_thresholds and hasattr(self.index, "run_local_begin"):
-                # threshold exchange: after the first row segment every shard knows the score of its current
-                # k'-th best per list; the maximum over the shards is a lower bound of the GLOBAL k'-th best, so
-                # the remaining segments of every shard can ignore rows below it (they would lose at the merge)
-                tau = self._buf_f32("tau", 2 * B)
-                self.index.run_local_begin()
-                self.index.tau_export(tau.data_ptr())
-                dist.all_reduce(tau, op=dist.ReduceOp.MAX, group=self.group)
-                self.index.tau_import(tau.data_ptr())
             self.index.run_local(local.data_ptr())
             if self.world > 1:
                 dist.all_gather_into_tensor(gathered, local, group=self.group)
