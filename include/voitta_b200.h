@@ -202,7 +202,9 @@ int vb_search_dev(vb_index* h, const vb_query_batch* q, const float* dense_dev, 
  * "seg_first", "seg_ratio", "safe_mode", "profile" (per-phase CUDA-event times in vb_stats),
  * "stream" (a cudaStream_t to run on instead of the index's own stream; 0 restores it),
  * "dense_compact" (row selection for the tensor-core kernels under a batch-wide filter: -1 auto, 0 off,
- * 1..100 = walk the compacted copy when at most that % of a segment passes), "dense_compact_min_rows".
+ * 1..100 = walk the compacted copy when at most that % of a segment passes), "dense_compact_min_rows",
+ * "sel_reuse" (1, the default: keep that copy across batches while the filter, the index and the plan stay the same;
+ * 0: copy it every batch).
  * The full list with defaults is vb_set_option in csrc/vb_api.cu; unknown keys are an error. */
 int vb_set_option(vb_index* h, const char* key, int64_t value);
 

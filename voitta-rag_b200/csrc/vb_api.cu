@@ -16,6 +16,7 @@
 #include <unistd.h>
 
 #include <algorithm>
+#include <array>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -86,6 +87,7 @@ struct Batch {
     uint64_t gen = 0;                          // write generation of the index when the batch was staged
     uint32_t seg_ratio = 32;                   // growth factor of the segment schedule for this batch
     std::vector<int32_t> mode, mask_of_host;
+    std::vector<uint64_t> sel_filter;          // every query on one filter: its content as the mask kernel sees it (else empty)
     // device pointers into h->args
     const float* d_q = nullptr;
     const int64_t* d_qindptr = nullptr;
@@ -173,6 +175,11 @@ struct vb_index {
     DevBuf args, mask, cand, lists, offs, plan, out, q_hat, q_bf16, q_scale, tmp;
     DevBuf sel_rows, sel_inv, sel_ids, sel_meta;   // K2T row selection (dense_compact.cuh): compacted copy, its inverse norms / row ids, {count, decision, block sums}
     bool sel_no_memory = false;               // the scratch matrix did not fit once: do not try again
+    // What the row-selection scratch holds (run_branches): the copy depends only on the batch-wide filter's content, the
+    // rows / inverse norms / filter columns / alive bits (versioned by write_gen) and the plan, never on the queries.  A
+    // batch whose key equals it skips the copy of every segment listed in sel_segs.  Empty sel_key = nothing valid.
+    std::vector<uint64_t> sel_key;
+    std::vector<std::array<uint64_t, 5>> sel_segs;   // {r0, r1, row_off, meta_off, cap_rows} of every valid segment
     DevBuf ms_rec, ms_q, ms_units, ms_counters, mh_units;  // K3M / K3H: plan output, work-unit prefixes, counters
     HostBuf h_args_s[2], h_out_s[2], h_stage, h_sel[2];
     bool sel_ran[2] = {false, false};         // the row selection ran for the batch staged in this slot
@@ -193,6 +200,7 @@ struct vb_index {
     int64_t opt_dense_compact_min_rows = 1 << 18;   // ... on segments of at least this many rows (tests lower it)
     int64_t opt_sel_ctas = 4;              // row selection: CTAs per SM of the copy kernel (1..8 measured at cfg4: 15.1-15.4 ms per batch, no trend)
     int64_t opt_dense_wait_sparse = 0;     // 1: the large tensor-core segments start after the K3M stages (no co-running with the sparse chain)
+    int64_t opt_sel_reuse = 1;             // row selection: 1 = keep the copy across batches while its key holds, 0 = copy every batch
     int64_t opt_dense_compact = -1;        // K2 / K2T: walk a compacted copy of the passing rows when a batch-wide filter passes at most this % of a
                                            // segment (0 = never, -1 = auto: where the copy costs less than the passes over the dropped rows)
     int64_t opt_ms_ctas = 0;               // K3M: resident CTAs per SM of the persistent score kernel (0 = auto, see ms_launch)
@@ -432,6 +440,7 @@ extern "C" int vb_set_option(vb_index* h, const char* key, int64_t value) {
     else if (k == "sel_ctas") h->opt_sel_ctas = value;
     else if (k == "dense_wait_sparse") h->opt_dense_wait_sparse = value;
     else if (k == "dense_compact") h->opt_dense_compact = value;   // row selection threshold in % of the segment's rows (0 = off, -1 = auto)
+    else if (k == "sel_reuse") h->opt_sel_reuse = value;           // 0: copy the passing rows every batch (A/B runs, tests)
     else if (k == "ms_ctas") h->opt_ms_ctas = value;               // K3M: CTAs per SM of the score kernel (0 = auto)
     else if (k == "k2t_stages") g_k2t_stages = (int)value;         // K2T: TMA ring depth (0 = default 4); process-wide
     else if (k == "ms_long_terms") h->opt_ms_long_terms = value;   // K3M: queries above this many terms use ms_budget_long
@@ -443,6 +452,7 @@ extern "C" int vb_set_option(vb_index* h, const char* key, int64_t value) {
     else if (k == "k2_precision") h->opt_k2_precision = value;   // 0 auto, 1 bf16 query, 2 bf16x2 (hi+lo) query
     else if (k == "stream") {   // run on the caller's stream (e.g. torch's current stream); 0 = own stream
         h->stream = value ? reinterpret_cast<cudaStream_t>(static_cast<uintptr_t>(value)) : h->own_stream;
+        h->sel_key.clear();     // a kept row selection is ordered on the old stream only: copy again on the new one
     }
     else return vb_fail("vb_set_option: unknown key '%s'", key);
     return 0;
@@ -701,12 +711,12 @@ extern "C" int vb_delete_rows(vb_index* h, uint64_t n, const uint64_t* rows) {
         if (w & (1u << (r & 31u))) { w &= ~(1u << (r & 31u)); ++killed; touched.push_back((uint32_t)(r >> 5)); dead.push_back((uint32_t)r); }
     }
     if (!killed) return 0;
+    ++h->write_gen;                        // before the upload: a failed one must not leave a kept row selection valid
     // one ranged upload of the touched bitmap words (a folder delete touches tens of thousands of them)
     const uint32_t w_lo = *std::min_element(touched.begin(), touched.end()), w_hi = *std::max_element(touched.begin(), touched.end());
     CK(cudaMemcpyAsync(h->alive.as<uint32_t>() + w_lo, &h->alive_host[w_lo], (size_t)(w_hi - w_lo + 1) * 4, cudaMemcpyHostToDevice, h->stream));
     CK(cudaStreamSynchronize(h->stream));
     h->n_live -= killed;
-    ++h->write_gen;
     if (h->sparse_dirty) return 0;
     // Incremental path: the postings of the dead rows stay in the index (the alive bits mask them); only the live
     // document frequencies change.  Large deletes, or too many dead postings, fall back to a rebuild.
@@ -1228,6 +1238,14 @@ static int prepare_batch(vb_index* h, const vb_query_batch* q, Batch& b, bool ne
     }
     b.use_mask = any_filter && need_corpus;
     b.mask_of_host = mask_of;
+    if (b.use_mask && mask_of[0] >= 0 && std::all_of(mask_of.begin(), mask_of.end(), [&](int32_t f) { return f == mask_of[0]; })) {
+        // the row selection's cache key: equal for content-equal filters (the normalisation of filter_key)
+        const FilterKey fk = filter_key(&flt[mask_of[0]]);
+        const vb_filter& x = *fk.f;
+        const bool ts = x.ts_field != VB_TS_NONE;
+        b.sel_filter = {x.scope_bits != nullptr, (uint64_t)(uint32_t)x.ts_field, ts ? (uint64_t)x.ts_lo : 0u, ts ? (uint64_t)x.ts_hi : 0u};
+        b.sel_filter.insert(b.sel_filter.end(), x.scope_bits, x.scope_bits + fk.words);
+    }
     b.n_filters = b.use_mask ? (uint32_t)flt.size() : 0;
     b.mask_words = (uint32_t)((h->n_rows + 31) / 32);
     b.n_blocks = (uint32_t)((h->base_rows + VB_ROWS_PER_BLOCK - 1) / VB_ROWS_PER_BLOCK);   // row blocks of the inverted index
@@ -1567,9 +1585,12 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
     // segment of at least dense_compact_min_rows rows.  Count, list and copy run on a side stream right after the mask
     // kernel: the copy of segment s + 1 (HBM-bound) hides behind the GEMM of segment s (tensor-bound).  With the chains
     // serialised (overlap = 0: per-phase timing) they run inline on the dense stream and are charged to the dense phase.
-    struct SelSeg { bool on = false; uint32_t cap_rows = 0, n_blocks = 0, ev = 0; size_t row_off = 0, meta_off = 0; };
+    // The copy is kept across batches (h->sel_key): a segment whose key matches the scratch is not copied again, and
+    // the tensor-core kernel reads the scratch and its device-side {count, decision} as they are.
+    struct SelSeg { bool on = false, kept = false; uint32_t cap_rows = 0, n_blocks = 0, ev = 0; size_t row_off = 0, meta_off = 0; };
     std::vector<SelSeg> selseg(bounds.size() - 1);
-    bool sel_any = false;
+    bool sel_any = false, sel_copy = false;
+    std::vector<uint64_t> sel_key;
     const bool sel_side = h->opt_overlap != 0;
     // auto threshold: the copy costs ~0.49 ns per passing row (read + write of 2 * d_pad bytes at HBM speed, d_pad = 768);
     // one pass of the tensor-core kernel over a row costs max(0.245 ns (HBM), 1.08 ns * queries / 1024 (tensor pipe)) — both
@@ -1600,15 +1621,34 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
             if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess || free_b + h->sel_rows.cap < scratch + (4ull << 30)) {
                 cudaGetLastError();
                 h->sel_no_memory = true;                         // the scratch matrix does not fit beside the shard: stay in place
+                h->sel_key.clear();
                 n_on = 0;
             }
         }
         if (n_on) {
+            const void* before[4] = {h->sel_rows.p, h->sel_inv.p, h->sel_ids.p, h->sel_meta.p};
+            // Invalid from here until this batch has enqueued all of its work (end of run_branches): an error return
+            // in between (a failed reserve, a copy enqueued in part) leaves the next batch to copy again.
+            std::vector<uint64_t> cached_key;
+            cached_key.swap(h->sel_key);
             TRY(dev_reserve(h, h->sel_rows, scratch, false));
             TRY(dev_reserve(h, h->sel_inv, rows_total * 4, false));
             TRY(dev_reserve(h, h->sel_ids, rows_total * 4, false));
             TRY(dev_reserve(h, h->sel_meta, meta_total * 4, false));
+            const bool moved = before[0] != h->sel_rows.p || before[1] != h->sel_inv.p || before[2] != h->sel_ids.p || before[3] != h->sel_meta.p;
             sel_any = true;
+            // the key: filter content, index version, and every input of the plan above
+            sel_key = b.sel_filter;
+            sel_key.insert(sel_key.end(), {h->write_gen, (uint64_t)n, (uint64_t)h->d_pad, sel_pct, (uint64_t)h->opt_dense_compact_min_rows,
+                                           (uint64_t)path, (uint64_t)tiled, direct_rows});
+            const bool key_holds = h->opt_sel_reuse && !moved && sel_key == cached_key;
+            for (size_t si = 0; si < selseg.size(); ++si) {
+                SelSeg& z = selseg[si];
+                if (!z.on) continue;
+                const std::array<uint64_t, 5> zk{bounds[si], bounds[si + 1], z.row_off, z.meta_off, z.cap_rows};
+                z.kept = key_holds && std::find(h->sel_segs.begin(), h->sel_segs.end(), zk) != h->sel_segs.end();
+                sel_copy |= !z.kept;
+            }
         } else for (auto& z : selseg) z.on = false;
     }
     auto sel_launch = [&](size_t si, cudaStream_t st) -> int {
@@ -1630,7 +1670,12 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
         h->stats.last_launches += 3;
         return 0;
     };
-    if (sel_any && sel_side) {
+    // Ordering of the scratch (two batches can be in flight).  A kept segment is only read, by kernels on the dense
+    // stream.  A copy waits for ev_sel_fork, recorded on the dense stream after this batch's mask kernel and therefore
+    // after every kernel an earlier batch enqueued there, so it cannot overwrite the scratch while an earlier batch's
+    // tensor-core kernel still reads it — whether that batch copied or kept.  A batch that keeps a copy made by an earlier
+    // one reads it after that batch's dense kernels, which waited for the copy's events: the copy has finished.
+    if (sel_copy && sel_side) {
         if (!h->sel_stream) {
             CK(cudaStreamCreateWithFlags(&h->sel_stream, cudaStreamNonBlocking));
             CK(cudaEventCreateWithFlags(&h->ev_sel_fork, cudaEventDisableTiming));
@@ -1639,7 +1684,7 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
         CK(cudaEventRecord(h->ev_sel_fork, sd));                 // after the mask kernel (and after the previous batch's dense chain)
         CK(cudaStreamWaitEvent(h->sel_stream, h->ev_sel_fork, 0));
         for (size_t si = 0; si < selseg.size(); ++si)
-            if (selseg[si].on) {
+            if (selseg[si].on && !selseg[si].kept) {
                 TRY(sel_launch(si, h->sel_stream));
                 CK(cudaEventRecord(h->ev_sel[selseg[si].ev], h->sel_stream));
             }
@@ -1679,16 +1724,16 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
     };
     auto dense_segment = [&](uint32_t r0, uint32_t r1, uint32_t direct, bool big) -> int {
         if (k1f) return 0;                                      // the single pass covers every segment
-        // Row selection (planned before the segment loop): wait for this segment's copy (side stream), or run the
-        // selection here (chains serialised: its own timed region of the dense phase, so that the PH_BIG region
-        // stays the tensor-core kernel alone)
+        // Row selection (planned before the segment loop): nothing to do when the scratch kept this segment's copy;
+        // otherwise wait for its copy (side stream), or run the selection here (chains serialised: its own timed region
+        // of the dense phase, so that the PH_BIG region stays the tensor-core kernel alone)
         const SelSeg* zsel = nullptr;
         if (path == 2)
             for (size_t si = 0; si + 1 < bounds.size(); ++si)
                 if (bounds[si] == r0 && selseg[si].on) {
                     zsel = &selseg[si];
-                    if (sel_side) CK(cudaStreamWaitEvent(sd, h->ev_sel[zsel->ev], 0));
-                    else {
+                    if (!zsel->kept && sel_side) CK(cudaStreamWaitEvent(sd, h->ev_sel[zsel->ev], 0));
+                    else if (!zsel->kept) {
                         const int pz = prof_begin(h, PH_DENSE, sd);
                         TRY(sel_launch(si, sd));
                         prof_end(h, pz, sd);
@@ -1953,6 +1998,12 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
     if (two_streams) {
         CK(cudaEventRecord(h->ev_join, ss));
         CK(cudaStreamWaitEvent(sd, h->ev_join, 0));
+    }
+    if (sel_any) {                                              // every selected segment is in the scratch now
+        h->sel_segs.clear();
+        for (size_t si = 0; si < selseg.size(); ++si)
+            if (selseg[si].on) h->sel_segs.push_back({bounds[si], bounds[si + 1], selseg[si].row_off, selseg[si].meta_off, selseg[si].cap_rows});
+        h->sel_key = std::move(sel_key);
     }
     return 0;
 }
