@@ -205,7 +205,8 @@ int vb_search_dev(vb_index* h, const vb_query_batch* q, const float* dense_dev, 
  * 1..100 = walk the compacted copy when at most that % of a segment passes), "dense_compact_min_rows",
  * "sel_reuse" (1, the default: keep that copy across batches while the filter, the index and the plan stay the same;
  * 0: copy it every batch).
- * The full list with defaults is vb_set_option in csrc/vb_api.cu; unknown keys are an error. */
+ * The full list with defaults is vb_set_option in csrc/vb_api.cu; unknown keys are an error.  Options belong to one
+ * index, and every index starts at the defaults: the process environment does not change them. */
 int vb_set_option(vb_index* h, const char* key, int64_t value);
 
 int vb_get_stats(vb_index* h, vb_stats* out);

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """A/B runs of index options on ONE resident shard (building a 12.5M-row shard costs more GPU time than timing it).
 
-    python tools/ab_opts.py --workload cfg4 --set "" --set "ms_ctas=6,k2t_stages=3" --set "ms_ctas=4"
+    python tools/ab_opts.py --workload cfg4 --set "" --set "seg_ratio=8,ms_chunk=1024" --set "dense_compact=0"
 
 Per option set: the options are applied on top of the DEFAULTS given by --base (every key named in any set is reset
 to its --base value first), 3 warm-up batches, then --batches batches timed with CUDA events on the launching
@@ -33,7 +33,7 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--workload", default="cfg4", choices=sorted(bench.WORKLOADS))
     ap.add_argument("--set", action="append", default=[], help="comma-separated key=value list; repeatable")
-    ap.add_argument("--base", default="", help="values the keys fall back to between sets, e.g. ms_ctas=0,k2t_stages=0")
+    ap.add_argument("--base", default="", help="values the keys fall back to between sets, e.g. seg_ratio=0,ms_chunk=0")
     ap.add_argument("--batches", type=int, default=10)
     ap.add_argument("--out", default=None)
     args = ap.parse_args()

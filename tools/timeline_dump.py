@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Print the CUDA-event timeline (every timed region, per stream) of one batch of a bench workload on a resident shard:
-python tools/timeline_dump.py --workload cfg4 --set dense_wait_sparse=1"""
+python tools/timeline_dump.py --workload cfg4 --set seg_ratio=8"""
 import argparse, json, sys
 from pathlib import Path
 ROOT = Path(__file__).resolve().parents[1]

@@ -42,15 +42,6 @@ def build_debug() -> Path:
     return LIB_DEBUG
 
 
-def build_variant(name: str, *defines: str) -> Path:
-    """A/B builds (tools/gpu_r2_m.sh): the library with extra -D flags as libvoitta_b200_<name>.so; select with VB200_LIB."""
-    out = HERE / f"libvoitta_b200_{name}.so"
-    r = subprocess.run([nvcc_path(), *FLAGS, *[f"-D{d}" for d in defines], "-o", str(out), str(SRC)], capture_output=True, text=True)
-    if r.returncode != 0:
-        raise RuntimeError(f"nvcc failed:\n{r.stdout}\n{r.stderr}")
-    return out
-
-
 def build(force: bool = False, verbose: bool = False, debug: bool = True) -> Path:
     """Release library and (debug=True) the bounds-checked one, each only when older than its sources; the two nvcc
     runs go side by side.  A stale debug library once made tools/gpu_sanitize.sh test yesterday's kernels."""

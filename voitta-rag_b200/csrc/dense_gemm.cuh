@@ -20,7 +20,6 @@
 #include "common.cuh"
 #include <cuda.h>
 #include <string>
-#include <cstdlib>
 #include <algorithm>
 
 #define VB_GEMM_THREADS 320          // warp 0 TMA, warp 1 MMA, warps 2-9 epilogue (two per TMEM lane quadrant)
@@ -168,7 +167,6 @@ struct VbGemmArgs {
     int32_t  uniform_filter;         // mask_mode 1: the filter index
     uint32_t split;                  // 1: columns [0,bn/2) hold q_hi, [bn/2,bn) hold q_lo (bf16x2 query precision)
     uint32_t kbox;                   // K-blocks (of 64) per TMA box / pipeline stage
-    uint32_t debug;                  // perf triage only (VB200_K2_DEBUG): 1 skip epilogue math, 2 skip MMA, 4 skip TMA
     // SEL (dense_compact.cuh): sel[1] != 0 -> walk the compacted copy of the rows that pass the shared filter instead
     const uint32_t* sel;             // [0] rows of the copy, [1] decision (taken on the device)
     const uint32_t* sel_ids;         // [rows of the copy] shard row id of each copied row
@@ -249,12 +247,9 @@ vb_dense_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_co
                 const int32_t row0 = (int32_t)((tile_begin + t) * VB_TILE_M);
                 for (uint32_t kb = 0; kb < a.k_blocks; kb += a.kbox) {
                     vb_mbar_wait(bar_empty + 8u * stage, phase ^ 1u);
-                    if (a.debug & 4u) { vb_mbar_arrive(bar_full + 8u * stage); }
-                    else {
                     vb_mbar_expect_tx(bar_full + 8u * stage, stage_bytes);
                     // one box = 128 rows x kbox K-blocks: [kb][row][64] in smem, i.e. kbox UMMA slabs
                     vb_tma_load_3d(vb_smem_u32(smem_a + stage * stage_bytes), tmap_rows, 0, row0, (int32_t)kb, bar_full + 8u * stage);
-                    }
                     if (++stage == S) { stage = 0; phase ^= 1u; }
                 }
             }
@@ -274,7 +269,7 @@ vb_dense_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_co
                     vb_mbar_wait(bar_full + 8u * stage, phase);
                     vb_tcgen05_fence_after();
                     const uint32_t nkb = min(a.kbox, a.k_blocks - kb0);
-                    for (uint32_t kk = 0; kk < nkb && !(a.debug & 2u); ++kk) {
+                    for (uint32_t kk = 0; kk < nkb; ++kk) {
                         const uint32_t kb = kb0 + kk;
                         const uint32_t a_addr = vb_smem_u32(smem_a + stage * stage_bytes + kk * VB_STAGE_BYTES);
                         const uint32_t q_addr = vb_smem_u32(smem_q + kb * a.bn * 128u);
@@ -334,7 +329,6 @@ vb_dense_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_co
             const uint32_t slot = row - a.tile_begin * VB_TILE_M;      // direct mode: position inside the segment
             // one 16-column chunk: compare, then (rarely) append — or, in direct mode, store all
             auto process = [&](const uint32_t (&v)[16], const uint32_t (&w)[16], uint32_t c0) {
-                if (a.debug & 8u) return;
                 uint32_t m = 0;
 #pragma unroll
                 for (uint32_t j4 = 0; j4 < 4u; ++j4) {
@@ -387,14 +381,13 @@ vb_dense_gemm_kernel(const __grid_constant__ CUtensorMap tmap_a, const __grid_co
             };
             uint32_t va[16], vb[16], wa[16], wb[16];
             auto load = [&](uint32_t (&v)[16], uint32_t (&w)[16], uint32_t c0) {
-                if (a.debug & 16u) return;
                 vb_tmem_ld16(taddr + c0, v);
                 if (split) vb_tmem_ld16(taddr + ncol + c0, w);
             };
             // this warp's chunks: 16*(2i + half); the next one is in flight while one is processed
             const uint32_t first = 16u * half;
-            if (first < ncol && !(a.debug & 1u)) load(va, wa, first);
-            for (uint32_t c0 = first; c0 < ncol && !(a.debug & 1u); c0 += 64u) {
+            if (first < ncol) load(va, wa, first);
+            for (uint32_t c0 = first; c0 < ncol; c0 += 64u) {
                 vb_tmem_ld_wait();
                 const bool second = c0 + 32u < ncol;
                 if (second) load(vb, wb, c0 + 32u);
@@ -648,11 +641,7 @@ vb_dense_gemm_tiled_kernel(const __grid_constant__ CUtensorMap tmap_a, const __g
                         // rare path (see the resident kernel): a COMPACT loop over the flagged columns
                         const uint32_t mm = __reduce_or_sync(0xffffffffu, m);
                         if (mm != 0u)
-#ifdef VB_K2T_DIRECT_APPEND
-                            vb_append_flagged(a.lists, a.q_begin + qoff + c0, sub, mm, m, lane, lane_lt, a.row_base + row,
-#else
                             pn = vb_park_flagged(a.lists, a.q_begin + qoff + c0, sub, mm, m, lane_lt, a.row_base + row, pk_addr, pl_addr, pn, lane,
-#endif
                                               [&](uint32_t jj) -> float { return __uint_as_float(vb_sel16(v, jj)) * invn * __uint_as_float(vb_lds_u32(qs_addr + (qoff + c0 + jj) * 4u)); },
                                               [&](uint32_t jj, float fs) -> bool { return fs > __uint_as_float(vb_lds_u32(tex_addr + (qoff + c0 + jj) * 4u)); });
                     }
@@ -738,26 +727,16 @@ static int vb_gemm_configure() {
 }
 
 static const uint32_t VB_GEMM_TAIL_BYTES = 320u + 4u * 256u * 4u + 8u * VB_GEMM_MAX_FILTERS * 4u;
+static const uint32_t VB_K2_KBOX = 3u;         // K-blocks per TMA box of the resident kernel (pipeline stage granularity)
+static const uint32_t VB_K2_MAX_STAGES = 12u;  // ring depth cap of the resident kernel
+static const uint32_t VB_K2T_STAGES = 4u;      // ring depth of K2T (3 measured no faster, DESIGN §Scheduling)
 
-// largest padded sub-batch whose resident query matrix leaves room for >= 4 stages
-static int vb_env_int(const char* name, int dflt) {
-    const char* e = getenv(name);
-    return e ? atoi(e) : dflt;
-}
 // K-blocks per TMA box (pipeline stage granularity)
 static uint32_t vb_gemm_kbox(uint32_t d_pad) {
     const uint32_t k_blocks = d_pad / VB_BLOCK_K;
-    uint32_t kbox = (uint32_t)vb_env_int("VB200_K2_KBOX", 3);
-    if (kbox < 1u) kbox = 1u;
-    return kbox > k_blocks ? k_blocks : kbox;
+    return VB_K2_KBOX > k_blocks ? k_blocks : VB_K2_KBOX;
 }
-// shared-memory budget of the resident kernel: the device maximum, or VB200_K2_SMEM_KB (leaves room for CTAs of
-// the sparse chain to be co-resident with the persistent GEMM CTA)
-static uint32_t vb_gemm_smem_budget() {
-    const int kb = vb_env_int("VB200_K2_SMEM_KB", 0);
-    const uint32_t mx = (uint32_t)g_gemm_smem_max;
-    return kb > 0 ? std::min<uint32_t>(mx, (uint32_t)kb * 1024u) : mx;
-}
+// largest padded sub-batch whose resident query matrix leaves room for >= 4 stages
 static uint32_t vb_gemm_max_bn(uint32_t d_pad) {
     const uint32_t reserve = std::max(4u, 2u * vb_gemm_kbox(d_pad)) * VB_STAGE_BYTES;   // room for the A ring
     const uint32_t avail = (uint32_t)g_gemm_smem_max - 1024u - VB_GEMM_TAIL_BYTES - reserve;
@@ -774,8 +753,7 @@ static VbGemmPlan vb_gemm_plan(uint32_t d_pad, uint32_t B, int precision /*0 aut
     const uint32_t bn_max = vb_gemm_max_bn(d_pad);
     const uint32_t half = (bn_max / 2u) / 16u * 16u;
     VbGemmPlan p;
-    const uint32_t split_max = (uint32_t)vb_env_int("VB200_K2_SPLIT_MAX_B", 1 << 20);
-    p.split = precision == 2 ? 1u : (precision == 1 ? 0u : ((B <= half && B <= split_max) ? 1u : 0u));
+    p.split = precision == 2 ? 1u : (precision == 1 ? 0u : (B <= half ? 1u : 0u));
     if (p.split && half < 16u) p.split = 0u;
     p.sub = p.split ? half : bn_max;
     return p;
@@ -825,14 +803,13 @@ static int vb_encode_2d(CUtensorMap* map, const void* base, uint64_t rows, uint6
 
 // A operand as a 3-D tensor [k_block][row][64]: one TMA box brings `kbox` K-blocks of 128 rows,
 // landing as kbox consecutive [128 rows x 128 B] swizzled slabs (what the UMMA descriptors expect).
-static int vb_encode_a3d(CUtensorMap* map, const void* base, uint64_t rows, uint64_t d_pad, uint32_t kbox, int promo) {
+static int vb_encode_a3d(CUtensorMap* map, const void* base, uint64_t rows, uint64_t d_pad, uint32_t kbox) {
     cuuint64_t dims[3] = {VB_BLOCK_K, rows, d_pad / VB_BLOCK_K};
     cuuint64_t strides[2] = {d_pad * 2, VB_BLOCK_K * 2};
     cuuint32_t box[3] = {VB_BLOCK_K, VB_TILE_M, kbox};
     cuuint32_t estr[3] = {1, 1, 1};
     CUresult r = g_encode_tiled(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), dims, strides, box, estr,
-                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                promo == 2 ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B : (promo == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : CU_TENSOR_MAP_L2_PROMOTION_L2_128B),
+                                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                                 CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { g_gemm_err = "cuTensorMapEncodeTiled(3d) failed (" + std::to_string((int)r) + ")"; return 1; }
     return 0;
@@ -846,9 +823,9 @@ static int vb_gemm_launch(const VbGemmLaunch& g, int* launches) {
     const uint32_t kbox = vb_gemm_kbox(g.d_pad);
     (void)k_blocks;
     CUtensorMap tmap_a;
-    if (vb_encode_a3d(&tmap_a, g.rows, g.n_rows_total, g.d_pad, kbox, vb_env_int("VB200_K2_L2PROMO", 1))) return 1;
+    if (vb_encode_a3d(&tmap_a, g.rows, g.n_rows_total, g.d_pad, kbox)) return 1;
     CUtensorMap tmap_c = tmap_a;
-    if (g.sel && vb_encode_a3d(&tmap_c, g.sel_rows, g.sel_cap_rows, g.d_pad, kbox, vb_env_int("VB200_K2_L2PROMO", 1))) return 1;
+    if (g.sel && vb_encode_a3d(&tmap_c, g.sel_rows, g.sel_cap_rows, g.d_pad, kbox)) return 1;
     for (uint32_t q0 = 0; q0 < g.n_queries; q0 += sub) {
         const uint32_t n_q = std::min(sub, g.n_queries - q0);
         const uint32_t bn = (n_q + 15u) / 16u * 16u * mult;
@@ -875,11 +852,8 @@ static int vb_gemm_launch(const VbGemmLaunch& g, int* launches) {
         }
         const uint32_t q_bytes = bn * g.d_pad * 2u;
         a.kbox = kbox;
-        a.debug = (uint32_t)vb_env_int("VB200_K2_DEBUG", 0);
-        const uint32_t budget = std::max<uint32_t>(vb_gemm_smem_budget(), 1024u + VB_GEMM_TAIL_BYTES + q_bytes + 2u * kbox * VB_STAGE_BYTES);
-        uint32_t stages = (std::min<uint32_t>(budget, (uint32_t)g_gemm_smem_max) - 1024u - VB_GEMM_TAIL_BYTES - q_bytes) / (kbox * VB_STAGE_BYTES);
-        const uint32_t cap_stages = (uint32_t)vb_env_int("VB200_K2_STAGES", 12);
-        a.stages = stages > cap_stages ? cap_stages : stages;
+        const uint32_t stages = ((uint32_t)g_gemm_smem_max - 1024u - VB_GEMM_TAIL_BYTES - q_bytes) / (kbox * VB_STAGE_BYTES);
+        a.stages = stages > VB_K2_MAX_STAGES ? VB_K2_MAX_STAGES : stages;
         if (a.stages < 2u) { g_gemm_err = "not enough shared memory for a 2-stage pipeline"; return 1; }
         const size_t smem = 1024u + q_bytes + a.stages * kbox * VB_STAGE_BYTES + VB_GEMM_TAIL_BYTES;
         const uint32_t tiles = a.tile_end - a.tile_begin;
@@ -900,12 +874,10 @@ static int vb_gemm_launch(const VbGemmLaunch& g, int* launches) {
 // ---- K2T launcher -------------------------------------------------------------------------------------
 static const uint32_t VB_TILED_TAIL_BYTES = 320u + VB_TILED_MAX_Q * 16u + 8u * VB_GEMM_MAX_FILTERS * 4u + 8u * VB_PEND * 12u;
 
-static int g_k2t_stages = 0;           // vb_set_option("k2t_stages"): 0 = VB200_K2T_STAGES or 4 (process-wide)
 static uint32_t vb_gemm_tiled_stages() {
     const uint32_t avail = (uint32_t)g_gemm_smem_max - 1024u - VB_TILED_TAIL_BYTES;
-    uint32_t st = avail / VB_TILED_STAGE_BYTES;
-    const uint32_t cap = g_k2t_stages > 0 ? (uint32_t)g_k2t_stages : (uint32_t)vb_env_int("VB200_K2T_STAGES", 4);
-    return st > cap ? cap : st;
+    const uint32_t st = avail / VB_TILED_STAGE_BYTES;
+    return st > VB_K2T_STAGES ? VB_K2T_STAGES : st;
 }
 static bool vb_gemm_tiled_supported(int d_pad) {
     return g_encode_tiled != nullptr && d_pad % 64 == 0 && vb_gemm_tiled_stages() >= 2u;

@@ -226,15 +226,10 @@ __device__ __noinline__ void vb_k1f_sort(uint64_t* s, uint32_t P) {
     __syncthreads();
 }
 
-// A/B builds: -DVB_K1F_MINBLOCKS=5 / 6 / 8 ask the compiler for that many resident CTAs per SM (fewer registers, spills);
-// the default passes no such bound — an explicit 1 lets ptxas take 89-138 registers instead of 62-79
-#ifdef VB_K1F_MINBLOCKS
-#define VB_K1F_BOUNDS __launch_bounds__(VB_K1F_THREADS, VB_K1F_MINBLOCKS)
-#else
-#define VB_K1F_BOUNDS __launch_bounds__(VB_K1F_THREADS)
-#endif
+// No minimum-CTAs bound: an explicit 1 lets ptxas take 89-138 registers instead of 62-79, and 5 / 6 / 8 (fewer
+// registers, spills) measured slower (DESIGN §K1F)
 template <int NCH>
-__global__ void VB_K1F_BOUNDS
+__global__ void __launch_bounds__(VB_K1F_THREADS)
 vb_dense_scan1_kernel(const VbScan1Args a)
 {
     constexpr int ROWS = 4;

@@ -114,7 +114,6 @@ struct VbSparseArgs {
     uint32_t direct;            // 1: first segment — store keys at slot (row - segment begin), no atomics
     const uint32_t* q_sel;      // [n_sel] queries this launch scores (the rest go to K3M, sparse_ms.cuh); nullptr = all
     uint32_t n_sel;
-    uint32_t debug;             // perf triage only (VB200_SPARSE_DEBUG): 1 stop after the term table, 2 skip the posting scatter, 4 skip the scan, 8 skip the accumulator init
 };
 
 // ---- MaxScore plan: which query terms are essential under the current thresholds --------------------
@@ -240,11 +239,9 @@ vb_sparse_kernel(const VbSparseArgs a)
         if (f >= 0) mask = a.mask + (size_t)f * a.mask_words;
     }
     const double neg_zero = __longlong_as_double((long long)VB_ACC_SENTINEL);
-    if (!(a.debug & 8u)) {
 #pragma unroll
-        for (uint32_t r = 2u * tid; r < VB_ROWS_PER_BLOCK + VB_SPARSE_PAD; r += 2u * VB_SPARSE_THREADS)
-            *reinterpret_cast<double2*>(&acc[r]) = make_double2(neg_zero, neg_zero);
-    }
+    for (uint32_t r = 2u * tid; r < VB_ROWS_PER_BLOCK + VB_SPARSE_PAD; r += 2u * VB_SPARSE_THREADS)
+        *reinterpret_cast<double2*>(&acc[r]) = make_double2(neg_zero, neg_zero);
     uint32_t nnz = 0, n_all = 0, nh = 0;                        // essential terms with postings here / terms that can touch
     {                                                           // this block / essential terms read from a dense column
         uint32_t cum_base = 0;
@@ -277,8 +274,7 @@ vb_sparse_kernel(const VbSparseArgs a)
         }
     }
     __syncthreads();
-    if ((nnz == 0 && nh == 0) || (a.debug & 1u)) return;
-    if (a.debug & 2u) nnz = 0;                            // no row of this block can beat tau (direct-mode slots were zeroed by the host)
+    if (nnz == 0 && nh == 0) return;
 
     const uint32_t row0 = blk * VB_ROWS_PER_BLOCK;
     const uint32_t dummy = VB_ROWS_PER_BLOCK + (tid & 31u);     // this lane's private padding slot
@@ -350,7 +346,6 @@ vb_sparse_kernel(const VbSparseArgs a)
         }
     }
 
-    if (a.debug & 4u) return;
     const uint32_t seg_row0 = a.blk_begin * VB_ROWS_PER_BLOCK;
     const uint32_t sub = blk_rel & a.lists.sub_mask;            // append counter of this row block
     const double tau_d = (double)tau;
@@ -414,7 +409,7 @@ vb_sparse_kernel(const VbSparseArgs a)
 #pragma unroll
         for (uint32_t g = 0; g < 4u; ++g) {
             const uint32_t r = 4u * tid + g * 4u * VB_SPARSE_THREADS;
-            in[g] = row0 + r < a.n_rows && !(a.debug & 32u);
+            in[g] = row0 + r < a.n_rows;
             s32[g][0] = s32[g][1] = s32[g][2] = s32[g][3] = 0.0f;
             if (has_acc) {
                 const double2 c01 = *reinterpret_cast<const double2*>(&acc[r]), c23 = *reinterpret_cast<const double2*>(&acc[r + 2u]);

@@ -140,7 +140,7 @@ struct vb_index {
     cudaStream_t stream = nullptr, own_stream = nullptr, aux_stream = nullptr, sel_stream = nullptr;
     cudaEvent_t ev_sel_fork = nullptr, ev_sel[8] = {};
     cudaEvent_t ev0s[2] = {nullptr, nullptr}, ev1s[2] = {nullptr, nullptr}, ev_done[2] = {nullptr, nullptr};
-    cudaEvent_t ev_fork = nullptr, ev_join = nullptr, ev_sp_done = nullptr;
+    cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     int cur = 0;                               // current slot: two batches can be in flight (pipelined callers)
     std::recursive_mutex mu;               // one-call entry points hold it for the whole call; staged calls re-enter
     int sm_count = 148;
@@ -195,17 +195,11 @@ struct vb_index {
                                            // measured on the cfg5 shard: K3 190 ms, K3H 346-715 ms depending on the budget (sparse_mh.cuh)
     int64_t opt_k1f = 1;                   // single-pass dense scan (K1F) for batches of at most VB_K1F_MAX_B queries
     int64_t opt_ms_staged = 1;             // K3M: 1 = posting stages over the whole index, 0 = once per row segment
-    int64_t opt_ms_stage_ratio = 0;        // K3M: growth of the posting stages (0 = auto: 32, up to 1024 for tiny batches)
     int64_t opt_delta_max = 0;             // rows the delta may hold before vb_upsert merges it into the index (0 = auto)
     int64_t opt_dense_compact_min_rows = 1 << 18;   // ... on segments of at least this many rows (tests lower it)
-    int64_t opt_sel_ctas = 4;              // row selection: CTAs per SM of the copy kernel (1..8 measured at cfg4: 15.1-15.4 ms per batch, no trend)
-    int64_t opt_dense_wait_sparse = 0;     // 1: the large tensor-core segments start after the K3M stages (no co-running with the sparse chain)
     int64_t opt_sel_reuse = 1;             // row selection: 1 = keep the copy across batches while its key holds, 0 = copy every batch
     int64_t opt_dense_compact = -1;        // K2 / K2T: walk a compacted copy of the passing rows when a batch-wide filter passes at most this % of a
                                            // segment (0 = never, -1 = auto: where the copy costs less than the passes over the dropped rows)
-    int64_t opt_ms_ctas = 0;               // K3M: resident CTAs per SM of the persistent score kernel (0 = auto, see ms_launch)
-    int64_t opt_ms_long_terms = 16, opt_ms_budget_long = 85;   // K3M: queries of more terms than the first plan with the second budget
-                                           // (cfg5 shard, 2..65-term queries: 561 ms per batch at 100 %, 154 at 92, 153-156 at 85, 160 at 70, 188 at 40)
     int64_t opt_ms_max_terms = VB_MS_MAX_TERMS;         // K3M scores queries of at most this many terms; longer ones accumulate (K3)
 
     const float* q_dev = nullptr;          // vb_stage_dev / vb_search_dev: dense queries of the batch being staged live on this device
@@ -280,6 +274,12 @@ __global__ void vb_find_tail_kernel(const uint64_t* keys, uint64_t n, uint64_t* 
 
 static int g_delta_smem_max = 48 * 1024;
 
+// K3M queries of more than VB_MS_LONG_TERMS terms are planned with a non-essential budget of VB_MS_BUDGET_LONG % of tau
+// instead of the full MaxScore partition (cfg5 shard, 2..65-term queries: 561 ms per batch at 100 %, 154 at 92,
+// 153-156 at 85, 160 at 70, 188 at 40)
+#define VB_MS_LONG_TERMS 16u
+#define VB_MS_BUDGET_LONG 85u
+
 #define VB_K1F_MAX_B 8u
 // CTAs per query of the single-pass scan: ONE wave of resident CTAs (the register file holds 5 x 256 threads per SM;
 // round 2 launched 8 per SM = 1.6 waves, so the kernel lasted two CTA lifetimes: 52 us for 77 MB at cfg1); fewer for
@@ -351,17 +351,6 @@ extern "C" int vb_create(int32_t dim, int32_t device, uint64_t capacity_hint, ui
     }
     h->stream = h->own_stream;
     if (vb_gemm_configure() != 0) { delete h; return vb_fail("vb_create: tensor-core kernel configuration failed: %s", vb_gemm_last_error()); }
-    if (const char* env = getenv("VB200_SPARSE_CARVEOUT")) {
-        // Experiment: the persistent GEMM CTAs configure their SM for the maximum shared-memory carveout; give the
-        // sparse chain's kernels the same preference so that they can be co-resident without an SM reconfiguration.
-        const int pct = atoi(env);
-        if (pct >= 0) {
-            cudaFuncSetAttribute(vb_ms_score_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-            cudaFuncSetAttribute(vb_ms_plan_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-            cudaFuncSetAttribute(vb_compact_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-            cudaFuncSetAttribute(vb_sparse_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
-        }
-    }
     if (cudaFuncSetAttribute(vb_mh_score_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)vb_mh_smem_bytes(VB_MS_MAX_TERMS)) != cudaSuccess) {
         delete h;
         return vb_fail("vb_create: cannot reserve shared memory for the long-query sparse kernel");
@@ -371,23 +360,6 @@ extern "C" int vb_create(int32_t dim, int32_t device, uint64_t capacity_hint, ui
         if (cudaFuncSetAttribute(vb_sparse_delta_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, want) == cudaSuccess) g_delta_smem_max = want;
     }
     (void)capacity_hint;
-    if (const char* env = getenv("VB200_DENSE_PATH")) h->opt_dense_path = atoi(env);   // 0 auto, 1 K1, 2 K2
-    if (const char* env = getenv("VB200_SEG_FIRST")) h->opt_seg_first = std::max<int64_t>(VB_ROWS_PER_BLOCK, (int64_t)align_up((size_t)atoll(env), VB_ROWS_PER_BLOCK));
-    if (const char* env = getenv("VB200_SEG_RATIO")) h->opt_seg_ratio = std::max<int64_t>(2, atoll(env));   // unset = auto
-    if (const char* env = getenv("VB200_OVERLAP")) h->opt_overlap = atoi(env);
-    if (const char* env = getenv("VB200_SPARSE_PRUNE")) h->opt_sparse_prune = atoi(env);
-    if (const char* env = getenv("VB200_SPARSE_PRUNE_FORCE")) h->opt_sparse_prune_force = atoi(env);
-    if (const char* env = getenv("VB200_SPARSE_DENSE")) h->opt_sparse_dense = atoi(env);
-    if (const char* env = getenv("VB200_SPARSE_MS")) h->opt_sparse_ms = atoi(env);
-    if (const char* env = getenv("VB200_MS_BUDGET")) h->opt_ms_budget = atoi(env);
-    if (const char* env = getenv("VB200_MS_CHUNK")) h->opt_ms_chunk = atoi(env);
-    if (const char* env = getenv("VB200_MS_STAGED")) h->opt_ms_staged = atoi(env);
-    if (const char* env = getenv("VB200_K1F")) h->opt_k1f = atoi(env);
-    if (const char* env = getenv("VB200_SPARSE_MH")) h->opt_sparse_mh = atoi(env);
-    if (const char* env = getenv("VB200_MH_BUDGET")) h->opt_mh_budget = atoi(env);
-    if (const char* env = getenv("VB200_MS_STAGE_RATIO")) h->opt_ms_stage_ratio = atoi(env);
-    if (const char* env = getenv("VB200_MS_MAX_TERMS")) h->opt_ms_max_terms = atoi(env);
-    if (const char* env = getenv("VB200_MS_CTAS")) h->opt_ms_ctas = atoi(env);
     *out = h;
     return 0;
 }
@@ -408,13 +380,13 @@ extern "C" void vb_destroy(vb_index* h) {
     if (h->ev_q) cudaEventDestroy(h->ev_q);
     cudaEventDestroy(h->ev_fork);
     cudaEventDestroy(h->ev_join);
-    if (h->ev_sp_done) cudaEventDestroy(h->ev_sp_done);
     cudaStreamDestroy(h->aux_stream);
     if (h->sel_stream) { cudaStreamDestroy(h->sel_stream); cudaEventDestroy(h->ev_sel_fork); for (auto e : h->ev_sel) cudaEventDestroy(e); }
     cudaStreamDestroy(h->own_stream);
     delete h;
 }
 
+// Every option changes this index only; an index starts at the defaults in vb_index.
 extern "C" int vb_set_option(vb_index* h, const char* key, int64_t value) {
     if (!h || !key) return vb_fail("vb_set_option: NULL argument");
     std::lock_guard<std::recursive_mutex> lk(h->mu);
@@ -434,17 +406,10 @@ extern "C" int vb_set_option(vb_index* h, const char* key, int64_t value) {
     else if (k == "sparse_mh") h->opt_sparse_mh = value;           // 0: long queries stay on K3
     else if (k == "k1f") h->opt_k1f = value;                       // 0: K1 in row segments even for single queries
     else if (k == "ms_staged") h->opt_ms_staged = value;           // K3M: posting stages (1) or row segments (0)
-    else if (k == "ms_stage_ratio") h->opt_ms_stage_ratio = value; // K3M: growth of the posting stages
     else if (k == "delta_max") h->opt_delta_max = value;           // delta rows that trigger a merge (0 = max(16384, base/32))
     else if (k == "dense_compact_min_rows") h->opt_dense_compact_min_rows = value;
-    else if (k == "sel_ctas") h->opt_sel_ctas = value;
-    else if (k == "dense_wait_sparse") h->opt_dense_wait_sparse = value;
     else if (k == "dense_compact") h->opt_dense_compact = value;   // row selection threshold in % of the segment's rows (0 = off, -1 = auto)
     else if (k == "sel_reuse") h->opt_sel_reuse = value;           // 0: copy the passing rows every batch (A/B runs, tests)
-    else if (k == "ms_ctas") h->opt_ms_ctas = value;               // K3M: CTAs per SM of the score kernel (0 = auto)
-    else if (k == "k2t_stages") g_k2t_stages = (int)value;         // K2T: TMA ring depth (0 = default 4); process-wide
-    else if (k == "ms_long_terms") h->opt_ms_long_terms = value;   // K3M: queries above this many terms use ms_budget_long
-    else if (k == "ms_budget_long") h->opt_ms_budget_long = value; // K3M non-essential budget of those queries, % of tau
     else if (k == "ms_max_terms") h->opt_ms_max_terms = value;     // K3M only for queries of at most this many terms
     else if (k == "sparse_prune_force") h->opt_sparse_prune_force = value;   // 1: prune in every non-direct segment (tests)
     else if (k == "sparse_prune") h->opt_sparse_prune = value;     // MaxScore budget in % of tau (0: score every term's postings)
@@ -1663,7 +1628,7 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
         CKK("vb_rowsel_count_kernel");
         vb_rowsel_scatter_kernel<<<z.n_blocks, VB_SEL_THREADS, 0, st>>>(sa);
         CKK("vb_rowsel_scatter_kernel");
-        vb_rowsel_gather_kernel<<<h->sm_count * (int)std::max<int64_t>(1, std::min<int64_t>(8, h->opt_sel_ctas)), 256, 0, st>>>(h->rows.as<uint4>(), h->inv_norm.as<float>(), sa.ids, sa.sel,
+        vb_rowsel_gather_kernel<<<h->sm_count * 4, 256, 0, st>>>(h->rows.as<uint4>(), h->inv_norm.as<float>(), sa.ids, sa.sel,
                                                                 h->sel_rows.as<uint4>() + z.row_off * (h->d_pad / 8), h->sel_inv.as<float>() + z.row_off,
                                                                 (uint32_t)h->d_pad / 8u);
         CKK("vb_rowsel_gather_kernel");
@@ -1689,7 +1654,6 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
                 CK(cudaEventRecord(h->ev_sel[selseg[si].ev], h->sel_stream));
             }
     }
-    bool sp_done_recorded = false;                                // dense_wait_sparse: an event after the K3M stages exists
     auto dense_single_pass = [&]() -> int {
         const int pi = prof_begin(h, PH_DENSE | PH_BIG, sd);
         VbScan1Args a{};
@@ -1744,7 +1708,6 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
                         h->sel_ran[h->cur] = true;
                     }
                 }
-        if (sp_done_recorded && path == 2 && r1 - r0 >= (1u << 20)) CK(cudaStreamWaitEvent(sd, h->ev_sp_done, 0));
         const int pi = prof_begin(h, PH_DENSE | (big ? PH_BIG : 0), sd);
         if (path == 2) {
             VbGemmLaunch g{};
@@ -1777,8 +1740,6 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
     };
     const uint32_t ms_chunk = h->opt_ms_chunk > 0 ? (uint32_t)align_up((size_t)h->opt_ms_chunk, VB_MS_U * VB_MS_THREADS)
                                                    : 512u;
-    // Resident CTAs per SM of the persistent K3M score kernel.  16 (every register of the SM) when it runs alone.
-    const uint32_t ms_per_sm = h->opt_ms_ctas > 0 ? (uint32_t)std::min<int64_t>(16, h->opt_ms_ctas) : 16u;
     // classes: bit 0 = plan + score the K3M queries, bit 1 = the K3H (long) queries
     auto ms_launch = [&](uint32_t r0, uint32_t r1, uint64_t stage_lo, uint64_t stage_hi, uint32_t classes) -> int {
         VbMsPlanArgs pa{};
@@ -1791,8 +1752,7 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
         pa.seg_row0 = r0; pa.seg_row1 = r1; pa.stage_lo = stage_lo; pa.stage_hi = stage_hi;
         pa.chunk = ms_chunk; pa.budget_pct = (uint32_t)std::max<int64_t>(0, h->opt_ms_budget);
         pa.budget_pct_long = (uint32_t)std::max<int64_t>(0, h->opt_mh_budget);
-        pa.long_terms = (uint32_t)std::max<int64_t>(0, h->opt_ms_long_terms);
-        pa.budget_pct_mslong = (uint32_t)std::max<int64_t>(0, h->opt_ms_budget_long);
+        pa.long_terms = VB_MS_LONG_TERMS; pa.budget_pct_mslong = VB_MS_BUDGET_LONG;
         vb_ms_plan_kernel<<<b.B, 256, 0, ss>>>(pa);
         CKK("vb_ms_plan_kernel");
         ++h->stats.last_launches;
@@ -1824,10 +1784,11 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
         a.mask = b.use_mask ? h->mask.as<uint32_t>() : nullptr; a.mask_of = b.use_mask ? b.d_maskof : nullptr;
         a.tau = b.tau; a.lists = L; a.mask_words = b.mask_words; a.n_qterms = b.n_qterms; a.n_queries = b.B;
         a.row_base = (uint32_t)h->row_base; a.chunk = ms_chunk; a.nt_max = b.nt_max;
-        // persistent grid: enough CTAs to fill the machine, never more than the largest possible unit count
+        // persistent grid: enough CTAs to fill the machine (16 per SM: every register of the SM), never more than the
+        // largest possible unit count
         const uint64_t span = std::min<uint64_t>(r1 - r0, stage_hi - stage_lo);
         const uint64_t max_units = std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)h->nnz_live / ms_chunk + b.n_qterms, (uint64_t)b.n_qterms * (span / ms_chunk + 1)));
-        const uint32_t grid = (uint32_t)std::min<uint64_t>((uint64_t)h->sm_count * ms_per_sm, max_units);
+        const uint32_t grid = (uint32_t)std::min<uint64_t>((uint64_t)h->sm_count * 16u, max_units);
         vb_ms_score_kernel<<<grid, VB_MS_THREADS, vb_ms_smem_bytes(b.nt_max), ss>>>(a);
         CKK("vb_ms_score_kernel");
         ++h->stats.last_launches;
@@ -1885,7 +1846,6 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
                 a.row_base = (uint32_t)h->row_base; a.direct = direct;
                 const uint32_t n_q = k3_n;
                 if (k3_list != nullptr) { a.q_sel = k3_list; a.n_sel = k3_n; }          // K3M / K3H have the rest
-                { static const char* dbg = getenv("VB200_SPARSE_DEBUG"); a.debug = dbg ? (uint32_t)atoi(dbg) : 0u; }
                 const uint32_t nblk = (r1 - r0 + VB_ROWS_PER_BLOCK - 1) / VB_ROWS_PER_BLOCK;
                 vb_sparse_kernel<<<nblk * n_q, VB_SPARSE_THREADS, vb_sparse_smem_bytes(b.nt_max), ss>>>(a);
                 CKK("vb_sparse_kernel");
@@ -1937,8 +1897,7 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
             TRY(sparse_compact(L.sub_cap));
             lo = hi;
             // a stage appends ~ratio * k' candidates per list at worst (rows are visited best-first, usually far fewer)
-            const uint64_t ratio = h->opt_ms_stage_ratio > 0 ? (uint64_t)std::max<int64_t>(2, h->opt_ms_stage_ratio)
-                                   : std::min<uint64_t>(1024, std::max<uint64_t>(32, h->cand_cap / (16ull * b.k)));
+            const uint64_t ratio = std::min<uint64_t>(1024, std::max<uint64_t>(32, h->cand_cap / (16ull * b.k)));
             hi = hi * ratio;
         }
         return 0;
@@ -1957,14 +1916,7 @@ static int run_branches(vb_index* h, const Batch& b, bool safe) {
         if (big && !k1f) h->stats.last_big_rows = bounds[s + 1] - bounds[s];
         TRY(dense_segment(bounds[s], bounds[s + 1], direct, big));
         TRY(sparse_segment(bounds[s], bounds[s + 1], direct, big));
-        if (s == 0 && ms_staged) {
-            TRY(ms_stages());
-            if (two_streams && h->opt_dense_wait_sparse) {
-                if (!h->ev_sp_done) CK(cudaEventCreateWithFlags(&h->ev_sp_done, cudaEventDisableTiming));
-                CK(cudaEventRecord(h->ev_sp_done, ss));
-                sp_done_recorded = true;
-            }
-        }
+        if (s == 0 && ms_staged) TRY(ms_stages());
     }
     if (do_delta) {
         // K3D: the rows appended since the index was built, straight from the forward CSR.  One launch (a few
