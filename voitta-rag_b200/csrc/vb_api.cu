@@ -77,6 +77,33 @@ struct HostBuf {
 
 static size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
+struct Arena {
+    size_t off = 0;
+    size_t take(size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; }
+};
+
+// The staged argument block of a batch.  add() lays out n elements + `pad` bytes (an empty array still gets an address)
+// and names the field that receives their device address; src = nullptr: no copy.  fill() points every field, then
+// copies every array into the pinned block (in that order: the filter table holds the addresses of the scope bits).
+struct Packer {
+    struct Item { const void* src; size_t bytes, off; void* field; void (*point)(void* field, const unsigned char* p); };
+    Arena ar;
+    std::vector<Item> items;
+    Packer& reset() { ar = Arena(); items.clear(); return *this; }
+    template <class T> size_t add(const T*& field, const T* src, size_t n, size_t pad = 8) {
+        const size_t off = ar.take(n * sizeof(T) + pad);
+        items.push_back({src, n * sizeof(T), off, &field,
+                         [](void* f, const unsigned char* p) { *static_cast<const T**>(f) = reinterpret_cast<const T*>(p); }});
+        return off;
+    }
+    template <class T> size_t add(const T*& field, const std::vector<T>& v, size_t pad = 8) { return add(field, v.data(), v.size(), pad); }
+    void fill(unsigned char* hp, const unsigned char* dp) const {
+        for (const Item& it : items) it.point(it.field, dp + it.off);
+        for (const Item& it : items)
+            if (it.src && it.bytes) memcpy(hp + it.off, it.src, it.bytes);
+    }
+};
+
 struct Batch {
     uint32_t B = 0, k = 0, limit = 0, n_lists = 0, n_qterms = 0, nt_max = 1, n_filters = 0, mask_words = 0, n_blocks = 0;
     bool any_sparse = false, use_mask = false, any_heavy = false;
@@ -182,6 +209,7 @@ struct vb_index {
     std::vector<std::array<uint64_t, 5>> sel_segs;   // {r0, r1, row_off, meta_off, cap_rows} of every valid segment
     DevBuf ms_rec, ms_q, ms_units, ms_counters, mh_units;  // K3M / K3H: plan output, work-unit prefixes, counters
     HostBuf h_args_s[2], h_out_s[2], h_stage, h_sel[2];
+    Packer staging;                           // prepare_batch's layout of h_args_s (kept: no allocation per batch)
     bool sel_ran[2] = {false, false};         // the row selection ran for the batch staged in this slot
     uint32_t cand_cap = 0;
 
@@ -208,7 +236,6 @@ struct vb_index {
 
     vb_stats stats{};
     Batch staged_s[2];
-    bool staged_safe = false;
     std::vector<cudaEvent_t> prof_events;
     std::vector<int> prof_phase;
     std::vector<double> timeline;          // profile: (phase, start ms, end ms) of every timed region of the last search
@@ -930,12 +957,6 @@ extern "C" int vb_term_stats(vb_index* h, uint32_t n_terms, const uint32_t* term
 // ------------------------------------------------------------------------------------------------
 // search
 // ------------------------------------------------------------------------------------------------
-struct Arena {
-    size_t off = 0;
-    size_t take(size_t bytes) { size_t o = off; off = align_up(off + bytes, 256); return o; }
-};
-
-
 enum { PH_MASK = 0, PH_DENSE = 1, PH_SPARSE = 2, PH_SELECT = 3, PH_FUSE = 4, PH_N = 5, PH_BIG = 8 /* flag: largest segment */ };
 
 static int prof_begin(vb_index* h, int phase, cudaStream_t st = nullptr) {
@@ -1068,106 +1089,114 @@ static VbFilterTiles build_filter_tiles(const std::vector<int32_t>& mask_of, uin
     return ft;
 }
 
-// Upload the batch, evaluate the filters, initialise the candidate lists.
-static int prepare_batch(vb_index* h, const vb_query_batch* q, Batch& b, bool need_corpus) {
-    b = Batch();
-    b.need_corpus = need_corpus;
-    b.w_sparse = q->sparse_weight;
-    b.B = q->n_queries;
-    b.k = q->kprime;
-    b.limit = q->limit;
-    b.n_lists = 2 * b.B;
-    b.mode.assign(b.B, 0);
-    const bool sparse_enabled = q->fusion != VB_FUSE_DENSE_ONLY && q->sp_indptr != nullptr;
-
-    // ---- sparse queries: sort by term id, resolve posting ranges, apply IDF ----
-    std::vector<int64_t> indptr(b.B + 1, 0);
-    std::vector<double> weight, qub;
-    std::vector<uint32_t> qlo, qhi, qterm, qplo, qphi, slotq, oldq, dirq;
+// A batch's sparse terms on the host, per (query, term) with terms ascending, and with delta rows the batch inverted by term
+struct QueryTerms {
+    std::vector<int64_t> indptr;
+    std::vector<double> weight, qub, uw;
+    std::vector<uint32_t> qlo, qhi, qterm, qplo, qphi, slotq, oldq, dirq, qtab, ut, up, uq;
     std::vector<int32_t> qhidx;
-    std::vector<uint8_t> qrelaxed(b.B, 0), qms(b.B, 0), qshift;
-    std::vector<uint32_t> qtab;
-    if (sparse_enabled) {
-        if (need_corpus) TRY(ensure_sparse_index(h));
-        std::vector<std::pair<uint32_t, double>> tw;
-        for (uint32_t i = 0; i < b.B; ++i) {
-            const int64_t lo = q->sp_indptr[i], hi = q->sp_indptr[i + 1];
-            if (hi < lo) return vb_fail("sp_indptr not monotone at query %u", i);
-            if (hi - lo > VB_MAX_QUERY_TERMS) return vb_fail("query %u has %lld terms (max %d)", i, (long long)(hi - lo), VB_MAX_QUERY_TERMS);
-            tw.clear();
-            for (int64_t p = lo; p < hi; ++p) tw.emplace_back(q->sp_term[p], q->sp_weight[p]);
-            std::sort(tw.begin(), tw.end(), [](const auto& x, const auto& y) { return x.first < y.first; });
-            for (size_t t = 1; t < tw.size(); ++t)
-                if (tw[t].first == tw[t - 1].first) return vb_fail("query %u repeats sparse index %u", i, tw[t].first);
-            const size_t q_first = weight.size();
-            bool all_pos = true;                                // dense columns need every product >= 0 (error bound)
-            for (auto& pr : tw) {
-                uint64_t plo = 0, phi = 0;
-                int64_t slot = -1;
-                if (need_corpus) {
-                    slot = term_slot(h, pr.first);
-                    if (slot >= 0) { plo = h->term_ptr[slot]; phi = h->term_ptr[slot + 1]; }
-                }
-                double w = pr.second;
-                if (q->apply_idf) {
-                    const double df = (double)(need_corpus ? live_df(h, pr.first, slot) : 0);
-                    // local_collection.py _compute_idf: log((N - df + 0.5) / (df + 0.5) + 1)
-                    w = w * std::log(((double)h->n_live - df + 0.5) / (df + 0.5) + 1.0);
-                }
-                all_pos = all_pos && w > 0.0 && w < INFINITY;
-                qhidx.push_back((need_corpus && slot >= 0 && h->n_heavy) ? h->heavy_of_slot[slot] : -1);
-                // MaxScore upper bound of this term's contribution to any row of the shard; +inf = "always
-                // essential" (non-positive or non-finite weights are never pruned)
-                double ub = INFINITY;
-                if (w > 0.0 && w < INFINITY) ub = (slot >= 0 && h->term_maxval[slot] > 0.0f) ? w * (double)h->term_maxval[slot] : 0.0;
-                weight.push_back(w);
-                qub.push_back(ub);
-                qterm.push_back(pr.first);
-                qlo.push_back((uint32_t)plo);
-                qhi.push_back((uint32_t)phi);
-                qplo.push_back((uint32_t)plo);
-                qphi.push_back((uint32_t)phi);
-                slotq.push_back(i);
-                qtab.push_back((need_corpus && slot >= 0 && !h->tab_off_of_slot.empty()) ? h->tab_off_of_slot[slot] : VB_MS_NO_TAB);
-                qshift.push_back((need_corpus && slot >= 0 && !h->tab_shift_of_slot.empty()) ? h->tab_shift_of_slot[slot] : 0);
-            }
-            // terms routed to their dense column are not walked as postings (empty slice)
-            // relaxed mode (order-free sums, dense columns) needs every product >= 0 for its error bound
-            const bool relax = all_pos && need_corpus && h->sparse_nonneg && h->opt_sparse_dense;
-            qrelaxed[i] = relax ? 1 : 0;
-            // MaxScore kernel: bounds and the order-free sum need every product >= 0 as well
-            // Every query length comes this way (up to VB_MS_MAX_TERMS terms).  Until the kernel tested the score
-            // bound BEFORE the ownership lookups, a long query paid ~pe lookups per surviving posting and K3's
-            // accumulate-everything beat it (hence the ms_max_terms option, then 16); now K3M with an 85 % budget for
-            // long queries runs the 2..65-term MCP replay in 155 ms per 4096-query batch against 214 with K3.
-            const bool bounded = all_pos && need_corpus && h->sparse_nonneg && h->opt_sparse_ms && hi > lo;
-            const bool ms = bounded && hi - lo <= h->opt_ms_max_terms;
-            const bool mh = bounded && !ms && h->opt_sparse_mh;         // long query: hash-accumulate MaxScore (K3H)
-            qms[i] = ms ? 1 : (mh ? 2 : 0);
-            if (ms) {
-                b.any_ms = true;
-                uint64_t tot = 0;
-                for (size_t t = q_first; t < weight.size(); ++t) tot += qphi[t] - qplo[t];
-                b.ms_max_post = std::max(b.ms_max_post, tot);
-            }
-            else if (hi > lo) {
-                dirq.push_back(i);
-                if (mh) b.any_mh = true;
-                else { b.any_old = true; oldq.push_back(i); }
-            }
-            for (size_t t = q_first; t < weight.size(); ++t) {
-                if (!relax) qhidx[t] = -1;
-                if (qhidx[t] >= 0) { qlo[t] = qhi[t] = 0; b.any_heavy = true; }
-            }
-            indptr[i + 1] = (int64_t)weight.size();
-            b.nt_max = std::max<uint32_t>(b.nt_max, (uint32_t)(indptr[i + 1] - indptr[i]));
-            if (hi > lo) { b.mode[i] = q->fusion; b.any_sparse = true; }
-        }
-    }
-    b.n_qterms = (uint32_t)weight.size();
+    std::vector<uint8_t> qrelaxed, qms, qshift;
+    explicit QueryTerms(uint32_t B) : indptr(B + 1, 0), qrelaxed(B, 0), qms(B, 0) {}
+};
 
-    // ---- filters: the ones no query uses are dropped, the ones with equal content merged, so that every consumer
-    // (mask kernel, mask mode, row selection) sees distinct, used filters: at most B + 1 of them ----
+// ---- sparse queries: sort by term id, resolve posting ranges, apply IDF ----
+static int stage_terms(vb_index* h, const vb_query_batch* q, Batch& b, QueryTerms& qt) {
+    if (q->fusion == VB_FUSE_DENSE_ONLY || q->sp_indptr == nullptr) return 0;
+    if (b.need_corpus) TRY(ensure_sparse_index(h));
+    std::vector<std::pair<uint32_t, double>> tw;
+    for (uint32_t i = 0; i < b.B; ++i) {
+        const int64_t lo = q->sp_indptr[i], hi = q->sp_indptr[i + 1];
+        if (hi < lo) return vb_fail("sp_indptr not monotone at query %u", i);
+        if (hi - lo > VB_MAX_QUERY_TERMS) return vb_fail("query %u has %lld terms (max %d)", i, (long long)(hi - lo), VB_MAX_QUERY_TERMS);
+        tw.clear();
+        for (int64_t p = lo; p < hi; ++p) tw.emplace_back(q->sp_term[p], q->sp_weight[p]);
+        std::sort(tw.begin(), tw.end(), [](const auto& x, const auto& y) { return x.first < y.first; });
+        for (size_t t = 1; t < tw.size(); ++t)
+            if (tw[t].first == tw[t - 1].first) return vb_fail("query %u repeats sparse index %u", i, tw[t].first);
+        const size_t q_first = qt.weight.size();
+        bool all_pos = true;                                // dense columns need every product >= 0 (error bound)
+        for (auto& pr : tw) {
+            uint64_t plo = 0, phi = 0;
+            int64_t slot = -1;
+            if (b.need_corpus) {
+                slot = term_slot(h, pr.first);
+                if (slot >= 0) { plo = h->term_ptr[slot]; phi = h->term_ptr[slot + 1]; }
+            }
+            double w = pr.second;
+            if (q->apply_idf) {
+                const double df = (double)(b.need_corpus ? live_df(h, pr.first, slot) : 0);
+                // local_collection.py _compute_idf: log((N - df + 0.5) / (df + 0.5) + 1)
+                w = w * std::log(((double)h->n_live - df + 0.5) / (df + 0.5) + 1.0);
+            }
+            all_pos = all_pos && w > 0.0 && w < INFINITY;
+            qt.qhidx.push_back((b.need_corpus && slot >= 0 && h->n_heavy) ? h->heavy_of_slot[slot] : -1);
+            // MaxScore upper bound of this term's contribution to any row of the shard; +inf = "always
+            // essential" (non-positive or non-finite weights are never pruned)
+            double ub = INFINITY;
+            if (w > 0.0 && w < INFINITY) ub = (slot >= 0 && h->term_maxval[slot] > 0.0f) ? w * (double)h->term_maxval[slot] : 0.0;
+            qt.weight.push_back(w);
+            qt.qub.push_back(ub);
+            qt.qterm.push_back(pr.first);
+            qt.qlo.push_back((uint32_t)plo);
+            qt.qhi.push_back((uint32_t)phi);
+            qt.qplo.push_back((uint32_t)plo);
+            qt.qphi.push_back((uint32_t)phi);
+            qt.slotq.push_back(i);
+            qt.qtab.push_back((b.need_corpus && slot >= 0 && !h->tab_off_of_slot.empty()) ? h->tab_off_of_slot[slot] : VB_MS_NO_TAB);
+            qt.qshift.push_back((b.need_corpus && slot >= 0 && !h->tab_shift_of_slot.empty()) ? h->tab_shift_of_slot[slot] : 0);
+        }
+        // terms routed to their dense column are not walked as postings (empty slice)
+        // relaxed mode (order-free sums, dense columns) needs every product >= 0 for its error bound
+        const bool relax = all_pos && b.need_corpus && h->sparse_nonneg && h->opt_sparse_dense;
+        qt.qrelaxed[i] = relax ? 1 : 0;
+        // MaxScore kernel: bounds and the order-free sum need every product >= 0 as well
+        // Every query length comes this way (up to VB_MS_MAX_TERMS terms): K3M with an 85 % budget for long
+        // queries runs the 2..65-term MCP replay in 155 ms per 4096-query batch against 214 with K3.
+        const bool bounded = all_pos && b.need_corpus && h->sparse_nonneg && h->opt_sparse_ms && hi > lo;
+        const bool ms = bounded && hi - lo <= h->opt_ms_max_terms;
+        const bool mh = bounded && !ms && h->opt_sparse_mh;         // long query: hash-accumulate MaxScore (K3H)
+        qt.qms[i] = ms ? 1 : (mh ? 2 : 0);
+        if (ms) {
+            b.any_ms = true;
+            uint64_t tot = 0;
+            for (size_t t = q_first; t < qt.weight.size(); ++t) tot += qt.qphi[t] - qt.qplo[t];
+            b.ms_max_post = std::max(b.ms_max_post, tot);
+        }
+        else if (hi > lo) {
+            qt.dirq.push_back(i);
+            if (mh) b.any_mh = true;
+            else { b.any_old = true; qt.oldq.push_back(i); }
+        }
+        for (size_t t = q_first; t < qt.weight.size(); ++t) {
+            if (!relax) qt.qhidx[t] = -1;
+            if (qt.qhidx[t] >= 0) { qt.qlo[t] = qt.qhi[t] = 0; b.any_heavy = true; }
+        }
+        qt.indptr[i + 1] = (int64_t)qt.weight.size();
+        b.nt_max = std::max<uint32_t>(b.nt_max, (uint32_t)(qt.indptr[i + 1] - qt.indptr[i]));
+        if (hi > lo) { b.mode[i] = q->fusion; b.any_sparse = true; }
+    }
+    b.n_qterms = (uint32_t)qt.weight.size();
+    b.n_old = (uint32_t)qt.oldq.size();
+    b.n_dir = (uint32_t)qt.dirq.size();
+    // delta rows present: the batch inverted by term (term -> queries, weights) for K3D
+    if (b.need_corpus && b.any_sparse && h->n_rows > h->base_rows) {
+        std::vector<uint32_t> order(b.n_qterms);
+        for (uint32_t t = 0; t < b.n_qterms; ++t) order[t] = t;
+        std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return qt.qterm[x] < qt.qterm[y]; });   // (term, query)
+        for (uint32_t t : order) {
+            if (qt.ut.empty() || qt.ut.back() != qt.qterm[t]) { qt.ut.push_back(qt.qterm[t]); qt.up.push_back((uint32_t)qt.uq.size()); }
+            qt.uq.push_back(qt.slotq[t]);
+            qt.uw.push_back(qt.weight[t]);
+        }
+        qt.up.push_back((uint32_t)qt.uq.size());
+        b.n_uterms = (uint32_t)qt.ut.size();
+    }
+    return 0;
+}
+
+// ---- filters: the ones no query uses are dropped, the ones with equal content merged, so that every consumer
+// (mask kernel, mask mode, row selection) sees distinct, used filters: at most B + 1 of them ----
+static std::vector<vb_filter> merge_filters(const vb_index* h, const vb_query_batch* q, Batch& b) {
     const bool tombstones = h->n_live < h->n_rows;
     std::vector<int32_t> mask_of(b.B, -1);
     std::vector<vb_filter> flt;
@@ -1201,8 +1230,7 @@ static int prepare_batch(vb_index* h, const vb_query_batch* q, Batch& b, bool ne
             }
         any_filter = true;
     }
-    b.use_mask = any_filter && need_corpus;
-    b.mask_of_host = mask_of;
+    b.use_mask = any_filter && b.need_corpus;
     if (b.use_mask && mask_of[0] >= 0 && std::all_of(mask_of.begin(), mask_of.end(), [&](int32_t f) { return f == mask_of[0]; })) {
         // the row selection's cache key: equal for content-equal filters (the normalisation of filter_key)
         const FilterKey fk = filter_key(&flt[mask_of[0]]);
@@ -1212,153 +1240,94 @@ static int prepare_batch(vb_index* h, const vb_query_batch* q, Batch& b, bool ne
         b.sel_filter.insert(b.sel_filter.end(), x.scope_bits, x.scope_bits + fk.words);
     }
     b.n_filters = b.use_mask ? (uint32_t)flt.size() : 0;
+    b.mask_of_host = std::move(mask_of);
+    return flt;
+}
+
+// Upload the batch, evaluate the filters, initialise the candidate lists.
+static int prepare_batch(vb_index* h, const vb_query_batch* q, Batch& b, bool need_corpus) {
+    b = Batch();
+    b.need_corpus = need_corpus;
+    b.w_sparse = q->sparse_weight;
+    b.B = q->n_queries;
+    b.k = q->kprime;
+    b.limit = q->limit;
+    b.n_lists = 2 * b.B;
+    b.mode.assign(b.B, 0);
+
+    QueryTerms qt(b.B);
+    TRY(stage_terms(h, q, b, qt));
+    const std::vector<vb_filter> flt = merge_filters(h, q, b);
     b.mask_words = (uint32_t)((h->n_rows + 31) / 32);
     b.n_blocks = (uint32_t)((h->base_rows + VB_ROWS_PER_BLOCK - 1) / VB_ROWS_PER_BLOCK);   // row blocks of the inverted index
-
-    // ---- pack everything into one pinned block, one H2D copy ----
-    Arena ar;
-    const size_t o_q = ar.take((size_t)b.B * h->dim * 4);
-    const size_t o_ip = ar.take((b.B + 1) * 8);
-    const size_t o_w = ar.take((size_t)b.n_qterms * 8 + 8);
-    const size_t o_ub = ar.take((size_t)b.n_qterms * 8 + 8);
-    const size_t o_tid = ar.take((size_t)b.n_qterms * 4 + 8);
-    const size_t o_hx = ar.take((size_t)b.n_qterms * 4 + 8);
-    const size_t o_rx = ar.take((size_t)b.B + 8);
-    const size_t o_lo = ar.take((size_t)b.n_qterms * 4 + 8);
-    const size_t o_hi = ar.take((size_t)b.n_qterms * 4 + 8);
-    const size_t o_plo = ar.take((size_t)b.n_qterms * 4 + 8);
-    const size_t o_phi = ar.take((size_t)b.n_qterms * 4 + 8);
-    const size_t o_sq = ar.take((size_t)b.n_qterms * 4 + 8);
-    const size_t o_ms = ar.take((size_t)b.B + 8);
-    const size_t o_oq = ar.take((size_t)oldq.size() * 4 + 8);
-    const size_t o_dq = ar.take((size_t)dirq.size() * 4 + 8);
-    const size_t o_tab = ar.take((size_t)b.n_qterms * 4 + 8);
-    const size_t o_tsh = ar.take((size_t)b.n_qterms + 8);
-    // delta rows present: the batch inverted by term (term -> queries, weights) for K3D
-    std::vector<uint32_t> ut, up, uq;
-    std::vector<double> uw;
-    if (need_corpus && b.any_sparse && h->n_rows > h->base_rows) {
-        std::vector<uint32_t> order(b.n_qterms);
-        for (uint32_t t = 0; t < b.n_qterms; ++t) order[t] = t;
-        std::stable_sort(order.begin(), order.end(), [&](uint32_t x, uint32_t y) { return qterm[x] < qterm[y]; });   // (term, query)
-        for (uint32_t t : order) {
-            if (ut.empty() || ut.back() != qterm[t]) { ut.push_back(qterm[t]); up.push_back((uint32_t)uq.size()); }
-            uq.push_back(slotq[t]);
-            uw.push_back(weight[t]);
-        }
-        up.push_back((uint32_t)uq.size());
-        b.n_uterms = (uint32_t)ut.size();
-    }
-    const size_t o_ut = ar.take(ut.size() * 4 + 8);
-    const size_t o_up = ar.take(up.size() * 4 + 8);
-    const size_t o_uq = ar.take(uq.size() * 4 + 8);
-    const size_t o_uw = ar.take(uw.size() * 8 + 8);
-    const size_t o_mo = ar.take((size_t)b.B * 4);
-    const size_t o_md = ar.take((size_t)b.B * 4);
-    const size_t o_fl = ar.take((size_t)std::max<uint32_t>(1, b.n_filters) * sizeof(VbFilterDev));
-    std::vector<size_t> o_bits(b.n_filters, 0);
-    for (uint32_t f = 0; f < b.n_filters; ++f)
-        if (flt[f].scope_bits) o_bits[f] = ar.take((size_t)flt[f].scope_words * 4);
-    // mask mode 3 tables: K2T tiles of VB_TILE_N queries, resident-K2 sub-batches as vb_gemm_plan cuts them
-    const bool ftabs = b.n_filters > 31u && vb_gemm_supported(h->d_pad, b.B);
-    const uint32_t k2_sub = ftabs ? vb_gemm_plan((uint32_t)h->d_pad, b.B, (int)h->opt_k2_precision).sub : 0u;
-    const size_t o_ft2t = ftabs ? ar.take(filter_tiles_bytes(b.B, VB_TILE_N)) : 0;
-    const size_t o_ft2 = ftabs ? ar.take(filter_tiles_bytes(b.B, k2_sub)) : 0;
-    TRY(host_reserve(h->h_args_s[h->cur], ar.off));
-    TRY(dev_reserve(h, h->args, ar.off, false));
-    unsigned char* hp = h->h_args_s[h->cur].as<unsigned char>();
-    unsigned char* dp = h->args.as<unsigned char>();
-    if (!h->q_dev) {
-        if (!q->dense) return vb_fail("dense queries are NULL");   // validate_batch ran before the lock
-        memcpy(hp + o_q, q->dense, (size_t)b.B * h->dim * 4);
-    }
-    memcpy(hp + o_ip, indptr.data(), (b.B + 1) * 8);
-    if (b.n_qterms) {
-        memcpy(hp + o_w, weight.data(), (size_t)b.n_qterms * 8);
-        memcpy(hp + o_ub, qub.data(), (size_t)b.n_qterms * 8);
-        memcpy(hp + o_tid, qterm.data(), (size_t)b.n_qterms * 4);
-        memcpy(hp + o_hx, qhidx.data(), (size_t)b.n_qterms * 4);
-        memcpy(hp + o_rx, qrelaxed.data(), (size_t)b.B);
-        memcpy(hp + o_lo, qlo.data(), (size_t)b.n_qterms * 4);
-        memcpy(hp + o_hi, qhi.data(), (size_t)b.n_qterms * 4);
-        memcpy(hp + o_plo, qplo.data(), (size_t)b.n_qterms * 4);
-        memcpy(hp + o_phi, qphi.data(), (size_t)b.n_qterms * 4);
-        memcpy(hp + o_sq, slotq.data(), (size_t)b.n_qterms * 4);
-        memcpy(hp + o_ms, qms.data(), (size_t)b.B);
-        if (!oldq.empty()) memcpy(hp + o_oq, oldq.data(), oldq.size() * 4);
-        if (!dirq.empty()) memcpy(hp + o_dq, dirq.data(), dirq.size() * 4);
-        memcpy(hp + o_tab, qtab.data(), (size_t)b.n_qterms * 4);
-        memcpy(hp + o_tsh, qshift.data(), (size_t)b.n_qterms);
-    }
-    if (b.n_uterms) {
-        memcpy(hp + o_ut, ut.data(), ut.size() * 4);
-        memcpy(hp + o_up, up.data(), up.size() * 4);
-        memcpy(hp + o_uq, uq.data(), uq.size() * 4);
-        memcpy(hp + o_uw, uw.data(), uw.size() * 8);
-    }
-    b.n_old = (uint32_t)oldq.size();
-    b.n_dir = (uint32_t)dirq.size();
     b.n_rows = (uint32_t)h->n_rows;
     b.base_rows = (uint32_t)h->base_rows;
     b.gen = h->write_gen;
-    memcpy(hp + o_mo, mask_of.data(), (size_t)b.B * 4);
-    if (ftabs) {
-        b.ft_k2t = build_filter_tiles(mask_of, b.n_filters, VB_TILE_N, VB_TILED_MAX_Q, hp, dp, o_ft2t);
-        b.ft_k2 = build_filter_tiles(mask_of, b.n_filters, k2_sub, k2_sub, hp, dp, o_ft2);
-    }
-    memcpy(hp + o_md, b.mode.data(), (size_t)b.B * 4);
-    VbFilterDev* hf = reinterpret_cast<VbFilterDev*>(hp + o_fl);
+
+    // ---- pack everything into one pinned block, one H2D copy ----
+    if (!h->q_dev && !q->dense) return vb_fail("dense queries are NULL");   // validate_batch ran before the lock
+    Packer& pk = h->staging.reset();
+    const size_t o_q = pk.add(b.d_q, h->q_dev ? nullptr : q->dense, (size_t)b.B * h->dim, 0);   // first: see h2d_skip
+    const size_t o_ip = pk.add(b.d_qindptr, qt.indptr, 0);
+    pk.add(b.d_qweight, qt.weight);
+    pk.add(b.d_qub, qt.qub);
+    pk.add(b.d_qterm, qt.qterm);
+    pk.add(b.d_qhidx, qt.qhidx);
+    pk.add(b.d_qrelaxed, qt.qrelaxed);
+    pk.add(b.d_qlo, qt.qlo);
+    pk.add(b.d_qhi, qt.qhi);
+    pk.add(b.d_qplo, qt.qplo);
+    pk.add(b.d_qphi, qt.qphi);
+    pk.add(b.d_slotq, qt.slotq);
+    pk.add(b.d_qms, qt.qms);
+    pk.add(b.d_oldq, qt.oldq);
+    pk.add(b.d_dirq, qt.dirq);
+    pk.add(b.d_qtab, qt.qtab);
+    pk.add(b.d_qshift, qt.qshift);
+    pk.add(b.d_ut, qt.ut);
+    pk.add(b.d_up, qt.up);
+    pk.add(b.d_uq, qt.uq);
+    pk.add(b.d_uw, qt.uw);
+    pk.add(b.d_maskof, b.mask_of_host, 0);
+    pk.add(b.d_mode, b.mode, 0);
+    std::vector<VbFilterDev> fdev(b.n_filters);
+    pk.add(b.d_filters, b.n_filters ? fdev.data() : nullptr, std::max<uint32_t>(1, b.n_filters), 0);
     for (uint32_t f = 0; f < b.n_filters; ++f) {
-        hf[f].scope_bits = flt[f].scope_bits ? reinterpret_cast<const uint32_t*>(dp + o_bits[f]) : nullptr;
-        hf[f].scope_words = flt[f].scope_words;
-        hf[f].ts_field = flt[f].ts_field;
-        hf[f].ts_lo = flt[f].ts_lo;
-        hf[f].ts_hi = flt[f].ts_hi;
-        if (flt[f].scope_bits) { memcpy(hp + o_bits[f], flt[f].scope_bits, (size_t)flt[f].scope_words * 4); b.need_scope = 1; }
-        if (flt[f].ts_field == VB_TS_CREATED) b.need_created = 1;
-        if (flt[f].ts_field == VB_TS_MODIFIED) b.need_modified = 1;
+        const vb_filter& x = flt[f];
+        fdev[f] = VbFilterDev{nullptr, x.scope_words, x.ts_field, x.ts_lo, x.ts_hi};
+        if (x.scope_bits) { pk.add(fdev[f].scope_bits, x.scope_bits, x.scope_words, 0); b.need_scope = 1; }
+        if (x.ts_field == VB_TS_CREATED) b.need_created = 1;
+        if (x.ts_field == VB_TS_MODIFIED) b.need_modified = 1;
+    }
+    // mask mode 3 tables: K2T tiles of VB_TILE_N queries, resident-K2 sub-batches as vb_gemm_plan cuts them
+    const bool ftabs = b.n_filters > 31u && vb_gemm_supported(h->d_pad, b.B);
+    const uint32_t k2_sub = ftabs ? vb_gemm_plan((uint32_t)h->d_pad, b.B, (int)h->opt_k2_precision).sub : 0u;
+    const size_t o_ft2t = ftabs ? pk.ar.take(filter_tiles_bytes(b.B, VB_TILE_N)) : 0;
+    const size_t o_ft2 = ftabs ? pk.ar.take(filter_tiles_bytes(b.B, k2_sub)) : 0;
+    TRY(host_reserve(h->h_args_s[h->cur], pk.ar.off));
+    TRY(dev_reserve(h, h->args, pk.ar.off, false));
+    unsigned char* hp = h->h_args_s[h->cur].as<unsigned char>();
+    unsigned char* dp = h->args.as<unsigned char>();
+    pk.fill(hp, dp);
+    if (ftabs) {
+        b.ft_k2t = build_filter_tiles(b.mask_of_host, b.n_filters, VB_TILE_N, VB_TILED_MAX_Q, hp, dp, o_ft2t);
+        b.ft_k2 = build_filter_tiles(b.mask_of_host, b.n_filters, k2_sub, k2_sub, hp, dp, o_ft2);
     }
     // device hand-off (SURVEY §8 f-4): the query rows never visit the host — the H2D copy starts after their slot and a
     // D2D copy, ordered after the producer's stream, fills it
     const size_t h2d_skip = h->q_dev ? o_ip : 0;
-    CK(cudaMemcpyAsync(dp + h2d_skip, hp + h2d_skip, ar.off - h2d_skip, cudaMemcpyHostToDevice, h->stream));
+    CK(cudaMemcpyAsync(dp + h2d_skip, hp + h2d_skip, pk.ar.off - h2d_skip, cudaMemcpyHostToDevice, h->stream));
     if (h->q_dev) {
         if (!h->ev_q) CK(cudaEventCreateWithFlags(&h->ev_q, cudaEventDisableTiming));
         CK(cudaEventRecord(h->ev_q, h->q_dev_stream));
         CK(cudaStreamWaitEvent(h->stream, h->ev_q, 0));
         CK(cudaMemcpyAsync(dp + o_q, h->q_dev, (size_t)b.B * h->dim * 4, cudaMemcpyDeviceToDevice, h->stream));
     }
-    b.d_q = reinterpret_cast<const float*>(dp + o_q);
-    b.d_qindptr = reinterpret_cast<const int64_t*>(dp + o_ip);
-    b.d_qweight = reinterpret_cast<const double*>(dp + o_w);
-    b.d_qub = reinterpret_cast<const double*>(dp + o_ub);
-    b.d_qterm = reinterpret_cast<const uint32_t*>(dp + o_tid);
-    b.d_qhidx = reinterpret_cast<const int32_t*>(dp + o_hx);
-    b.d_qrelaxed = reinterpret_cast<const uint8_t*>(dp + o_rx);
-    b.d_qlo = reinterpret_cast<const uint32_t*>(dp + o_lo);
-    b.d_qhi = reinterpret_cast<const uint32_t*>(dp + o_hi);
-    b.d_qplo = reinterpret_cast<const uint32_t*>(dp + o_plo);
-    b.d_qphi = reinterpret_cast<const uint32_t*>(dp + o_phi);
-    b.d_slotq = reinterpret_cast<const uint32_t*>(dp + o_sq);
-    b.d_qms = reinterpret_cast<const uint8_t*>(dp + o_ms);
-    b.d_oldq = reinterpret_cast<const uint32_t*>(dp + o_oq);
-    b.d_dirq = reinterpret_cast<const uint32_t*>(dp + o_dq);
-    b.d_qtab = reinterpret_cast<const uint32_t*>(dp + o_tab);
-    b.d_qshift = reinterpret_cast<const uint8_t*>(dp + o_tsh);
-    b.d_ut = reinterpret_cast<const uint32_t*>(dp + o_ut);
-    b.d_up = reinterpret_cast<const uint32_t*>(dp + o_up);
-    b.d_uq = reinterpret_cast<const uint32_t*>(dp + o_uq);
-    b.d_uw = reinterpret_cast<const double*>(dp + o_uw);
-    b.d_maskof = reinterpret_cast<const int32_t*>(dp + o_mo);
-    b.d_mode = reinterpret_cast<const int32_t*>(dp + o_md);
-    b.d_filters = reinterpret_cast<const VbFilterDev*>(dp + o_fl);
 
     // ---- candidate lists ----
-    // segment growth: each segment appends ~ratio * k' candidates per list before the next compaction.  Batches
-    // keep 32 (list memory and compaction time scale with B); single queries are launch-latency bound and take
-    // 128 (one segment fewer on 100k..10M rows; measured +7..25 % q/s at B = 1).
-    // (round 2: 8 instead of 32 for batches — the appends of a segment cost more than the extra launch + compaction:
-    //  cfg4 dense 18.0 -> 15.8 ms)
+    // segment growth: each segment appends ~ratio * k' candidates per list before the next compaction.  Batches take 8
+    // (the appends of a segment cost more than the extra launch + compaction: cfg4 dense 15.8 ms, 18.0 with 32); single
+    // queries are launch-latency bound and take 128 (one segment fewer on 100k..10M rows; measured +7..25 % q/s at B = 1).
     b.seg_ratio = h->opt_seg_ratio > 0 ? (uint32_t)h->opt_seg_ratio : (b.B <= 4 ? 128u : 8u);
     uint32_t need_cap = std::max<uint32_t>(16384u, (uint32_t)align_up((size_t)2 * (size_t)std::max<uint32_t>(b.seg_ratio, 32u) * b.k, 4096));
     // roomier lists (up to 256 MB in all) let K3M take larger posting stages: fewer launches on small corpora
@@ -1375,8 +1344,8 @@ static int prepare_batch(vb_index* h, const vb_query_batch* q, Batch& b, bool ne
     b.cnt = h->lists.as<uint32_t>() + 2 * (size_t)b.n_lists;      // [n_lists][VB_SUB]
     b.gtau = h->lists.as<uint32_t>() + (2 + (size_t)VB_SUB) * b.n_lists;
     b.done = h->lists.as<uint32_t>() + (3 + (size_t)VB_SUB) * b.n_lists;
-    b.h2d_bytes = ar.off - h2d_skip;
-    h->stats.last_h2d_bytes = ar.off - h2d_skip;
+    b.h2d_bytes = pk.ar.off - h2d_skip;
+    h->stats.last_h2d_bytes = pk.ar.off - h2d_skip;
     // output block layout
     Arena ao;
     b.o_rows = ao.take((size_t)b.B * b.limit * 4);
@@ -1394,13 +1363,6 @@ static int prepare_batch(vb_index* h, const vb_query_batch* q, Batch& b, bool ne
     return 0;
 }
 
-// direct_rows > 0: the first segment stores its keys at fixed slots [0, direct_rows) of every
-// list (no atomics); slots nobody writes (masked rows, rows without postings) must read as empty.
-static int init_lists(vb_index* h, const Batch& b, uint32_t direct_rows) {
-    if (direct_rows)
-        CK(cudaMemset2DAsync(h->cand.p, (size_t)h->cand_cap * 8, 0, (size_t)direct_rows * 8, b.n_lists, h->stream));
-    return 0;
-}
 // empty lists for the paths that score nothing (empty index, merge of gathered shard lists)
 __global__ void vb_init_lists_kernel(const VbListInit li) {
     vb_init_list(li, blockIdx.x * blockDim.x + threadIdx.x);
@@ -1427,536 +1389,569 @@ static VbLists make_lists(const vb_index* h, const Batch& b, bool safe) {
     return L;
 }
 
-static int launch_scan(vb_index* h, const Batch& b, const VbLists& L, uint32_t row_begin, uint32_t row_end, uint32_t direct, cudaStream_t st) {
-    VbScanArgs a{};
-    a.rows = h->rows.as<uint4>();
-    a.inv_norm = h->inv_norm.as<float>();
+// The filter masks as a kernel's arguments take them: nullptr when no query of the batch is filtered.
+template <class A> static void set_mask(A& a, const vb_index* h, const Batch& b) {
     a.mask = b.use_mask ? h->mask.as<uint32_t>() : nullptr;
     a.mask_of = b.use_mask ? b.d_maskof : nullptr;
-    a.q_hat = h->q_hat.as<float>();
-    a.tau = b.tau;
-    a.lists = L;
     a.mask_words = b.mask_words;
-    a.chunks = (uint32_t)h->d_pad / 8;
-    a.row_begin = row_begin;
-    a.row_end = row_end;
-    a.row_base = (uint32_t)h->row_base;
-    a.q_begin = 0;
-    a.direct = direct;
-    const uint32_t groups = (row_end - row_begin + 31) / 32;
-    const uint32_t per_q = std::max<uint32_t>(1, (uint32_t)(h->sm_count * 8) / std::min<uint32_t>(b.B, 8));
-    dim3 grid(std::min<uint32_t>((groups + 7) / 8, per_q), b.B);
-    const int nch = (int)((a.chunks + 31) / 32);
-    switch (nch) {
-        case 1: vb_dense_scan_kernel<1><<<grid, 256, 0, st>>>(a); break;
-        case 2: vb_dense_scan_kernel<2><<<grid, 256, 0, st>>>(a); break;
-        case 3: vb_dense_scan_kernel<3><<<grid, 256, 0, st>>>(a); break;
-        case 4: vb_dense_scan_kernel<4><<<grid, 256, 0, st>>>(a); break;
-        default: vb_dense_scan_generic_kernel<<<grid, 256, 0, st>>>(a); break;
+}
+
+// Which sparse kernel scores which query.  Queries whose products are all >= 0 and that are not too long go to K3M,
+// the posting-driven MaxScore kernel; the others (and everything when K3M is off) stay on K3 (block x query CTAs over
+// the row segments, first segment direct); long queries go to K3H when it is on (K3 direct segment, then K3H per segment).
+//   normal mode: K3M runs in STAGES over the whole index (sparse_ms.cuh): stage 0 scores the first ms_p0
+//                postings of every query in descending-ub order with no threshold, each later stage 32x more;
+//   safe mode:   K3M runs once per (small) row segment, like K3, so that no list can overflow.
+struct SparseRoute {
+    bool ms_on = false, ms_staged = false, mh_on = false, k3_direct = false, k3_all_segments = false;
+    uint32_t fine_blocks = 0;                  // fine (2048-row) slice table rows K3 will read
+    // K3's queries (nullptr = all B): all of them without K3M / K3H and in the direct segment of the per-segment flow;
+    // the K3 + K3H ones in the direct segment of the staged flow; elsewhere only the ones nobody else takes
+    const uint32_t *k3_q_direct = nullptr, *k3_q = nullptr;
+    uint32_t k3_n_direct = 0, k3_n = 0;
+};
+// One row segment's part of the K2T row selection (dense_compact.cuh)
+struct SelSeg { bool on = false, kept = false; uint32_t cap_rows = 0, n_blocks = 0, ev = 0; size_t row_off = 0, meta_off = 0; };
+// What run_branches decided for this search; its stages read it.
+struct Search {
+    vb_index* h;
+    const Batch& b;
+    bool safe_mode = false;                    // fixed small segments that can never overflow a list
+    std::vector<uint32_t> bounds{0};           // segment boundaries, multiples of VB_ROWS_PER_BLOCK
+    uint32_t n = 0, nb = 0;                    // rows; the inverted index covers [0, nb), rows appended since (the delta) go to K3D
+    VbLists L{};
+    int path = 1;                              // dense: 1 = K1 / K1F, 2 = tensor-core kernel
+    VbGemmPlan plan{1u, 0u};
+    bool tiled = false, k1f = false, do_sparse = false, do_delta = false;
+    SparseRoute sp;
+    uint32_t direct_rows = 0, ms_chunk = 0, sel_pct = 0;
+    std::vector<SelSeg> sel_seg;               // row selection, per segment
+    bool sel_copy = false, sel_side = false;   // some selected segment is copied / copies run on the side stream
+    std::vector<uint64_t> sel_key;             // what the scratch holds once this batch has enqueued its work (empty: no selection)
+    cudaStream_t sd = h->stream, ss = h->stream;   // dense chain, sparse chain (aux_stream when the two overlap)
+};
+
+static void schedule_segments(Search& s, bool safe) {
+    const vb_index* h = s.h;
+    s.safe_mode = safe || h->opt_safe_mode;
+    s.n = (uint32_t)h->n_rows;
+    if (s.safe_mode) {
+        const uint32_t step = (uint32_t)std::max<size_t>(VB_ROWS_PER_BLOCK, (h->cand_cap - s.b.k) / VB_ROWS_PER_BLOCK * VB_ROWS_PER_BLOCK);
+        for (uint64_t r = step; r < s.n; r += step) s.bounds.push_back((uint32_t)r);
+    } else {
+        for (uint64_t r = (uint64_t)h->opt_seg_first; r < s.n; r *= (uint64_t)s.b.seg_ratio) s.bounds.push_back((uint32_t)r);
     }
-    CKK("vb_dense_scan_kernel");
+    s.bounds.push_back(s.n);
+    s.L = make_lists(h, s.b, s.safe_mode);
+}
+static int choose_kernels(Search& s) {
+    vb_index* h = s.h; const Batch& b = s.b;
+    int path = (int)h->opt_dense_path;
+    if (path == 0) path = vb_gemm_supported(h->d_pad, b.B) && b.B >= 2 ? 2 : 1;
+    if (path == 2 && !vb_gemm_supported(h->d_pad, b.B)) return vb_fail("dense_path=2 requested but unsupported for d_pad=%d B=%u", h->d_pad, b.B);
+    h->stats.last_dense_path = (uint32_t)path;
+    s.path = path;
+    if (path == 2) s.plan = vb_gemm_plan((uint32_t)h->d_pad, b.B, (int)h->opt_k2_precision);
+    // batches too large to sit resident in shared memory go to the query-tiled, tensor-bound kernel
+    // (one corpus pass per 1024 queries)
+    s.tiled = path == 2 && b.B > s.plan.sub && !s.plan.split && h->opt_k2_tiled && vb_gemm_tiled_supported(h->d_pad);
+    h->stats.last_dense_passes = path == 2 ? (s.tiled ? (b.B + VB_TILED_MAX_Q - 1) / VB_TILED_MAX_Q : (b.B + s.plan.sub - 1) / s.plan.sub) : b.B;
+    // K1F: one pass over all rows for tiny batches (no segments, no direct slots)
+    // (on large corpora the segmented K1 streams faster — no per-stretch barriers — and its launches are noise there:
+    //  cfg3 10M rows, B = 1: K1 1.65 ms, K1F 1.83 ms; cfg1 100k rows: K1 59 us + 3 selects, K1F 48 us + 1 merge)
+    s.k1f = path == 1 && !s.safe_mode && h->opt_k1f && (h->opt_k1f > 1 || s.n <= (2u << 20)) && b.B <= VB_K1F_MAX_B && (h->d_pad / 8 + 31) / 32 <= 4 &&
+            b.k <= VB_K1F_CAP / 2u && (uint64_t)vb_k1f_grid(h->sm_count, b.k, b.B, h->d_pad) * b.k <= h->cand_cap;
+    SparseRoute& r = s.sp;
+    s.nb = (uint32_t)std::min<uint64_t>(h->base_rows, s.n);
+    s.do_sparse = b.any_sparse && h->nnz_live > 0 && b.n_qterms > 0 && s.nb > 0;
+    s.do_delta = b.any_sparse && b.n_uterms > 0 && s.nb < s.n;
+    r.ms_on = s.do_sparse && b.any_ms && h->opt_sparse_ms;
+    r.ms_staged = r.ms_on && !s.safe_mode && h->opt_ms_staged;
+    r.mh_on = s.do_sparse && b.any_mh;
+    // the first segment writes its keys to fixed slots at the front of the list (no atomics) — unless nobody runs
+    // a first segment: K1F scans in one pass, K3M in posting stages
+    r.k3_direct = s.do_sparse && (!r.ms_staged || b.n_dir > 0);
+    s.direct_rows = (s.bounds[1] <= h->cand_cap && (!s.k1f || r.k3_direct)) ? s.bounds[1] : 0u;
+    r.k3_all_segments = s.do_sparse && ((!r.ms_on && !r.mh_on) || b.any_old);
+    r.fine_blocks = r.k3_all_segments ? b.n_blocks
+                    : (r.k3_direct ? std::min<uint32_t>(b.n_blocks, (s.direct_rows + VB_ROWS_PER_BLOCK - 1) / VB_ROWS_PER_BLOCK) : 0u);
+    r.k3_n_direct = r.k3_n = b.B;
+    if (r.ms_on || r.mh_on) { r.k3_q = b.d_oldq; r.k3_n = b.n_old; }
+    if (r.ms_staged) { r.k3_q_direct = b.d_dirq; r.k3_n_direct = b.n_dir; }
+    s.ms_chunk = h->opt_ms_chunk > 0 ? (uint32_t)align_up((size_t)h->opt_ms_chunk, VB_MS_U * VB_MS_THREADS) : 512u;
+    return 0;
+}
+
+// List set-up + query prep (fp32 unit queries for K1, packed bf16 operand for K2) in ONE launch, then the K0 filter masks.
+static int prep_and_mask(Search& s) {
+    vb_index* h = s.h; const Batch& b = s.b;
+    // direct_rows > 0: the first segment stores its keys at fixed slots [0, direct_rows) of every
+    // list (no atomics); slots nobody writes (masked rows, rows without postings) must read as empty.
+    if (s.direct_rows)
+        CK(cudaMemset2DAsync(h->cand.p, (size_t)h->cand_cap * 8, 0, (size_t)s.direct_rows * 8, b.n_lists, h->stream));
+    TRY(dev_reserve(h, h->q_hat, (size_t)b.B * h->d_pad * 4, false));
+    TRY(dev_reserve(h, h->q_bf16, (size_t)(2 * ((size_t)b.B + 256)) * h->d_pad * 2, false));
+    TRY(dev_reserve(h, h->q_scale, (size_t)b.B * 4, false));
+    VbListInit li{};
+    li.tau = b.tau; li.cnt = b.cnt; li.overflow = b.overflow; li.gtau = b.gtau; li.n = b.n_lists; li.cnt0 = s.direct_rows;
+    li.no_direct = s.sp.ms_staged ? b.d_qms : nullptr; li.n_queries = b.B; li.dense_direct = s.k1f ? 0u : 1u;
+    vb_prep_query_kernel<<<b.B, 128, 0, h->stream>>>(b.d_q, (uint32_t)h->dim, (uint32_t)h->d_pad, b.B, s.plan.sub, s.plan.split,
+                                                     h->q_hat.as<float>(), h->q_bf16.as<__nv_bfloat16>(), h->q_scale.as<float>(),
+                                                     reinterpret_cast<uint32_t*>(h->out.as<unsigned char>() + b.o_bad), li);
+    CKK("vb_prep_query_kernel");
     ++h->stats.last_launches;
+    if (!b.use_mask) return 0;
+    prof_begin(h, PH_MASK);
+    const size_t mask_bytes = (size_t)b.n_filters * b.mask_words * 4;
+    if (dev_reserve(h, h->mask, mask_bytes, false) != 0) {
+        cudaGetLastError();
+        return vb_fail("filter masks of %u distinct filters over %u rows need %zu bytes of device memory: %s",
+                       b.n_filters, s.n, mask_bytes, g_err.c_str());
+    }
+    vb_mask_kernel<<<grid_for((uint64_t)b.mask_words * 32, 256, h->sm_count * 8), 256, 0, h->stream>>>(
+        h->scope_id.as<uint32_t>(), h->created.as<int64_t>(), h->modified.as<int64_t>(), h->alive.as<uint32_t>(), s.n,
+        b.d_filters, b.n_filters, b.mask_words, b.need_created, b.need_modified, b.need_scope, h->mask.as<uint32_t>());
+    CKK("vb_mask_kernel");
+    ++h->stats.last_launches;
+    prof_end(h);
+    return 0;
+}
+
+static int launch_rowsel(Search& s, size_t si, cudaStream_t st) {
+    vb_index* h = s.h;
+    const SelSeg& z = s.sel_seg[si];
+    const uint32_t r0 = s.bounds[si], r1 = s.bounds[si + 1];
+    VbRowSelArgs sa{};
+    sa.mask = h->mask.as<uint32_t>() + (size_t)s.b.mask_of_host[0] * s.b.mask_words;
+    sa.word_begin = r0 / 32u; sa.word_end = (r1 + 31u) / 32u; sa.row_end = r1;
+    sa.sel = h->sel_meta.as<uint32_t>() + z.meta_off; sa.block_sums = sa.sel + 4; sa.ids = h->sel_ids.as<uint32_t>() + z.row_off;
+    sa.pct = s.sel_pct; sa.pad_row = r0; sa.cap_rows = z.cap_rows;
+    vb_rowsel_count_kernel<<<z.n_blocks, VB_SEL_THREADS, 0, st>>>(sa);
+    CKK("vb_rowsel_count_kernel");
+    vb_rowsel_scatter_kernel<<<z.n_blocks, VB_SEL_THREADS, 0, st>>>(sa);
+    CKK("vb_rowsel_scatter_kernel");
+    vb_rowsel_gather_kernel<<<h->sm_count * 4, 256, 0, st>>>(h->rows.as<uint4>(), h->inv_norm.as<float>(), sa.ids, sa.sel,
+                                                            h->sel_rows.as<uint4>() + z.row_off * (h->d_pad / 8), h->sel_inv.as<float>() + z.row_off,
+                                                            (uint32_t)h->d_pad / 8u);
+    CKK("vb_rowsel_gather_kernel");
+    h->stats.last_launches += 3;
+    return 0;
+}
+// ---- K2T row selection (dense_compact.cuh): the tensor-bound kernel, ONE filter for the whole batch, every segment of
+// at least dense_compact_min_rows rows.  Count, list and copy run on a side stream right after the mask kernel: the
+// copy of segment s + 1 (HBM-bound) hides behind the GEMM of segment s (tensor-bound).  With the chains serialised
+// (overlap = 0: per-phase timing) they run inline on the dense stream and are charged to the dense phase.
+// The copy is kept across batches (h->sel_key): a segment whose key matches the scratch is not copied again, and the
+// tensor-core kernel reads the scratch and its device-side {count, decision} as they are.
+static int plan_rowsel(Search& s) {
+    vb_index* h = s.h; const Batch& b = s.b;
+    s.sel_seg.assign(s.bounds.size() - 1, SelSeg{});
+    s.sel_side = h->opt_overlap != 0;
+    // auto threshold: the copy costs ~0.49 ns per passing row (read + write of 2 * d_pad bytes at HBM speed, d_pad = 768);
+    // one pass of the tensor-core kernel over a row costs max(0.245 ns (HBM), 1.08 ns * queries / 1024 (tensor pipe)) — both
+    // scale with d_pad alike.  Copying pays when (1 - p) * passes' time > p * copy time.
+    s.sel_pct = (uint32_t)std::max<int64_t>(0, std::min<int64_t>(100, h->opt_dense_compact));
+    if (h->opt_dense_compact < 0 && s.path == 2) {
+        double T = 0.0;
+        if (s.tiled) for (uint32_t q0 = 0; q0 < b.B; q0 += VB_TILED_MAX_Q) T += std::max(0.245, 1.08 * std::min(VB_TILED_MAX_Q, b.B - q0) / 1024.0);
+        else T = 0.245 * ((b.B + s.plan.sub - 1) / s.plan.sub);
+        s.sel_pct = (uint32_t)(95.0 * T / (T + 0.49));
+    }
+    if (s.path != 2 || s.k1f || b.sel_filter.empty() || s.sel_pct == 0 || h->sel_no_memory || h->d_pad > 1024) return 0;
+    size_t rows_total = 0, meta_total = 0;
+    uint32_t n_on = 0;
+    for (size_t si = (s.direct_rows ? 1 : 0); si < s.sel_seg.size() && n_on < 8u; ++si) {
+        const uint32_t r0 = s.bounds[si], r1 = s.bounds[si + 1];
+        if ((r0 % 128u) != 0u || (int64_t)(r1 - r0) < h->opt_dense_compact_min_rows) continue;
+        SelSeg& z = s.sel_seg[si];
+        z.on = true; z.cap_rows = (uint32_t)align_up(r1 - r0, 128); z.n_blocks = ((r1 - r0 + 31u) / 32u + VB_SEL_WORDS - 1u) / VB_SEL_WORDS;
+        z.row_off = rows_total; z.meta_off = meta_total; z.ev = n_on++;
+        rows_total += z.cap_rows; meta_total += align_up((size_t)4 + z.n_blocks, 4);
+    }
+    const size_t scratch = rows_total * h->d_pad * 2;
+    if (n_on && scratch > h->sel_rows.cap) {
+        size_t free_b = 0, total_b = 0;
+        if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess || free_b + h->sel_rows.cap < scratch + (4ull << 30)) {
+            cudaGetLastError();
+            h->sel_no_memory = true;                         // the scratch matrix does not fit beside the shard: stay in place
+            h->sel_key.clear();
+            s.sel_seg.assign(s.sel_seg.size(), SelSeg{});
+            return 0;
+        }
+    }
+    if (!n_on) return 0;
+    const void* before[4] = {h->sel_rows.p, h->sel_inv.p, h->sel_ids.p, h->sel_meta.p};
+    // Invalid from here until this batch has enqueued all of its work (commit_rowsel): an error return in between (a
+    // failed reserve, a copy enqueued in part) leaves the next batch to copy again.
+    std::vector<uint64_t> cached_key;
+    cached_key.swap(h->sel_key);
+    TRY(dev_reserve(h, h->sel_rows, scratch, false));
+    TRY(dev_reserve(h, h->sel_inv, rows_total * 4, false));
+    TRY(dev_reserve(h, h->sel_ids, rows_total * 4, false));
+    TRY(dev_reserve(h, h->sel_meta, meta_total * 4, false));
+    const bool moved = before[0] != h->sel_rows.p || before[1] != h->sel_inv.p || before[2] != h->sel_ids.p || before[3] != h->sel_meta.p;
+    // the key: filter content, index version, and every input of the plan above
+    s.sel_key = b.sel_filter;
+    s.sel_key.insert(s.sel_key.end(), {h->write_gen, (uint64_t)s.n, (uint64_t)h->d_pad, s.sel_pct, (uint64_t)h->opt_dense_compact_min_rows,
+                                   (uint64_t)s.path, (uint64_t)s.tiled, s.direct_rows});
+    const bool key_holds = h->opt_sel_reuse && !moved && s.sel_key == cached_key;
+    for (size_t si = 0; si < s.sel_seg.size(); ++si) {
+        SelSeg& z = s.sel_seg[si];
+        if (!z.on) continue;
+        const std::array<uint64_t, 5> zk{s.bounds[si], s.bounds[si + 1], z.row_off, z.meta_off, z.cap_rows};
+        z.kept = key_holds && std::find(h->sel_segs.begin(), h->sel_segs.end(), zk) != h->sel_segs.end();
+        s.sel_copy |= !z.kept;
+    }
+    if (!s.sel_copy || !s.sel_side) return 0;
+    // Ordering of the scratch (two batches can be in flight).  A kept segment is only read, by kernels on the dense
+    // stream.  A copy waits for ev_sel_fork, recorded on the dense stream after this batch's mask kernel and therefore
+    // after every kernel an earlier batch enqueued there, so it cannot overwrite the scratch while an earlier batch's
+    // tensor-core kernel still reads it — whether that batch copied or kept.  A batch that keeps a copy made by an earlier
+    // one reads it after that batch's dense kernels, which waited for the copy's events: the copy has finished.
+    if (!h->sel_stream) {
+        CK(cudaStreamCreateWithFlags(&h->sel_stream, cudaStreamNonBlocking));
+        CK(cudaEventCreateWithFlags(&h->ev_sel_fork, cudaEventDisableTiming));
+        for (auto& e : h->ev_sel) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    }
+    CK(cudaEventRecord(h->ev_sel_fork, s.sd));               // after the mask kernel (and after the previous batch's dense chain)
+    CK(cudaStreamWaitEvent(h->sel_stream, h->ev_sel_fork, 0));
+    for (size_t si = 0; si < s.sel_seg.size(); ++si)
+        if (s.sel_seg[si].on && !s.sel_seg[si].kept) {
+            TRY(launch_rowsel(s, si, h->sel_stream));
+            CK(cudaEventRecord(h->ev_sel[s.sel_seg[si].ev], h->sel_stream));
+        }
+    return 0;
+}
+// Called once the batch has enqueued all of its work: every selected segment is in the scratch now.
+static void commit_rowsel(Search& s) {
+    if (s.sel_key.empty()) return;
+    s.h->sel_segs.clear();
+    for (size_t si = 0; si < s.sel_seg.size(); ++si)
+        if (s.sel_seg[si].on) s.h->sel_segs.push_back({s.bounds[si], s.bounds[si + 1], s.sel_seg[si].row_off, s.sel_seg[si].meta_off, s.sel_seg[si].cap_rows});
+    s.h->sel_key = std::move(s.sel_key);
+}
+
+// Select of the lists [q0, q0 + B) (q0 = 0: dense, B: sparse) on stream st.
+static int compact_lists(Search& s, cudaStream_t st, uint32_t q0, uint32_t lim0) {
+    const int ps = prof_begin(s.h, PH_SELECT, st);
+    vb_compact_kernel<<<s.b.B, VB_COMPACT_THREADS, 0, st>>>(s.L, s.b.tau, s.b.overflow, s.b.k, q0, lim0);
+    CKK("vb_compact_kernel");
+    ++s.h->stats.last_launches;
+    prof_end(s.h, ps, st);
+    return 0;
+}
+static int dense_single_pass(Search& s) {
+    vb_index* h = s.h; const Batch& b = s.b;
+    const int pi = prof_begin(h, PH_DENSE | PH_BIG, s.sd);
+    VbScan1Args a{};
+    a.rows = h->rows.as<uint4>(); a.inv_norm = h->inv_norm.as<float>();
+    set_mask(a, h, b);
+    a.q_hat = h->q_hat.as<float>(); a.gtau = b.gtau; a.cand = h->cand.as<uint64_t>(); a.cnt = b.cnt;
+    a.cap = h->cand_cap; a.k = b.k; a.chunks = (uint32_t)h->d_pad / 8; a.n_rows = s.n;
+    a.row_base = (uint32_t)h->row_base;
+    a.done = b.done; a.tau = b.tau;
+    const dim3 grid(vb_k1f_grid(h->sm_count, b.k, b.B, h->d_pad), b.B);
+    // small corpora: fewer 32-row groups than warps — give each warp a half / quarter / eighth of a group
+    const uint32_t n_groups = (s.n + 31u) / 32u, n_warps = grid.x * (VB_K1F_THREADS / 32u);
+    a.split_shift = 0;
+    while (a.split_shift < 3u && (n_groups << (a.split_shift + 1u)) <= n_warps) ++a.split_shift;
+    // large corpora: units of 2..32 groups (one coalesced filter-word load per unit, row batches filled across its
+    // groups), as long as every warp still gets >= 4 units (static interleaved assignment: +-1 unit of imbalance)
+    a.unit_shift = 0;
+    if (!a.split_shift)
+        while (a.unit_shift < 5u && (n_groups >> (a.unit_shift + 1u)) >= 4u * n_warps) ++a.unit_shift;
+    switch ((a.chunks + 31) / 32) {
+        case 1: vb_dense_scan1_kernel<1><<<grid, VB_K1F_THREADS, 0, s.sd>>>(a); break;
+        case 2: vb_dense_scan1_kernel<2><<<grid, VB_K1F_THREADS, 0, s.sd>>>(a); break;
+        case 3: vb_dense_scan1_kernel<3><<<grid, VB_K1F_THREADS, 0, s.sd>>>(a); break;
+        default: vb_dense_scan1_kernel<4><<<grid, VB_K1F_THREADS, 0, s.sd>>>(a); break;
+    }
+    CKK("vb_dense_scan1_kernel");
+    ++h->stats.last_launches;
+    prof_end(h, pi, s.sd);                                  // (the merge of the per-CTA lists happens inside: last CTA)
+    h->stats.last_big_rows = s.n;
+    h->stats.last_dense_path = 3u;                          // K1F
+    return 0;
+}
+static int dense_segment(Search& s, size_t si, uint32_t direct, bool big) {
+    vb_index* h = s.h; const Batch& b = s.b;
+    const uint32_t r0 = s.bounds[si], r1 = s.bounds[si + 1];
+    if (big) h->stats.last_big_rows = r1 - r0;          // the segment with the most rows: the roofline's launch
+    // Row selection: nothing to do when the scratch kept this segment's copy; otherwise wait for its copy (side
+    // stream), or run the selection here (chains serialised: its own timed region of the dense phase, so that the
+    // PH_BIG region stays the tensor-core kernel alone)
+    const SelSeg& z = s.sel_seg[si];
+    if (z.on) {
+        if (!z.kept && s.sel_side) CK(cudaStreamWaitEvent(s.sd, h->ev_sel[z.ev], 0));
+        else if (!z.kept) {
+            const int pz = prof_begin(h, PH_DENSE, s.sd);
+            TRY(launch_rowsel(s, si, s.sd));
+            prof_end(h, pz, s.sd);
+        }
+        if (big) {                                       // {rows, decision} of the roofline's segment for vb_stats
+            TRY(host_reserve(h->h_sel[h->cur], 16));
+            CK(cudaMemcpyAsync(h->h_sel[h->cur].p, h->sel_meta.as<uint32_t>() + z.meta_off, 8, cudaMemcpyDeviceToHost, s.sd));
+            h->sel_ran[h->cur] = true;
+        }
+    }
+    const int pi = prof_begin(h, PH_DENSE | (big ? PH_BIG : 0), s.sd);
+    if (s.path == 2) {
+        VbGemmLaunch g{};
+        g.rows = h->rows.p; g.inv_norm = h->inv_norm.as<float>(); g.q_bf16 = h->q_bf16.p;
+        set_mask(g, h, b);
+        g.n_filters = b.n_filters; g.tau = b.tau; g.q_scale = h->q_scale.as<float>(); g.lists = s.L;
+        g.n_rows_total = s.n; g.row_begin = r0; g.row_end = r1; g.row_base = (uint32_t)h->row_base;
+        g.d_pad = (uint32_t)h->d_pad; g.n_queries = b.B; g.sm_count = h->sm_count; g.stream = s.sd;
+        g.direct = direct; g.plan = s.plan; g.mask_of_host = b.mask_of_host.data();
+        g.ftab = s.tiled ? b.ft_k2t : b.ft_k2;
+        if (z.on) {                                          // K2T walks the compacted copy when the device-side decision says so
+            g.sel = h->sel_meta.as<uint32_t>() + z.meta_off; g.sel_ids = h->sel_ids.as<uint32_t>() + z.row_off;
+            g.sel_inv_norm = h->sel_inv.as<float>() + z.row_off;
+            g.sel_rows = h->sel_rows.as<unsigned char>() + z.row_off * h->d_pad * 2; g.sel_cap_rows = z.cap_rows;
+        }
+        int launches = 0;
+        if ((s.tiled ? vb_gemm_tiled_launch(g, &launches) : vb_gemm_launch(g, &launches)) != 0)
+            return vb_fail("tensor-core dense kernel: %s", vb_gemm_last_error());
+        h->stats.last_launches += (uint32_t)launches;
+    } else {
+        VbScanArgs a{};
+        a.rows = h->rows.as<uint4>();
+        a.inv_norm = h->inv_norm.as<float>();
+        set_mask(a, h, b);
+        a.q_hat = h->q_hat.as<float>();
+        a.tau = b.tau;
+        a.lists = s.L;
+        a.chunks = (uint32_t)h->d_pad / 8;
+        a.row_begin = r0;
+        a.row_end = r1;
+        a.row_base = (uint32_t)h->row_base;
+        a.q_begin = 0;
+        a.direct = direct;
+        const uint32_t groups = (r1 - r0 + 31) / 32;
+        const uint32_t per_q = std::max<uint32_t>(1, (uint32_t)(h->sm_count * 8) / std::min<uint32_t>(b.B, 8));
+        dim3 grid(std::min<uint32_t>((groups + 7) / 8, per_q), b.B);
+        const int nch = (int)((a.chunks + 31) / 32);
+        switch (nch) {
+            case 1: vb_dense_scan_kernel<1><<<grid, 256, 0, s.sd>>>(a); break;
+            case 2: vb_dense_scan_kernel<2><<<grid, 256, 0, s.sd>>>(a); break;
+            case 3: vb_dense_scan_kernel<3><<<grid, 256, 0, s.sd>>>(a); break;
+            case 4: vb_dense_scan_kernel<4><<<grid, 256, 0, s.sd>>>(a); break;
+            default: vb_dense_scan_generic_kernel<<<grid, 256, 0, s.sd>>>(a); break;
+        }
+        CKK("vb_dense_scan_kernel");
+        ++h->stats.last_launches;
+    }
+    prof_end(h, pi, s.sd);
+    return compact_lists(s, s.sd, 0u, direct ? std::max(s.direct_rows, s.L.sub_cap) : s.L.sub_cap);
+}
+
+// classes: bit 0 = plan + score the K3M queries, bit 1 = the K3H (long) queries
+static int ms_launch(Search& s, uint32_t r0, uint32_t r1, uint64_t stage_lo, uint64_t stage_hi, uint32_t classes) {
+    vb_index* h = s.h; const Batch& b = s.b;
+    VbMsPlanArgs pa{};
+    pa.classes = classes; pa.hunit_prefix = h->mh_units.as<uint32_t>();
+    pa.post_row = h->post_row.as<uint32_t>(); pa.term_tab = h->term_tab.as<uint32_t>(); pa.q_tab = b.d_qtab; pa.q_shift = b.d_qshift;
+    pa.n_rows = (uint32_t)h->base_rows; pa.q_indptr = b.d_qindptr; pa.q_weight = b.d_qweight; pa.q_ub = b.d_qub;
+    pa.q_hidx = b.any_heavy ? b.d_qhidx : nullptr; pa.q_plo = b.d_qplo; pa.q_phi = b.d_qphi; pa.q_ms = b.d_qms; pa.tau = b.tau;
+    pa.rec = h->ms_rec.as<VbMsRec>(); pa.qinfo = h->ms_q.as<VbMsQuery>(); pa.unit_prefix = h->ms_units.as<uint32_t>();
+    pa.counters = h->ms_counters.as<uint32_t>(); pa.n_queries = b.B; pa.n_qterms = b.n_qterms;
+    pa.seg_row0 = r0; pa.seg_row1 = r1; pa.stage_lo = stage_lo; pa.stage_hi = stage_hi;
+    pa.chunk = s.ms_chunk; pa.budget_pct = (uint32_t)std::max<int64_t>(0, h->opt_ms_budget);
+    pa.budget_pct_long = (uint32_t)std::max<int64_t>(0, h->opt_mh_budget);
+    pa.long_terms = VB_MS_LONG_TERMS; pa.budget_pct_mslong = VB_MS_BUDGET_LONG;
+    vb_ms_plan_kernel<<<b.B, 256, 0, s.ss>>>(pa);
+    CKK("vb_ms_plan_kernel");
+    ++h->stats.last_launches;
+    if (classes & 2u) {
+        VbMhArgs m{};
+        m.post_row = h->post_row.as<uint32_t>(); m.post_val = h->post_val.as<float>();
+        m.heavy_vals = h->heavy_vals.as<float>(); m.heavy_stride = h->heavy_stride; m.term_tab = h->term_tab.as<uint32_t>();
+        m.sp_indptr = h->sp_indptr.as<int64_t>(); m.sp_term = h->sp_term.as<uint32_t>(); m.sp_val = h->sp_val.as<float>();
+        m.q_indptr = b.d_qindptr; m.q_term = b.d_qterm; m.q_weight = b.d_qweight;
+        m.rec = h->ms_rec.as<VbMsRec>(); m.qinfo = h->ms_q.as<VbMsQuery>(); m.hunit_prefix = h->mh_units.as<uint32_t>();
+        m.counters = h->ms_counters.as<uint32_t>();
+        set_mask(m, h, b);
+        m.tau = b.tau; m.lists = s.L; m.n_queries = b.B; m.n_rows = (uint32_t)h->base_rows;
+        m.row_base = (uint32_t)h->row_base; m.nt_max = b.nt_max; m.seg_row0 = r0; m.seg_row1 = r1;
+        const uint64_t max_units = std::max<uint64_t>(1, (uint64_t)h->nnz_live / 256 + b.B);
+        const uint32_t grid = (uint32_t)std::min<uint64_t>((uint64_t)h->sm_count * 4u, max_units);
+        vb_mh_score_kernel<<<grid, VB_MH_THREADS, vb_mh_smem_bytes(b.nt_max), s.ss>>>(m);
+        CKK("vb_mh_score_kernel");
+        ++h->stats.last_launches;
+    }
+    if (!(classes & 1u)) return 0;
+    VbMsArgs a{};
+    a.post_row = h->post_row.as<uint32_t>(); a.post_val = h->post_val.as<float>();
+    a.heavy_vals = h->heavy_vals.as<float>(); a.heavy_stride = h->heavy_stride;
+    a.sp_indptr = h->sp_indptr.as<int64_t>(); a.sp_term = h->sp_term.as<uint32_t>(); a.sp_val = h->sp_val.as<float>();
+    a.q_indptr = b.d_qindptr; a.q_term = b.d_qterm; a.q_weight = b.d_qweight; a.slot_q = b.d_slotq;
+    a.rec = h->ms_rec.as<VbMsRec>(); a.qinfo = h->ms_q.as<VbMsQuery>(); a.unit_prefix = h->ms_units.as<uint32_t>();
+    a.counters = h->ms_counters.as<uint32_t>(); a.term_tab = h->term_tab.as<uint32_t>();
+    set_mask(a, h, b);
+    a.tau = b.tau; a.lists = s.L; a.n_qterms = b.n_qterms; a.n_queries = b.B;
+    a.row_base = (uint32_t)h->row_base; a.chunk = s.ms_chunk; a.nt_max = b.nt_max;
+    // persistent grid: enough CTAs to fill the machine (16 per SM: every register of the SM), never more than the
+    // largest possible unit count
+    const uint64_t span = std::min<uint64_t>(r1 - r0, stage_hi - stage_lo);
+    const uint64_t max_units = std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)h->nnz_live / s.ms_chunk + b.n_qterms, (uint64_t)b.n_qterms * (span / s.ms_chunk + 1)));
+    const uint32_t grid = (uint32_t)std::min<uint64_t>((uint64_t)h->sm_count * 16u, max_units);
+    vb_ms_score_kernel<<<grid, VB_MS_THREADS, vb_ms_smem_bytes(b.nt_max), s.ss>>>(a);
+    CKK("vb_ms_score_kernel");
+    ++h->stats.last_launches;
+    return 0;
+}
+static int sparse_segment(Search& s, size_t si, uint32_t direct, bool big) {
+    vb_index* h = s.h; const Batch& b = s.b;
+    const SparseRoute& r = s.sp;
+    const uint32_t r0 = s.bounds[si], r1 = std::min(s.bounds[si + 1], s.nb);   // the index stops at nb
+    const bool rows_here = s.do_sparse && r0 < r1;
+    const bool ms_here = rows_here && r.ms_on && !r.ms_staged && !direct;      // K3M once per segment (safe mode / ms_staged = 0)
+    const bool mh_here = rows_here && r.mh_on && !direct;                      // K3H for the long queries
+    const uint32_t* k3_list = direct ? r.k3_q_direct : r.k3_q;
+    const uint32_t k3_n = direct ? r.k3_n_direct : r.k3_n;
+    const bool k3_here = rows_here && k3_n > 0;
+    if (!direct && !ms_here && !mh_here && !k3_here) return 0;               // nothing scored, nothing to compact
+    if (ms_here || mh_here || k3_here) {
+        const int pi = prof_begin(h, PH_SPARSE | (big ? PH_BIG : 0), s.ss);
+        if (ms_here || mh_here) TRY(ms_launch(s, r0, r1, 0ull, ~0ull, (ms_here ? 1u : 0u) | (mh_here ? 2u : 0u)));
+        if (k3_here) {
+            // which terms are essential under the thresholds this segment starts with
+            double* d_ubne = h->plan.as<double>();
+            uint8_t* d_ess = reinterpret_cast<uint8_t*>(d_ubne + b.B);
+            // Pruning pays on long segments (measured: -10..-22 % sparse time from 2M rows per segment up, a loss
+            // on cfg2's 1M-row corpus where the per-survivor re-scoring outweighs the skipped postings).
+            const uint32_t nblk = (r1 - r0 + VB_ROWS_PER_BLOCK - 1) / VB_ROWS_PER_BLOCK;
+            const uint32_t budget = (!direct && (h->opt_sparse_prune_force || nblk >= 1000u)) ? (uint32_t)h->opt_sparse_prune : 0u;
+            if (budget) {                                       // no budget: every term is essential, no plan needed
+                vb_sparse_plan_kernel<<<b.B, 256, 0, s.ss>>>(b.d_qindptr, b.d_qub, b.tau, b.B, budget, d_ess, d_ubne);
+                CKK("vb_sparse_plan_kernel");
+                ++h->stats.last_launches;
+            }
+            VbSparseArgs a{};
+            a.post_row = h->post_row.as<uint32_t>(); a.post_val = h->post_val.as<float>(); a.off = h->offs.as<uint32_t>();
+            a.q_indptr = b.d_qindptr; a.q_weight = b.d_qweight; a.q_term = b.d_qterm; a.ess = budget ? d_ess : nullptr; a.ubne = d_ubne;
+            a.sp_indptr = h->sp_indptr.as<int64_t>(); a.sp_term = h->sp_term.as<uint32_t>(); a.sp_val = h->sp_val.as<float>();
+            a.q_hidx = b.any_heavy ? b.d_qhidx : nullptr; a.q_relaxed = b.d_qrelaxed; a.heavy_vals = h->heavy_vals.as<float>(); a.heavy_stride = h->heavy_stride;
+            set_mask(a, h, b);
+            a.tau = b.tau; a.lists = s.L;
+            a.n_qterms = b.n_qterms; a.nt_max = b.nt_max; a.blk_begin = r0 / VB_ROWS_PER_BLOCK; a.n_queries = b.B; a.n_rows = s.nb;
+            a.row_base = (uint32_t)h->row_base; a.direct = direct;
+            if (k3_list != nullptr) { a.q_sel = k3_list; a.n_sel = k3_n; }          // K3M / K3H have the rest
+            vb_sparse_kernel<<<nblk * k3_n, VB_SPARSE_THREADS, vb_sparse_smem_bytes(b.nt_max), s.ss>>>(a);
+            CKK("vb_sparse_kernel");
+            ++h->stats.last_launches;
+        }
+        prof_end(h, pi, s.ss);
+    }
+    // the sparse lists are compacted even without postings (first-segment slots -> empty lists)
+    return compact_lists(s, s.ss, b.B, direct ? std::max(s.direct_rows, s.L.sub_cap) : s.L.sub_cap);
+}
+// K3M stages (normal mode)
+static int ms_stages(Search& s) {
+    const Batch& b = s.b;
+    // stage 0 scores its postings with no threshold (every lookup of every posting): just enough of them to fill a
+    // list twice over after filters and ownership
+    const uint64_t p0 = std::max<uint64_t>(s.ms_chunk, std::min<uint64_t>(align_up((size_t)8 * b.k, s.ms_chunk), s.h->cand_cap / 4));
+    uint64_t lo = 0, hi = p0;
+    while (lo < b.ms_max_post) {
+        const bool last = hi >= b.ms_max_post;
+        const int pi = prof_begin(s.h, PH_SPARSE | (last ? PH_BIG : 0), s.ss);
+        TRY(ms_launch(s, 0u, s.nb, lo, last ? ~0ull : hi, 1u));
+        prof_end(s.h, pi, s.ss);
+        TRY(compact_lists(s, s.ss, b.B, s.L.sub_cap));
+        lo = hi;
+        // a stage appends ~ratio * k' candidates per list at worst (rows are visited best-first, usually far fewer)
+        const uint64_t ratio = std::min<uint64_t>(1024, std::max<uint64_t>(32, s.h->cand_cap / (16ull * b.k)));
+        hi = hi * ratio;
+    }
+    return 0;
+}
+// K3D: the rows appended since the index was built, straight from the forward CSR.  One launch (a few thousand rows
+// against thresholds the indexed rows have already established); the safe mode cuts it into pieces a list cannot
+// overflow on.
+static int sparse_delta(Search& s) {
+    vb_index* h = s.h; const Batch& b = s.b;
+    const uint32_t piece = s.safe_mode ? (uint32_t)std::max<size_t>(VB_ROWS_PER_BLOCK, h->cand_cap - b.k) : s.n - s.nb;
+    for (uint32_t r0 = s.nb; r0 < s.n; r0 += piece) {
+        const uint32_t r1 = (uint32_t)std::min<uint64_t>(s.n, (uint64_t)r0 + piece);
+        const int pi = prof_begin(h, PH_SPARSE, s.ss);
+        VbDeltaArgs a{};
+        a.sp_indptr = h->sp_indptr.as<int64_t>(); a.sp_term = h->sp_term.as<uint32_t>(); a.sp_val = h->sp_val.as<float>();
+        a.qt_term = b.d_ut; a.qt_ptr = b.d_up; a.qt_query = b.d_uq; a.qt_weight = b.d_uw;
+        set_mask(a, h, b);
+        a.tau = b.tau; a.lists = s.L; a.n_uterms = b.n_uterms; a.n_queries = b.B;
+        a.row_begin = r0; a.row_end = r1; a.row_base = (uint32_t)h->row_base;
+        const uint32_t warps = vb_delta_warps(b.B);
+        const size_t smem = (size_t)warps * b.B * 8;
+        if (smem > (size_t)g_delta_smem_max) return vb_fail("batch of %u queries is too large for the delta rows (%zu bytes of shared memory)", b.B, smem);
+        const uint32_t grid = std::min<uint32_t>((r1 - r0 + warps - 1) / warps, (uint32_t)h->sm_count * 8u);
+        vb_sparse_delta_kernel<<<grid, warps * 32, smem, s.ss>>>(a);
+        CKK("vb_sparse_delta_kernel");
+        ++h->stats.last_launches;
+        prof_end(h, pi, s.ss);
+        TRY(compact_lists(s, s.ss, b.B, s.L.sub_cap));
+    }
     return 0;
 }
 
 // Score both branches of this shard and leave the exact, sorted top-k' of every list in
 // cand[list][0..cnt).  `safe`: fixed small segments that can never overflow a list.
 static int run_branches(vb_index* h, const Batch& b, bool safe) {
-    const uint32_t n = (uint32_t)h->n_rows;
-    // segment schedule (boundaries are multiples of VB_ROWS_PER_BLOCK)
-    std::vector<uint32_t> bounds{0};
-    if (safe || h->opt_safe_mode) {
-        const uint32_t step = (uint32_t)std::max<size_t>(VB_ROWS_PER_BLOCK, (h->cand_cap - b.k) / VB_ROWS_PER_BLOCK * VB_ROWS_PER_BLOCK);
-        for (uint64_t r = step; r < n; r += step) bounds.push_back((uint32_t)r);
-    } else {
-        for (uint64_t r = (uint64_t)h->opt_seg_first; r < n; r *= (uint64_t)b.seg_ratio) bounds.push_back((uint32_t)r);
-    }
-    bounds.push_back(n);
-    const bool safe_mode = safe || h->opt_safe_mode;
-    const VbLists L = make_lists(h, b, safe_mode);
-    // dense path choice
-    int path = (int)h->opt_dense_path;
-    if (path == 0) path = vb_gemm_supported(h->d_pad, b.B) && b.B >= 2 ? 2 : 1;
-    if (path == 2 && !vb_gemm_supported(h->d_pad, b.B)) return vb_fail("dense_path=2 requested but unsupported for d_pad=%d B=%u", h->d_pad, b.B);
-    h->stats.last_dense_path = (uint32_t)path;
-    VbGemmPlan plan{1u, 0u};
-    if (path == 2) plan = vb_gemm_plan((uint32_t)h->d_pad, b.B, (int)h->opt_k2_precision);
-    // batches too large to sit resident in shared memory go to the query-tiled, tensor-bound kernel
-    // (one corpus pass per 1024 queries)
-    const bool tiled = path == 2 && b.B > plan.sub && !plan.split && h->opt_k2_tiled && vb_gemm_tiled_supported(h->d_pad);
-    h->stats.last_dense_passes = path == 2 ? (tiled ? (b.B + VB_TILED_MAX_Q - 1) / VB_TILED_MAX_Q : (b.B + plan.sub - 1) / plan.sub) : b.B;
-    // sparse work: the inverted index covers rows [0, nb); rows appended since (the delta) are scored by K3D
-    const uint32_t nb = (uint32_t)std::min<uint64_t>(h->base_rows, n);
-    const bool do_sparse = b.any_sparse && h->nnz_live > 0 && b.n_qterms > 0 && nb > 0;
-    const bool do_delta = b.any_sparse && b.n_uterms > 0 && nb < n;
-    // Which sparse kernel scores which query.  Queries whose products are all >= 0 and that are not too long go to
-    // K3M, the posting-driven MaxScore kernel; the others (and everything when K3M is off) stay on K3 (block x query
-    // CTAs over the row segments, first segment direct).
-    //   normal mode: K3M runs in STAGES over the whole index (sparse_ms.cuh): stage 0 scores the first ms_p0
-    //                postings of every query in descending-ub order with no threshold, each later stage 32x more;
-    //   safe mode:   K3M runs once per (small) row segment, like K3, so that no list can overflow.
-    const bool ms_on = do_sparse && b.any_ms && h->opt_sparse_ms;
-    const bool ms_staged = ms_on && !safe_mode && h->opt_ms_staged;
-    const bool mh_on = do_sparse && b.any_mh;                   // long queries: K3 direct segment, then K3H per segment
-    // K1F: one pass over all rows for tiny batches (no segments, no direct slots)
-    // (on large corpora the segmented K1 streams faster — no per-stretch barriers — and its launches are noise there:
-    //  cfg3 10M rows, B = 1: K1 1.65 ms, K1F 1.83 ms; cfg1 100k rows: K1 59 us + 3 selects, K1F 48 us + 1 merge)
-    const bool k1f = path == 1 && !safe_mode && h->opt_k1f && (h->opt_k1f > 1 || n <= (2u << 20)) && b.B <= VB_K1F_MAX_B && (h->d_pad / 8 + 31) / 32 <= 4 &&
-                     b.k <= VB_K1F_CAP / 2u && (uint64_t)vb_k1f_grid(h->sm_count, b.k, b.B, h->d_pad) * b.k <= h->cand_cap;
-    // the first segment writes its keys to fixed slots at the front of the list (no atomics) — unless nobody runs
-    // a first segment: K1F scans in one pass, K3M in posting stages
-    const bool k3_direct = do_sparse && (!ms_staged || b.n_dir > 0);
-    const uint32_t direct_rows = (bounds[1] <= h->cand_cap && (!k1f || k3_direct)) ? bounds[1] : 0u;
-    TRY(init_lists(h, b, direct_rows));
-    // list set-up + query prep (fp32 unit queries for K1, packed bf16 operand for K2) in ONE launch
-    TRY(dev_reserve(h, h->q_hat, (size_t)b.B * h->d_pad * 4, false));
-    TRY(dev_reserve(h, h->q_bf16, (size_t)(2 * ((size_t)b.B + 256)) * h->d_pad * 2, false));
-    TRY(dev_reserve(h, h->q_scale, (size_t)b.B * 4, false));
-    VbListInit li{};
-    li.tau = b.tau; li.cnt = b.cnt; li.overflow = b.overflow; li.gtau = b.gtau; li.n = b.n_lists; li.cnt0 = direct_rows;
-    li.no_direct = ms_staged ? b.d_qms : nullptr; li.n_queries = b.B; li.dense_direct = k1f ? 0u : 1u;
-    vb_prep_query_kernel<<<b.B, 128, 0, h->stream>>>(b.d_q, (uint32_t)h->dim, (uint32_t)h->d_pad, b.B, plan.sub, plan.split,
-                                                     h->q_hat.as<float>(), h->q_bf16.as<__nv_bfloat16>(), h->q_scale.as<float>(),
-                                                     reinterpret_cast<uint32_t*>(h->out.as<unsigned char>() + b.o_bad), li);
-    CKK("vb_prep_query_kernel");
-    ++h->stats.last_launches;
-    // K0 filter masks
-    if (b.use_mask) {
-        prof_begin(h, PH_MASK);
-        const size_t mask_bytes = (size_t)b.n_filters * b.mask_words * 4;
-        if (dev_reserve(h, h->mask, mask_bytes, false) != 0) {
-            cudaGetLastError();
-            return vb_fail("filter masks of %u distinct filters over %u rows need %zu bytes of device memory: %s",
-                           b.n_filters, n, mask_bytes, g_err.c_str());
-        }
-        vb_mask_kernel<<<grid_for((uint64_t)b.mask_words * 32, 256, h->sm_count * 8), 256, 0, h->stream>>>(
-            h->scope_id.as<uint32_t>(), h->created.as<int64_t>(), h->modified.as<int64_t>(), h->alive.as<uint32_t>(), n,
-            b.d_filters, b.n_filters, b.mask_words, b.need_created, b.need_modified, b.need_scope, h->mask.as<uint32_t>());
-        CKK("vb_mask_kernel");
-        ++h->stats.last_launches;
-        prof_end(h);
-    }
+    Search s{h, b};
+    schedule_segments(s, safe);
+    TRY(choose_kernels(s));
+    TRY(prep_and_mask(s));
     // The dense chain (K1/K2 + select of the dense lists) and the sparse chain (slice table, K3 +
     // select of the sparse lists) are independent until the fusion, so they run on two streams:
     // the small kernels of one chain (selects, first segments, slice table) hide behind the big
     // kernels of the other.
-    const bool two_streams = (do_sparse || do_delta) && h->opt_overlap;
-    cudaStream_t sd = h->stream, ss = two_streams ? h->aux_stream : h->stream;
+    const bool two_streams = (s.do_sparse || s.do_delta) && h->opt_overlap;
     if (two_streams) {
-        CK(cudaEventRecord(h->ev_fork, sd));
-        CK(cudaStreamWaitEvent(ss, h->ev_fork, 0));
+        s.ss = h->aux_stream;
+        CK(cudaEventRecord(h->ev_fork, s.sd));
+        CK(cudaStreamWaitEvent(s.ss, h->ev_fork, 0));
     }
-    // ---- K2T row selection plan (dense_compact.cuh): the tensor-bound kernel, ONE filter for the whole batch, every
-    // segment of at least dense_compact_min_rows rows.  Count, list and copy run on a side stream right after the mask
-    // kernel: the copy of segment s + 1 (HBM-bound) hides behind the GEMM of segment s (tensor-bound).  With the chains
-    // serialised (overlap = 0: per-phase timing) they run inline on the dense stream and are charged to the dense phase.
-    // The copy is kept across batches (h->sel_key): a segment whose key matches the scratch is not copied again, and
-    // the tensor-core kernel reads the scratch and its device-side {count, decision} as they are.
-    struct SelSeg { bool on = false, kept = false; uint32_t cap_rows = 0, n_blocks = 0, ev = 0; size_t row_off = 0, meta_off = 0; };
-    std::vector<SelSeg> selseg(bounds.size() - 1);
-    bool sel_any = false, sel_copy = false;
-    std::vector<uint64_t> sel_key;
-    const bool sel_side = h->opt_overlap != 0;
-    // auto threshold: the copy costs ~0.49 ns per passing row (read + write of 2 * d_pad bytes at HBM speed, d_pad = 768);
-    // one pass of the tensor-core kernel over a row costs max(0.245 ns (HBM), 1.08 ns * queries / 1024 (tensor pipe)) — both
-    // scale with d_pad alike.  Copying pays when (1 - p) * passes' time > p * copy time.
-    uint32_t sel_pct = (uint32_t)std::max<int64_t>(0, std::min<int64_t>(100, h->opt_dense_compact));
-    if (h->opt_dense_compact < 0 && path == 2) {
-        double T = 0.0;
-        if (tiled) for (uint32_t q0 = 0; q0 < b.B; q0 += VB_TILED_MAX_Q) T += std::max(0.245, 1.08 * std::min(VB_TILED_MAX_Q, b.B - q0) / 1024.0);
-        else T = 0.245 * ((b.B + plan.sub - 1) / plan.sub);
-        sel_pct = (uint32_t)(95.0 * T / (T + 0.49));
-    }
-    if (path == 2 && !k1f && b.use_mask && sel_pct > 0 && !h->sel_no_memory && h->d_pad <= 1024) {
-        bool uniform = b.mask_of_host[0] >= 0;
-        for (uint32_t i = 1; uniform && i < b.B; ++i) uniform = b.mask_of_host[i] == b.mask_of_host[0];
-        size_t rows_total = 0, meta_total = 0;
-        uint32_t n_on = 0;
-        for (size_t si = (direct_rows ? 1 : 0); uniform && si + 1 < bounds.size() && n_on < 8u; ++si) {
-            const uint32_t r0 = bounds[si], r1 = bounds[si + 1];
-            if ((r0 % 128u) != 0u || (int64_t)(r1 - r0) < h->opt_dense_compact_min_rows) continue;
-            SelSeg& z = selseg[si];
-            z.on = true; z.cap_rows = (uint32_t)align_up(r1 - r0, 128); z.n_blocks = ((r1 - r0 + 31u) / 32u + VB_SEL_WORDS - 1u) / VB_SEL_WORDS;
-            z.row_off = rows_total; z.meta_off = meta_total; z.ev = n_on++;
-            rows_total += z.cap_rows; meta_total += align_up((size_t)4 + z.n_blocks, 4);
-        }
-        const size_t scratch = rows_total * h->d_pad * 2;
-        if (n_on && scratch > h->sel_rows.cap) {
-            size_t free_b = 0, total_b = 0;
-            if (cudaMemGetInfo(&free_b, &total_b) != cudaSuccess || free_b + h->sel_rows.cap < scratch + (4ull << 30)) {
-                cudaGetLastError();
-                h->sel_no_memory = true;                         // the scratch matrix does not fit beside the shard: stay in place
-                h->sel_key.clear();
-                n_on = 0;
-            }
-        }
-        if (n_on) {
-            const void* before[4] = {h->sel_rows.p, h->sel_inv.p, h->sel_ids.p, h->sel_meta.p};
-            // Invalid from here until this batch has enqueued all of its work (end of run_branches): an error return
-            // in between (a failed reserve, a copy enqueued in part) leaves the next batch to copy again.
-            std::vector<uint64_t> cached_key;
-            cached_key.swap(h->sel_key);
-            TRY(dev_reserve(h, h->sel_rows, scratch, false));
-            TRY(dev_reserve(h, h->sel_inv, rows_total * 4, false));
-            TRY(dev_reserve(h, h->sel_ids, rows_total * 4, false));
-            TRY(dev_reserve(h, h->sel_meta, meta_total * 4, false));
-            const bool moved = before[0] != h->sel_rows.p || before[1] != h->sel_inv.p || before[2] != h->sel_ids.p || before[3] != h->sel_meta.p;
-            sel_any = true;
-            // the key: filter content, index version, and every input of the plan above
-            sel_key = b.sel_filter;
-            sel_key.insert(sel_key.end(), {h->write_gen, (uint64_t)n, (uint64_t)h->d_pad, sel_pct, (uint64_t)h->opt_dense_compact_min_rows,
-                                           (uint64_t)path, (uint64_t)tiled, direct_rows});
-            const bool key_holds = h->opt_sel_reuse && !moved && sel_key == cached_key;
-            for (size_t si = 0; si < selseg.size(); ++si) {
-                SelSeg& z = selseg[si];
-                if (!z.on) continue;
-                const std::array<uint64_t, 5> zk{bounds[si], bounds[si + 1], z.row_off, z.meta_off, z.cap_rows};
-                z.kept = key_holds && std::find(h->sel_segs.begin(), h->sel_segs.end(), zk) != h->sel_segs.end();
-                sel_copy |= !z.kept;
-            }
-        } else for (auto& z : selseg) z.on = false;
-    }
-    auto sel_launch = [&](size_t si, cudaStream_t st) -> int {
-        const SelSeg& z = selseg[si];
-        const uint32_t r0 = bounds[si], r1 = bounds[si + 1];
-        VbRowSelArgs sa{};
-        sa.mask = h->mask.as<uint32_t>() + (size_t)b.mask_of_host[0] * b.mask_words;
-        sa.word_begin = r0 / 32u; sa.word_end = (r1 + 31u) / 32u; sa.row_end = r1;
-        sa.sel = h->sel_meta.as<uint32_t>() + z.meta_off; sa.block_sums = sa.sel + 4; sa.ids = h->sel_ids.as<uint32_t>() + z.row_off;
-        sa.pct = sel_pct; sa.pad_row = r0; sa.cap_rows = z.cap_rows;
-        vb_rowsel_count_kernel<<<z.n_blocks, VB_SEL_THREADS, 0, st>>>(sa);
-        CKK("vb_rowsel_count_kernel");
-        vb_rowsel_scatter_kernel<<<z.n_blocks, VB_SEL_THREADS, 0, st>>>(sa);
-        CKK("vb_rowsel_scatter_kernel");
-        vb_rowsel_gather_kernel<<<h->sm_count * 4, 256, 0, st>>>(h->rows.as<uint4>(), h->inv_norm.as<float>(), sa.ids, sa.sel,
-                                                                h->sel_rows.as<uint4>() + z.row_off * (h->d_pad / 8), h->sel_inv.as<float>() + z.row_off,
-                                                                (uint32_t)h->d_pad / 8u);
-        CKK("vb_rowsel_gather_kernel");
-        h->stats.last_launches += 3;
-        return 0;
-    };
-    // Ordering of the scratch (two batches can be in flight).  A kept segment is only read, by kernels on the dense
-    // stream.  A copy waits for ev_sel_fork, recorded on the dense stream after this batch's mask kernel and therefore
-    // after every kernel an earlier batch enqueued there, so it cannot overwrite the scratch while an earlier batch's
-    // tensor-core kernel still reads it — whether that batch copied or kept.  A batch that keeps a copy made by an earlier
-    // one reads it after that batch's dense kernels, which waited for the copy's events: the copy has finished.
-    if (sel_copy && sel_side) {
-        if (!h->sel_stream) {
-            CK(cudaStreamCreateWithFlags(&h->sel_stream, cudaStreamNonBlocking));
-            CK(cudaEventCreateWithFlags(&h->ev_sel_fork, cudaEventDisableTiming));
-            for (auto& e : h->ev_sel) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-        }
-        CK(cudaEventRecord(h->ev_sel_fork, sd));                 // after the mask kernel (and after the previous batch's dense chain)
-        CK(cudaStreamWaitEvent(h->sel_stream, h->ev_sel_fork, 0));
-        for (size_t si = 0; si < selseg.size(); ++si)
-            if (selseg[si].on && !selseg[si].kept) {
-                TRY(sel_launch(si, h->sel_stream));
-                CK(cudaEventRecord(h->ev_sel[selseg[si].ev], h->sel_stream));
-            }
-    }
-    auto dense_single_pass = [&]() -> int {
-        const int pi = prof_begin(h, PH_DENSE | PH_BIG, sd);
-        VbScan1Args a{};
-        a.rows = h->rows.as<uint4>(); a.inv_norm = h->inv_norm.as<float>();
-        a.mask = b.use_mask ? h->mask.as<uint32_t>() : nullptr; a.mask_of = b.use_mask ? b.d_maskof : nullptr;
-        a.q_hat = h->q_hat.as<float>(); a.gtau = b.gtau; a.cand = h->cand.as<uint64_t>(); a.cnt = b.cnt;
-        a.cap = h->cand_cap; a.k = b.k; a.mask_words = b.mask_words; a.chunks = (uint32_t)h->d_pad / 8; a.n_rows = n;
-        a.row_base = (uint32_t)h->row_base;
-        a.done = b.done; a.tau = b.tau;
-        const dim3 grid(vb_k1f_grid(h->sm_count, b.k, b.B, h->d_pad), b.B);
-        // small corpora: fewer 32-row groups than warps — give each warp a half / quarter / eighth of a group
-        const uint32_t n_groups = (n + 31u) / 32u, n_warps = grid.x * (VB_K1F_THREADS / 32u);
-        a.split_shift = 0;
-        while (a.split_shift < 3u && (n_groups << (a.split_shift + 1u)) <= n_warps) ++a.split_shift;
-        // large corpora: units of 2..32 groups (one coalesced filter-word load per unit, row batches filled across its
-        // groups), as long as every warp still gets >= 4 units (static interleaved assignment: +-1 unit of imbalance)
-        a.unit_shift = 0;
-        if (!a.split_shift)
-            while (a.unit_shift < 5u && (n_groups >> (a.unit_shift + 1u)) >= 4u * n_warps) ++a.unit_shift;
-        switch ((a.chunks + 31) / 32) {
-            case 1: vb_dense_scan1_kernel<1><<<grid, VB_K1F_THREADS, 0, sd>>>(a); break;
-            case 2: vb_dense_scan1_kernel<2><<<grid, VB_K1F_THREADS, 0, sd>>>(a); break;
-            case 3: vb_dense_scan1_kernel<3><<<grid, VB_K1F_THREADS, 0, sd>>>(a); break;
-            default: vb_dense_scan1_kernel<4><<<grid, VB_K1F_THREADS, 0, sd>>>(a); break;
-        }
-        CKK("vb_dense_scan1_kernel");
-        ++h->stats.last_launches;
-        prof_end(h, pi, sd);                                    // (the merge of the per-CTA lists happens inside: last CTA)
-        h->stats.last_big_rows = n;
-        h->stats.last_dense_path = 3u;                          // K1F
-        return 0;
-    };
-    auto dense_segment = [&](uint32_t r0, uint32_t r1, uint32_t direct, bool big) -> int {
-        if (k1f) return 0;                                      // the single pass covers every segment
-        // Row selection (planned before the segment loop): nothing to do when the scratch kept this segment's copy;
-        // otherwise wait for its copy (side stream), or run the selection here (chains serialised: its own timed region
-        // of the dense phase, so that the PH_BIG region stays the tensor-core kernel alone)
-        const SelSeg* zsel = nullptr;
-        if (path == 2)
-            for (size_t si = 0; si + 1 < bounds.size(); ++si)
-                if (bounds[si] == r0 && selseg[si].on) {
-                    zsel = &selseg[si];
-                    if (!zsel->kept && sel_side) CK(cudaStreamWaitEvent(sd, h->ev_sel[zsel->ev], 0));
-                    else if (!zsel->kept) {
-                        const int pz = prof_begin(h, PH_DENSE, sd);
-                        TRY(sel_launch(si, sd));
-                        prof_end(h, pz, sd);
-                    }
-                    if (big) {                                   // {rows, decision} of the roofline's segment for vb_stats
-                        TRY(host_reserve(h->h_sel[h->cur], 16));
-                        CK(cudaMemcpyAsync(h->h_sel[h->cur].p, h->sel_meta.as<uint32_t>() + zsel->meta_off, 8, cudaMemcpyDeviceToHost, sd));
-                        h->sel_ran[h->cur] = true;
-                    }
-                }
-        const int pi = prof_begin(h, PH_DENSE | (big ? PH_BIG : 0), sd);
-        if (path == 2) {
-            VbGemmLaunch g{};
-            g.rows = h->rows.p; g.inv_norm = h->inv_norm.as<float>(); g.q_bf16 = h->q_bf16.p;
-            g.mask = b.use_mask ? h->mask.as<uint32_t>() : nullptr; g.mask_of = b.use_mask ? b.d_maskof : nullptr;
-            g.mask_words = b.mask_words; g.n_filters = b.n_filters; g.tau = b.tau; g.q_scale = h->q_scale.as<float>(); g.lists = L;
-            g.n_rows_total = n; g.row_begin = r0; g.row_end = r1; g.row_base = (uint32_t)h->row_base;
-            g.d_pad = (uint32_t)h->d_pad; g.n_queries = b.B; g.sm_count = h->sm_count; g.stream = sd;
-            g.direct = direct; g.plan = plan; g.mask_of_host = b.mask_of_host.data();
-            g.ftab = tiled ? b.ft_k2t : b.ft_k2;
-            if (zsel) {                                          // K2T walks the compacted copy when the device-side decision says so
-                g.sel = h->sel_meta.as<uint32_t>() + zsel->meta_off; g.sel_ids = h->sel_ids.as<uint32_t>() + zsel->row_off;
-                g.sel_inv_norm = h->sel_inv.as<float>() + zsel->row_off;
-                g.sel_rows = h->sel_rows.as<unsigned char>() + zsel->row_off * h->d_pad * 2; g.sel_cap_rows = zsel->cap_rows;
-            }
-            int launches = 0;
-            if ((tiled ? vb_gemm_tiled_launch(g, &launches) : vb_gemm_launch(g, &launches)) != 0)
-                return vb_fail("tensor-core dense kernel: %s", vb_gemm_last_error());
-            h->stats.last_launches += (uint32_t)launches;
-        } else {
-            TRY(launch_scan(h, b, L, r0, r1, direct, sd));
-        }
-        prof_end(h, pi, sd);
-        const int ps = prof_begin(h, PH_SELECT, sd);
-        vb_compact_kernel<<<b.B, VB_COMPACT_THREADS, 0, sd>>>(L, b.tau, b.overflow, b.k, 0u, direct ? std::max(direct_rows, L.sub_cap) : L.sub_cap);
-        CKK("vb_compact_kernel");
-        ++h->stats.last_launches;
-        prof_end(h, ps, sd);
-        return 0;
-    };
-    const uint32_t ms_chunk = h->opt_ms_chunk > 0 ? (uint32_t)align_up((size_t)h->opt_ms_chunk, VB_MS_U * VB_MS_THREADS)
-                                                   : 512u;
-    // classes: bit 0 = plan + score the K3M queries, bit 1 = the K3H (long) queries
-    auto ms_launch = [&](uint32_t r0, uint32_t r1, uint64_t stage_lo, uint64_t stage_hi, uint32_t classes) -> int {
-        VbMsPlanArgs pa{};
-        pa.classes = classes; pa.hunit_prefix = h->mh_units.as<uint32_t>();
-        pa.post_row = h->post_row.as<uint32_t>(); pa.term_tab = h->term_tab.as<uint32_t>(); pa.q_tab = b.d_qtab; pa.q_shift = b.d_qshift;
-        pa.n_rows = (uint32_t)h->base_rows; pa.q_indptr = b.d_qindptr; pa.q_weight = b.d_qweight; pa.q_ub = b.d_qub;
-        pa.q_hidx = b.any_heavy ? b.d_qhidx : nullptr; pa.q_plo = b.d_qplo; pa.q_phi = b.d_qphi; pa.q_ms = b.d_qms; pa.tau = b.tau;
-        pa.rec = h->ms_rec.as<VbMsRec>(); pa.qinfo = h->ms_q.as<VbMsQuery>(); pa.unit_prefix = h->ms_units.as<uint32_t>();
-        pa.counters = h->ms_counters.as<uint32_t>(); pa.n_queries = b.B; pa.n_qterms = b.n_qterms;
-        pa.seg_row0 = r0; pa.seg_row1 = r1; pa.stage_lo = stage_lo; pa.stage_hi = stage_hi;
-        pa.chunk = ms_chunk; pa.budget_pct = (uint32_t)std::max<int64_t>(0, h->opt_ms_budget);
-        pa.budget_pct_long = (uint32_t)std::max<int64_t>(0, h->opt_mh_budget);
-        pa.long_terms = VB_MS_LONG_TERMS; pa.budget_pct_mslong = VB_MS_BUDGET_LONG;
-        vb_ms_plan_kernel<<<b.B, 256, 0, ss>>>(pa);
-        CKK("vb_ms_plan_kernel");
-        ++h->stats.last_launches;
-        if (classes & 2u) {
-            VbMhArgs m{};
-            m.post_row = h->post_row.as<uint32_t>(); m.post_val = h->post_val.as<float>();
-            m.heavy_vals = h->heavy_vals.as<float>(); m.heavy_stride = h->heavy_stride; m.term_tab = h->term_tab.as<uint32_t>();
-            m.sp_indptr = h->sp_indptr.as<int64_t>(); m.sp_term = h->sp_term.as<uint32_t>(); m.sp_val = h->sp_val.as<float>();
-            m.q_indptr = b.d_qindptr; m.q_term = b.d_qterm; m.q_weight = b.d_qweight;
-            m.rec = h->ms_rec.as<VbMsRec>(); m.qinfo = h->ms_q.as<VbMsQuery>(); m.hunit_prefix = h->mh_units.as<uint32_t>();
-            m.counters = h->ms_counters.as<uint32_t>();
-            m.mask = b.use_mask ? h->mask.as<uint32_t>() : nullptr; m.mask_of = b.use_mask ? b.d_maskof : nullptr;
-            m.tau = b.tau; m.lists = L; m.mask_words = b.mask_words; m.n_queries = b.B; m.n_rows = (uint32_t)h->base_rows;
-            m.row_base = (uint32_t)h->row_base; m.nt_max = b.nt_max; m.seg_row0 = r0; m.seg_row1 = r1;
-            const uint64_t max_units = std::max<uint64_t>(1, (uint64_t)h->nnz_live / 256 + b.B);
-            const uint32_t grid = (uint32_t)std::min<uint64_t>((uint64_t)h->sm_count * 4u, max_units);
-            vb_mh_score_kernel<<<grid, VB_MH_THREADS, vb_mh_smem_bytes(b.nt_max), ss>>>(m);
-            CKK("vb_mh_score_kernel");
-            ++h->stats.last_launches;
-        }
-        if (!(classes & 1u)) return 0;
-        VbMsArgs a{};
-        a.post_row = h->post_row.as<uint32_t>(); a.post_val = h->post_val.as<float>();
-        a.heavy_vals = h->heavy_vals.as<float>(); a.heavy_stride = h->heavy_stride;
-        a.sp_indptr = h->sp_indptr.as<int64_t>(); a.sp_term = h->sp_term.as<uint32_t>(); a.sp_val = h->sp_val.as<float>();
-        a.q_indptr = b.d_qindptr; a.q_term = b.d_qterm; a.q_weight = b.d_qweight; a.slot_q = b.d_slotq;
-        a.rec = h->ms_rec.as<VbMsRec>(); a.qinfo = h->ms_q.as<VbMsQuery>(); a.unit_prefix = h->ms_units.as<uint32_t>();
-        a.counters = h->ms_counters.as<uint32_t>(); a.term_tab = h->term_tab.as<uint32_t>();
-        a.mask = b.use_mask ? h->mask.as<uint32_t>() : nullptr; a.mask_of = b.use_mask ? b.d_maskof : nullptr;
-        a.tau = b.tau; a.lists = L; a.mask_words = b.mask_words; a.n_qterms = b.n_qterms; a.n_queries = b.B;
-        a.row_base = (uint32_t)h->row_base; a.chunk = ms_chunk; a.nt_max = b.nt_max;
-        // persistent grid: enough CTAs to fill the machine (16 per SM: every register of the SM), never more than the
-        // largest possible unit count
-        const uint64_t span = std::min<uint64_t>(r1 - r0, stage_hi - stage_lo);
-        const uint64_t max_units = std::max<uint64_t>(1, std::min<uint64_t>((uint64_t)h->nnz_live / ms_chunk + b.n_qterms, (uint64_t)b.n_qterms * (span / ms_chunk + 1)));
-        const uint32_t grid = (uint32_t)std::min<uint64_t>((uint64_t)h->sm_count * 16u, max_units);
-        vb_ms_score_kernel<<<grid, VB_MS_THREADS, vb_ms_smem_bytes(b.nt_max), ss>>>(a);
-        CKK("vb_ms_score_kernel");
-        ++h->stats.last_launches;
-        return 0;
-    };
-    auto sparse_compact = [&](uint32_t lim0) -> int {
-        const int ps = prof_begin(h, PH_SELECT, ss);
-        vb_compact_kernel<<<b.B, VB_COMPACT_THREADS, 0, ss>>>(L, b.tau, b.overflow, b.k, b.B, lim0);
-        CKK("vb_compact_kernel");
-        ++h->stats.last_launches;
-        prof_end(h, ps, ss);
-        return 0;
-    };
-    // K3 scores: every sparse query if K3M is off; else the queries K3M does not take (b.d_oldq) — plus, in the
-    // segment flow, everybody in the direct segment
-    auto sparse_segment = [&](uint32_t r0, uint32_t r1_all, uint32_t direct, bool big) -> int {
-        const uint32_t r1 = std::min(r1_all, nb);               // the index stops at nb
-        const bool rows_here = do_sparse && r0 < r1;
-        const bool ms_here = rows_here && ms_on && !ms_staged && !direct;      // K3M once per segment (safe mode / ms_staged = 0)
-        const bool mh_here = rows_here && mh_on && !direct;                    // K3H for the long queries
-        // K3's queries here: everybody (no K3M / K3H at all, or the direct segment of the per-segment flow); in the
-        // direct segment of the staged flow the K3 + K3H queries; otherwise only the ones nobody else takes
-        const uint32_t* k3_list = nullptr;
-        uint32_t k3_n = b.B;
-        if (ms_on || mh_on) {
-            if (!direct) { k3_list = b.d_oldq; k3_n = b.n_old; }
-            else if (ms_staged) { k3_list = b.d_dirq; k3_n = b.n_dir; }
-        }
-        const bool k3_here = rows_here && k3_n > 0;
-        if (!direct && !ms_here && !mh_here && !k3_here) return 0;             // nothing scored, nothing to compact
-        if (ms_here || mh_here || k3_here) {
-            const int pi = prof_begin(h, PH_SPARSE | (big ? PH_BIG : 0), ss);
-            if (ms_here || mh_here) TRY(ms_launch(r0, r1, 0ull, ~0ull, (ms_here ? 1u : 0u) | (mh_here ? 2u : 0u)));
-            if (k3_here) {
-                // which terms are essential under the thresholds this segment starts with
-                double* d_ubne = h->plan.as<double>();
-                uint8_t* d_ess = reinterpret_cast<uint8_t*>(d_ubne + b.B);
-                // Pruning pays on long segments (measured: -10..-22 % sparse time from 2M rows per segment up, a loss
-                // on cfg2's 1M-row corpus where the per-survivor re-scoring outweighs the skipped postings).
-                const uint32_t nblk_seg = (r1 - r0 + VB_ROWS_PER_BLOCK - 1) / VB_ROWS_PER_BLOCK;
-                const uint32_t budget = (!direct && (h->opt_sparse_prune_force || nblk_seg >= 1000u)) ? (uint32_t)h->opt_sparse_prune : 0u;
-                if (budget) {                                       // no budget: every term is essential, no plan needed
-                    vb_sparse_plan_kernel<<<b.B, 256, 0, ss>>>(b.d_qindptr, b.d_qub, b.tau, b.B, budget, d_ess, d_ubne);
-                    CKK("vb_sparse_plan_kernel");
-                    ++h->stats.last_launches;
-                }
-                VbSparseArgs a{};
-                a.post_row = h->post_row.as<uint32_t>(); a.post_val = h->post_val.as<float>(); a.off = h->offs.as<uint32_t>();
-                a.q_indptr = b.d_qindptr; a.q_weight = b.d_qweight; a.q_term = b.d_qterm; a.ess = budget ? d_ess : nullptr; a.ubne = d_ubne;
-                a.sp_indptr = h->sp_indptr.as<int64_t>(); a.sp_term = h->sp_term.as<uint32_t>(); a.sp_val = h->sp_val.as<float>();
-                a.q_hidx = b.any_heavy ? b.d_qhidx : nullptr; a.q_relaxed = b.d_qrelaxed; a.heavy_vals = h->heavy_vals.as<float>(); a.heavy_stride = h->heavy_stride;
-                a.mask = b.use_mask ? h->mask.as<uint32_t>() : nullptr; a.mask_of = b.use_mask ? b.d_maskof : nullptr;
-                a.tau = b.tau; a.lists = L; a.mask_words = b.mask_words;
-                a.n_qterms = b.n_qterms; a.nt_max = b.nt_max; a.blk_begin = r0 / VB_ROWS_PER_BLOCK; a.n_queries = b.B; a.n_rows = nb;
-                a.row_base = (uint32_t)h->row_base; a.direct = direct;
-                const uint32_t n_q = k3_n;
-                if (k3_list != nullptr) { a.q_sel = k3_list; a.n_sel = k3_n; }          // K3M / K3H have the rest
-                const uint32_t nblk = (r1 - r0 + VB_ROWS_PER_BLOCK - 1) / VB_ROWS_PER_BLOCK;
-                vb_sparse_kernel<<<nblk * n_q, VB_SPARSE_THREADS, vb_sparse_smem_bytes(b.nt_max), ss>>>(a);
-                CKK("vb_sparse_kernel");
-                ++h->stats.last_launches;
-            }
-            prof_end(h, pi, ss);
-        }
-        // the sparse lists are compacted even without postings (first-segment slots -> empty lists)
-        return sparse_compact(direct ? std::max(direct_rows, L.sub_cap) : L.sub_cap);
-    };
-    // fine (2048-row) slice table rows K3 will read
-    const bool k3_all_segments = do_sparse && ((!ms_on && !mh_on) || b.any_old);
-    const uint32_t fine_blocks = k3_all_segments ? b.n_blocks
-                                 : (k3_direct ? std::min<uint32_t>(b.n_blocks, (direct_rows + VB_ROWS_PER_BLOCK - 1) / VB_ROWS_PER_BLOCK) : 0u);
-    if (do_sparse) {
-        const uint64_t total = (uint64_t)b.n_qterms * (fine_blocks + 1);
+    TRY(plan_rowsel(s));
+    if (s.do_sparse) {                                      // scratch of the sparse chain, slice tables (sparse stream)
+        const uint64_t total = (uint64_t)b.n_qterms * (s.sp.fine_blocks + 1);
         TRY(dev_reserve(h, h->offs, std::max<uint64_t>(total, 1) * 4, false));
         TRY(dev_reserve(h, h->plan, (size_t)b.B * 8 + b.n_qterms + 64, false));
-        if (ms_on || mh_on) {
+        if (s.sp.ms_on || s.sp.mh_on) {
             TRY(dev_reserve(h, h->mh_units, ((size_t)b.B + 1) * 4, false));
             TRY(dev_reserve(h, h->ms_rec, (size_t)b.n_qterms * sizeof(VbMsRec), false));
             TRY(dev_reserve(h, h->ms_q, (size_t)b.B * sizeof(VbMsQuery), false));
             TRY(dev_reserve(h, h->ms_units, ((size_t)b.n_qterms + 1) * 4, false));
             TRY(dev_reserve(h, h->ms_counters, 64, false));
         }
-    }
-    if (do_sparse) {                                            // sparse slice tables (sparse chain)
-        const int pi = prof_begin(h, PH_SPARSE, ss);
-        const uint64_t total = (uint64_t)b.n_qterms * (fine_blocks + 1);
-        if (fine_blocks) {
-            vb_slice_kernel<<<grid_for(total, 256), 256, 0, ss>>>(h->post_row.as<uint32_t>(), b.d_qlo, b.d_qhi, b.n_qterms, fine_blocks, h->offs.as<uint32_t>());
+        const int pi = prof_begin(h, PH_SPARSE, s.ss);
+        if (s.sp.fine_blocks) {
+            vb_slice_kernel<<<grid_for(total, 256), 256, 0, s.ss>>>(h->post_row.as<uint32_t>(), b.d_qlo, b.d_qhi, b.n_qterms, s.sp.fine_blocks, h->offs.as<uint32_t>());
             CKK("vb_slice_kernel");
             ++h->stats.last_launches;
         }
-        if (ms_on || mh_on) CK(cudaMemsetAsync(h->ms_counters.p, 0, 64, ss));
-        prof_end(h, pi, ss);
+        if (s.sp.ms_on || s.sp.mh_on) CK(cudaMemsetAsync(h->ms_counters.p, 0, 64, s.ss));
+        prof_end(h, pi, s.ss);
     }
-    // K3M stages (normal mode)
-    auto ms_stages = [&]() -> int {
-        // stage 0 scores its postings with no threshold (every lookup of every posting): just enough of them to fill a
-        // list twice over after filters and ownership
-        const uint64_t p0 = std::max<uint64_t>(ms_chunk, std::min<uint64_t>(align_up((size_t)8 * b.k, ms_chunk), h->cand_cap / 4));
-        uint64_t lo = 0, hi = p0;
-        while (lo < b.ms_max_post) {
-            const bool last = hi >= b.ms_max_post;
-            const int pi = prof_begin(h, PH_SPARSE | (last ? PH_BIG : 0), ss);
-            TRY(ms_launch(0u, nb, lo, last ? ~0ull : hi, 1u));
-            prof_end(h, pi, ss);
-            TRY(sparse_compact(L.sub_cap));
-            lo = hi;
-            // a stage appends ~ratio * k' candidates per list at worst (rows are visited best-first, usually far fewer)
-            const uint64_t ratio = std::min<uint64_t>(1024, std::max<uint64_t>(32, h->cand_cap / (16ull * b.k)));
-            hi = hi * ratio;
-        }
-        return 0;
-    };
     // enqueue the two chains interleaved so that neither stream starves on the host side
-    const size_t n_seg = bounds.size() - 1;
+    const size_t n_seg = s.bounds.size() - 1;
     size_t big_seg = 0;
-    for (size_t s = 1; s < n_seg; ++s) if (bounds[s + 1] - bounds[s] > bounds[big_seg + 1] - bounds[big_seg]) big_seg = s;
+    for (size_t si = 1; si < n_seg; ++si) if (s.bounds[si + 1] - s.bounds[si] > s.bounds[big_seg + 1] - s.bounds[big_seg]) big_seg = si;
     // Order on the sparse stream: K3's direct first segment (fixed slots, counted by the list set-up) and its
     // compaction come BEFORE the K3M stages — a stage's compaction runs over every sparse list and would turn a
     // still-unwritten direct block into an empty list.
-    if (k1f) TRY(dense_single_pass());
-    for (size_t s = 0; s < n_seg; ++s) {
-        const uint32_t direct = (s == 0 && direct_rows) ? 1u : 0u;
-        const bool big = s == big_seg;                          // the segment with the most rows: the roofline's launch
-        if (big && !k1f) h->stats.last_big_rows = bounds[s + 1] - bounds[s];
-        TRY(dense_segment(bounds[s], bounds[s + 1], direct, big));
-        TRY(sparse_segment(bounds[s], bounds[s + 1], direct, big));
-        if (s == 0 && ms_staged) TRY(ms_stages());
+    if (s.k1f) TRY(dense_single_pass(s));                  // the single pass covers every segment
+    for (size_t si = 0; si < n_seg; ++si) {
+        const uint32_t direct = (si == 0 && s.direct_rows) ? 1u : 0u;
+        if (!s.k1f) TRY(dense_segment(s, si, direct, si == big_seg));
+        TRY(sparse_segment(s, si, direct, si == big_seg));
+        if (si == 0 && s.sp.ms_staged) TRY(ms_stages(s));
     }
-    if (do_delta) {
-        // K3D: the rows appended since the index was built, straight from the forward CSR.  One launch (a few
-        // thousand rows against thresholds the indexed rows have already established); the safe mode cuts it into
-        // pieces a list cannot overflow on.
-        const uint32_t piece = safe_mode ? (uint32_t)std::max<size_t>(VB_ROWS_PER_BLOCK, h->cand_cap - b.k) : n - nb;
-        for (uint32_t r0 = nb; r0 < n; r0 += piece) {
-            const uint32_t r1 = (uint32_t)std::min<uint64_t>(n, (uint64_t)r0 + piece);
-            const int pi = prof_begin(h, PH_SPARSE, ss);
-            VbDeltaArgs a{};
-            a.sp_indptr = h->sp_indptr.as<int64_t>(); a.sp_term = h->sp_term.as<uint32_t>(); a.sp_val = h->sp_val.as<float>();
-            a.qt_term = b.d_ut; a.qt_ptr = b.d_up; a.qt_query = b.d_uq; a.qt_weight = b.d_uw;
-            a.mask = b.use_mask ? h->mask.as<uint32_t>() : nullptr; a.mask_of = b.use_mask ? b.d_maskof : nullptr;
-            a.tau = b.tau; a.lists = L; a.mask_words = b.mask_words; a.n_uterms = b.n_uterms; a.n_queries = b.B;
-            a.row_begin = r0; a.row_end = r1; a.row_base = (uint32_t)h->row_base;
-            const uint32_t warps = vb_delta_warps(b.B);
-            const size_t smem = (size_t)warps * b.B * 8;
-            if (smem > (size_t)g_delta_smem_max) return vb_fail("batch of %u queries is too large for the delta rows (%zu bytes of shared memory)", b.B, smem);
-            const uint32_t grid = std::min<uint32_t>((r1 - r0 + warps - 1) / warps, (uint32_t)h->sm_count * 8u);
-            vb_sparse_delta_kernel<<<grid, warps * 32, smem, ss>>>(a);
-            CKK("vb_sparse_delta_kernel");
-            ++h->stats.last_launches;
-            prof_end(h, pi, ss);
-            const int ps = prof_begin(h, PH_SELECT, ss);
-            vb_compact_kernel<<<b.B, VB_COMPACT_THREADS, 0, ss>>>(L, b.tau, b.overflow, b.k, b.B, L.sub_cap);
-            CKK("vb_compact_kernel");
-            ++h->stats.last_launches;
-            prof_end(h, ps, ss);
-        }
-    }
+    if (s.do_delta) TRY(sparse_delta(s));
     if (two_streams) {
-        CK(cudaEventRecord(h->ev_join, ss));
-        CK(cudaStreamWaitEvent(sd, h->ev_join, 0));
+        CK(cudaEventRecord(h->ev_join, s.ss));
+        CK(cudaStreamWaitEvent(s.sd, h->ev_join, 0));
     }
-    if (sel_any) {                                              // every selected segment is in the scratch now
-        h->sel_segs.clear();
-        for (size_t si = 0; si < selseg.size(); ++si)
-            if (selseg[si].on) h->sel_segs.push_back({bounds[si], bounds[si + 1], selseg[si].row_off, selseg[si].meta_off, selseg[si].cap_rows});
-        h->sel_key = std::move(sel_key);
-    }
+    commit_rowsel(s);
     return 0;
 }
 
@@ -2081,8 +2076,8 @@ extern "C" int vb_stage(vb_index* h, const vb_query_batch* q, int32_t want_branc
     return 0;
 }
 
-extern "C" int vb_run_local(vb_index* h, uint64_t* cand_dev) {
-    if (!h) return vb_fail("vb_run_local: NULL index");
+// `safe`: the re-run after an overflow (run_branches)
+static int run_local(vb_index* h, uint64_t* cand_dev, bool safe) {
     std::lock_guard<std::recursive_mutex> lk(h->mu);
     if (!h->staged_s[h->cur].valid) return vb_fail("vb_run_local: no staged batch");
     if (h->staged_s[h->cur].need_corpus && (h->staged_s[h->cur].n_rows != (uint32_t)h->n_rows || h->staged_s[h->cur].gen != h->write_gen))
@@ -2093,7 +2088,7 @@ extern "C" int vb_run_local(vb_index* h, uint64_t* cand_dev) {
     if (h->n_rows == 0) {
         TRY(empty_lists(h, h->staged_s[h->cur]));
     } else {
-        TRY(run_branches(h, h->staged_s[h->cur], h->staged_safe));
+        TRY(run_branches(h, h->staged_s[h->cur], safe));
     }
     if (cand_dev) {
         vb_export_kernel<<<h->staged_s[h->cur].n_lists, 128, 0, h->stream>>>(h->cand.as<uint64_t>(), h->staged_s[h->cur].cnt, h->cand_cap, h->staged_s[h->cur].k, cand_dev, h->staged_s[h->cur].overflow, h->staged_s[h->cur].n_lists);
@@ -2101,6 +2096,11 @@ extern "C" int vb_run_local(vb_index* h, uint64_t* cand_dev) {
         ++h->stats.last_launches;
     }
     return 0;
+}
+
+extern "C" int vb_run_local(vb_index* h, uint64_t* cand_dev) {
+    if (!h) return vb_fail("vb_run_local: NULL index");
+    return run_local(h, cand_dev, false);
 }
 
 extern "C" int vb_run_fuse(vb_index* h, uint32_t n_shards, const uint64_t* gathered_dev) {
@@ -2143,10 +2143,7 @@ extern "C" int vb_search(vb_index* h, const vb_query_batch* q, vb_result* out) {
     if (h->n_rows == 0) { zero_result(q, out); return 0; }
     for (int attempt = 0; attempt < 2; ++attempt) {
         TRY(vb_stage(h, q, wants_branches(out), 1));
-        h->staged_safe = attempt == 1;
-        int rc = vb_run_local(h, nullptr);
-        h->staged_safe = false;
-        TRY(rc);
+        TRY(run_local(h, nullptr, attempt == 1));
         TRY(vb_run_fuse(h, 0, nullptr));
         int32_t overflowed = 0;
         TRY(vb_fetch(h, out, &overflowed));
@@ -2202,10 +2199,7 @@ extern "C" int vb_search_local(vb_index* h, const vb_query_batch* q, uint64_t* c
     std::lock_guard<std::recursive_mutex> lk(h->mu);
     for (int attempt = 0; attempt < 2; ++attempt) {
         TRY(vb_stage(h, q, 0, 1));
-        h->staged_safe = attempt == 1;
-        int rc = vb_run_local(h, cand_dev);
-        h->staged_safe = false;
-        TRY(rc);
+        TRY(run_local(h, cand_dev, attempt == 1));
         // overflow flags
         TRY(host_reserve(h->h_stage, (size_t)h->staged_s[h->cur].n_lists * 4));
         CK(cudaMemcpyAsync(h->h_stage.p, h->staged_s[h->cur].overflow, (size_t)h->staged_s[h->cur].n_lists * 4, cudaMemcpyDeviceToHost, h->stream));
