@@ -51,9 +51,12 @@ enum vb_ts_field { VB_TS_NONE = 0, VB_TS_CREATED = 1, VB_TS_MODIFIED = 2 };
 
 /* One evaluated filter (vector_store.py:462-530 _build_filter).  The host layer folds the
  * folder_path / index_folder string clauses into a bitset over scope ids (one scope id per
- * distinct (folder_path, index_folder) pair): bit s set <=> rows of scope s pass
+ * distinct (folder_path, index_folder) pair of unrestricted rows, and one per distinct
+ * (folder_path, index_folder, allowed_users set) of rows that carry an ACL): bit s set <=> rows
+ * of scope s pass
  *   must folder_path == folder_filter, must folder_path IN include_folders,
- *   must_not folder_path == e (each), must_not index_folder == f (each).
+ *   must_not folder_path == e (each), must_not index_folder == f (each),
+ *   and, for a caller with principals P, allowed_users absent or sharing an entry with P.
  * scope_bits == NULL means "no folder clause".  The range is inclusive on both sides
  * (gte / lte); use INT64_MIN+1 / INT64_MAX for an absent bound. */
 typedef struct vb_filter {
@@ -144,6 +147,15 @@ int vb_upsert_dev(vb_index* h, uint64_t n, const void* rows_bf16,
  * resolves the payload predicate to rows; the library tombstones them (and they stop
  * counting towards N and df of the IDF, as in qdrant). */
 int vb_delete_rows(vb_index* h, uint64_t n, const uint64_t* rows);
+
+/* Replaces client.set_payload (vector_store.py:216-231) for the one payload field the device filters on:
+ * scope_id[rows[i]] = scope_id[i] for rows that already exist.  The host layer calls it when a file's
+ * allowed_users change, which moves its rows to another (folder, index folder, ACL) scope.  Rows are global
+ * ids (row_base included), as in vb_delete_rows; deleted rows are accepted.  A NULL pointer, a row out of
+ * range or a row given twice is an error that names the row, and then nothing is written.  Like every
+ * write it refuses a batch staged before it and drops the kept row selection; N, df and the inverted index
+ * do not change.  Synchronous: the new ids are in place when it returns. */
+int vb_set_scope(vb_index* h, uint64_t n, const uint64_t* rows, const uint32_t* scope_id);
 
 /* Index maintenance.  The reference interleaves store_chunks batches of 100 (indexing.py:434,560) and
  * deletes (indexing.py:284, watcher.py:149-171) with searches, so writes do not invalidate the sorted

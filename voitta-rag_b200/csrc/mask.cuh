@@ -60,6 +60,16 @@ vb_mask_kernel(const uint32_t* __restrict__ scope_id, const int64_t* __restrict_
     }
 }
 
+// vb_set_scope: scope_id[rows[i]] = ids[i].  The host checked that the rows are in range and distinct, so the
+// scatter has no write conflicts.
+__global__ void __launch_bounds__(256)
+vb_scatter_scope_kernel(uint32_t* __restrict__ scope_id, const uint32_t* __restrict__ rows,
+                        const uint32_t* __restrict__ ids, uint32_t n)
+{
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        scope_id[rows[i]] = ids[i];
+}
+
 // Ingest (K5): fp32 -> bf16 rows (zero padded to d_pad) + fp32 inverse norm of the ROUNDED row,
 // so that score = dot(bf16 row, q_hat) * inv_norm is the cosine against the stored point.
 // Replaces the normalise-at-upsert step of qdrant's COSINE distance (vector_store.py:93, :313).

@@ -756,6 +756,45 @@ extern "C" int vb_delete_rows(vb_index* h, uint64_t n, const uint64_t* rows) {
     return 0;
 }
 
+extern "C" int vb_set_scope(vb_index* h, uint64_t n, const uint64_t* rows, const uint32_t* scope_id) {
+    if (!h) return vb_fail("vb_set_scope: NULL index");
+    if (n == 0) return 0;
+    if (!rows) return vb_fail("vb_set_scope: rows is NULL");
+    if (!scope_id) return vb_fail("vb_set_scope: scope_id is NULL");
+    std::lock_guard<std::recursive_mutex> lk(h->mu);
+    CK(cudaSetDevice(h->device));
+    // (row, id) pairs, rows local to the shard; sorted on the host so that a row given twice is found here and the
+    // device scatter never has two writers for one row
+    std::vector<uint32_t> pairs(2 * n);
+    std::vector<uint64_t> order(n);
+    for (uint64_t i = 0; i < n; ++i) {
+        if (rows[i] < h->row_base || rows[i] - h->row_base >= h->n_rows)
+            return vb_fail("vb_set_scope: row %llu out of range", (unsigned long long)rows[i]);
+        order[i] = i;
+    }
+    std::sort(order.begin(), order.end(), [&](uint64_t a, uint64_t b) { return rows[a] < rows[b]; });
+    for (uint64_t i = 0; i < n; ++i) {
+        if (i > 0 && rows[order[i]] == rows[order[i - 1]])
+            return vb_fail("vb_set_scope: row %llu given twice", (unsigned long long)rows[order[i]]);
+        pairs[i] = (uint32_t)(rows[order[i]] - h->row_base);
+        pairs[n + i] = scope_id[order[i]];
+    }
+    ++h->write_gen;                        // before the upload: a staged batch and a kept row selection are stale from here
+    DevBuf d_pairs;
+    int rc = dev_reserve(h, d_pairs, (size_t)n * 8, false);
+    if (rc) return rc;
+    cudaError_t e = cudaMemcpyAsync(d_pairs.p, pairs.data(), (size_t)n * 8, cudaMemcpyHostToDevice, h->stream);
+    if (e == cudaSuccess) {
+        vb_scatter_scope_kernel<<<grid_for(n, 256), 256, 0, h->stream>>>(h->scope_id.as<uint32_t>(), d_pairs.as<uint32_t>(),
+                                                                        d_pairs.as<uint32_t>() + n, (uint32_t)n);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
+    dev_free(h, d_pairs);
+    if (e != cudaSuccess) return vb_fail("vb_set_scope: scatter of %llu scope ids failed: %s", (unsigned long long)n, cudaGetErrorString(e));
+    return 0;
+}
+
 // ------------------------------------------------------------------------------------------------
 // inverted index build (device; CUB radix sort of (term,row) keys)
 // ------------------------------------------------------------------------------------------------

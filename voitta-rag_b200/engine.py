@@ -74,7 +74,7 @@ class _Stats(C.Structure):
 ABI_VERSION = 4          # include/voitta_b200.h VB_ABI_VERSION
 
 EXPORTS = ["vb_abi_version", "vb_last_error", "vb_create", "vb_destroy", "vb_upsert", "vb_upsert_dev",
-           "vb_delete_rows", "vb_optimize", "vb_term_stats", "vb_search", "vb_search_local", "vb_merge_fuse",
+           "vb_delete_rows", "vb_set_scope", "vb_optimize", "vb_term_stats", "vb_search", "vb_search_local", "vb_merge_fuse",
            "vb_stage", "vb_run_local", "vb_run_fuse", "vb_fetch", "vb_stage_dev", "vb_search_dev",
            "vb_set_option", "vb_get_stats", "vb_get_timeline", "vb_sync", "vb_save", "vb_load"]
 
@@ -101,6 +101,7 @@ def load_library():
     lib.vb_upsert.argtypes = [vp, C.c_uint64, vp, vp, vp, vp, vp, vp, vp, u64p]
     lib.vb_upsert_dev.argtypes = [vp, C.c_uint64, vp, vp, vp, vp, vp, vp, vp, u64p]
     lib.vb_delete_rows.argtypes = [vp, C.c_uint64, vp]
+    lib.vb_set_scope.argtypes = [vp, C.c_uint64, vp, vp]
     lib.vb_optimize.argtypes = [vp]
     lib.vb_term_stats.argtypes = [vp, C.c_uint32, vp, vp, u64p]
     lib.vb_search.argtypes = [vp, C.POINTER(_QueryBatch), C.POINTER(_Result)]
@@ -394,6 +395,14 @@ class Index:
     def delete_rows(self, rows) -> None:
         r = np.ascontiguousarray(rows, dtype=np.uint64)
         self._check(self._lib.vb_delete_rows(self._h, r.size, _vp(r)))
+
+    def set_scope(self, rows, scope_id) -> None:
+        """Rewrite the scope id of existing rows (global ids, row_base included): rows[i] gets scope_id[i]."""
+        r = np.ascontiguousarray(rows, dtype=np.uint64)
+        s = np.ascontiguousarray(scope_id, dtype=np.uint32)
+        if r.shape != s.shape or r.ndim != 1:
+            raise ValueError(f"set_scope: rows {r.shape} and scope ids {s.shape} must be 1-d of equal length")
+        self._check(self._lib.vb_set_scope(self._h, r.size, _vp(r), _vp(s)))
 
     def optimize(self) -> None:
         """Merge the rows appended since the last index build into the inverted index now."""

@@ -14,8 +14,9 @@ State is process-global per collection name, so a second ``VectorStoreService()`
 api/routes/folders.py:139-141 creates) sees the same index.  Thread-safe (one re-entrant lock per
 collection; callers are MCP worker threads, the indexing worker and the watchdog thread).
 
-Additive API (not in the reference): ``search_batch`` and the ``fusion`` switch
-(``VOITTA_FUSION=weighted|rrf``; default ``weighted`` = the reference's behaviour).
+Additive API (not in the reference): ``search_batch``, ``search_visible`` (results restricted to the chunks a caller
+may see, by each chunk's ``allowed_users``) and the ``fusion`` switch (``VOITTA_FUSION=weighted|rrf``; default
+``weighted`` = the reference's behaviour).
 """
 from __future__ import annotations
 
@@ -95,6 +96,24 @@ def get_settings() -> _Settings:
 
 _OPTIONAL = ("start_page", "end_page", "source_page_count", "source_created_at",
              "source_modified_at", "allowed_users", "source_url")
+
+
+def _principals(v, what: str) -> list[str]:
+    """A list of principal strings (user e-mail, group ids).  A bare string is refused: iterating its characters
+    would grant access by single letters."""
+    if isinstance(v, (str, bytes)):
+        raise TypeError(f"{what} must be a list of strings, not a single string")
+    out = list(v)
+    for p in out:
+        if not isinstance(p, str):
+            raise TypeError(f"{what} entries must be strings, got {type(p).__name__}")
+    return out
+
+
+def _acl_of(allowed_users) -> frozenset | None:
+    """The ACL a row's ``allowed_users`` stands for: None = no ACL (visible to everyone), otherwise the set of
+    principals that may see the row (empty = nobody)."""
+    return None if allowed_users is None else frozenset(_principals(allowed_users, "allowed_users"))
 
 
 def _is_device_tensor(x) -> bool:
@@ -243,10 +262,18 @@ class _Collection:
         self.by_folder: dict[str, set[int]] = {}
         self.by_index_folder: dict[str, set[int]] = {}
         self.by_url: dict[str, set[int]] = {}
-        self.scopes: dict[tuple[str, str], int] = {}   # (folder_path, index_folder) -> scope id
-        self.scope_list: list[tuple[str, str]] = []
+        # scope key -> scope id.  A key is (folder_path, index_folder) for rows without allowed_users and
+        # (folder_path, index_folder, acl_id) for rows with them; acl_id indexes acl_list.
+        self.scopes: dict[tuple, int] = {}
+        self.scope_list: list[tuple] = []
+        self.acl_list: list[frozenset] = []    # acl id -> the distinct allowed_users sets (frozenset() included)
+        self.acl_ids: dict[frozenset, int] = {}
         self.scope_version = 0                 # bumped whenever a scope id is added: cached scope bitsets die with it
         self.bits_cache: dict = {}             # caller's scope_key -> (scope_version, args, bits)
+        self._acl_fold = None                  # (scope_version, acl id + 1 per scope, principal -> acl ids + 1, any ACL)
+        # set_file_acl met an index that cannot rewrite scope ids (no set_scope): its rows keep their old scope, so the
+        # collection refuses visible_to from then on rather than answer from stale ids
+        self.acl_stale = False
         self.coalescer = _Coalescer(self)
         self.dirty = False                     # written since the last snapshot
         self.last_save = time.monotonic()
@@ -259,8 +286,15 @@ class _Collection:
                 self._index = self._factory()
             return self._index
 
-    def scope_id(self, folder_path: str, index_folder: str) -> int:
-        key = (folder_path, index_folder)
+    def scope_id(self, folder_path: str, index_folder: str, acl: frozenset | None = None) -> int:
+        if acl is None:
+            key = (folder_path, index_folder)
+        else:
+            aid = self.acl_ids.get(acl)
+            if aid is None:
+                aid = self.acl_ids[acl] = len(self.acl_list)
+                self.acl_list.append(acl)
+            key = (folder_path, index_folder, aid)
         sid = self.scopes.get(key)
         if sid is None:
             sid = len(self.scope_list)
@@ -268,6 +302,42 @@ class _Collection:
             self.scope_list.append(key)
             self.scope_version += 1
         return sid
+
+    def acl_fold(self):
+        """What the ACL clause of a filter needs, rebuilt from scope_list / acl_list whenever scope_version changes:
+        per scope its acl id + 1 (0 = unrestricted), per principal the acl ids + 1 that name it, and whether any
+        scope carries an ACL.  Caller holds the lock."""
+        f = self._acl_fold
+        if f is None or f[0] != self.scope_version:
+            scope_acl = np.fromiter((k[2] + 1 if len(k) > 2 else 0 for k in self.scope_list), np.int64, len(self.scope_list))
+            by_principal: dict[str, list[int]] = {}
+            for aid, acl in enumerate(self.acl_list):
+                for p in acl:
+                    by_principal.setdefault(p, []).append(aid + 1)
+            f = self._acl_fold = (self.scope_version, scope_acl, {p: np.asarray(a, np.int64) for p, a in by_principal.items()},
+                                  bool((scope_acl > 0).any()))
+        return f
+
+    def acl_bits(self, principals: list[str]):
+        """Scope bitset of the rows visible to ``principals``, or None when every scope is (the clause drops out).
+        Caller holds the lock."""
+        _, scope_acl, by_principal, restricted = self.acl_fold()
+        if not restricted:
+            return None
+        ok = np.zeros(len(self.acl_list) + 1, bool)
+        ok[0] = True                                      # rows without allowed_users
+        for p in principals:
+            a = by_principal.get(p)
+            if a is not None:
+                ok[a] = True
+        passing = ok[scope_acl]
+        if passing.all():
+            return None
+        words = max(1, (len(passing) + 31) // 32)
+        packed = np.zeros(words * 4, np.uint8)
+        b = np.packbits(passing, bitorder="little")       # bit s of byte s / 8 = bit s of word s / 32 (little-endian words)
+        packed[:len(b)] = b
+        return packed.view("<u4").astype(np.uint32)
 
     def _map_add(self, m: dict, key, row: int):
         if key is not None:
@@ -331,14 +401,20 @@ class _Collection:
         with self.lock:
             self.index.save(dev_tmp)                       # vb_save flushes and fsyncs before it returns
             os.replace(dev_tmp, dev_path)
-            head = {"version": 2, "name": self.name, "dim": self.dim, "generation": generation,
+            # version 3 once a scope carries an ACL: a build that does not know ACLs refuses such a snapshot
+            version = 3 if any(len(k) > 2 for k in self.scope_list) else 2
+            head = {"version": version, "name": self.name, "dim": self.dim, "generation": generation,
                     "device_file": dev_path.name, "n_rows": len(self.ids), "n_live": self.n_live}
+            if self.acl_stale:
+                head["acl_stale"] = True
             with open(host_tmp, "w", encoding="utf-8") as f:
                 # the small header keys come first so that snapshot_paths can read them without parsing the payloads
                 f.write(json.dumps(head)[:-1] + ', "ids": ')
                 json.dump(self.ids, f)
                 f.write(', "scope_list": ')
                 json.dump([list(k) for k in self.scope_list], f)
+                f.write(', "acl_list": ')
+                json.dump([sorted(a) for a in self.acl_list], f)
                 f.write(', "payload": ')
                 json.dump(self.payload, f)
                 f.write("}")
@@ -370,10 +446,14 @@ class _Collection:
         _, host_path = self.snapshot_paths(d, "x")
         with open(host_path, "r", encoding="utf-8") as f:
             st = json.load(f)
-        if st.get("version") != 2 or st.get("dim") != self.dim or st.get("name") != self.name:
+        if st.get("version") not in (2, 3) or st.get("dim") != self.dim or st.get("name") != self.name:
             raise ValueError(f"snapshot {host_path} does not match collection '{self.name}' (dim {self.dim})")
         ids, payload = st["ids"], st["payload"]
         n_live = sum(1 for p in payload if p is not None)
+        scope_list = [tuple(k) for k in st["scope_list"]]
+        acl_list = [frozenset(a) for a in st.get("acl_list", [])]
+        if any(len(k) not in (2, 3) or (len(k) == 3 and not 0 <= k[2] < len(acl_list)) for k in scope_list):
+            raise ValueError(f"snapshot {host_path}: a scope names an ACL the snapshot does not hold")
         if len(ids) != len(payload) or len(ids) != st["n_rows"] or n_live != st["n_live"]:
             raise ValueError(f"snapshot {host_path} is inconsistent (ids {len(ids)}, payloads {len(payload)}, "
                              f"header rows {st['n_rows']} live {st['n_live']} / counted {n_live})")
@@ -398,8 +478,11 @@ class _Collection:
             self.payload = [None] * len(self.ids)
             self.n_live = 0
             self.by_file, self.by_folder, self.by_index_folder, self.by_url = {}, {}, {}, {}
-            self.scope_list = [tuple(k) for k in st["scope_list"]]
+            self.scope_list = scope_list
             self.scopes = {k: i for i, k in enumerate(self.scope_list)}
+            self.acl_list = acl_list
+            self.acl_ids = {a: i for i, a in enumerate(acl_list)}
+            self.acl_stale = bool(st.get("acl_stale", False))
             self.scope_version += 1
             self.bits_cache.clear()
             for r, pl in enumerate(payload):
@@ -527,14 +610,32 @@ class VectorStoreService:
         return chunks
 
     def set_file_acl(self, file_path: str, allowed_users: list[str]) -> None:
-        """Update allowed_users on all chunks for a specific file (reference :216)."""
+        """Update allowed_users on all chunks for a specific file (reference :216).
+
+        The rows move to the scope of their (folder, index folder, ACL) on the device first; the payloads change only
+        once that succeeded, so a failed device call leaves both sides as they were.  An index without ``set_scope``
+        gets the payload update only, and the collection then refuses ``visible_to`` (fails closed)."""
+        acl = _acl_of(allowed_users)
         coll = self._coll
         with coll.lock:
             rows = self._rows_where(coll, coll.by_file, file_path)
+            if not rows:
+                return
+            index = self.client
+            if not hasattr(index, "set_scope"):
+                # an index without vb_set_scope keeps the rows' scope ids: the payloads change as in the reference, and
+                # the collection refuses visible_to from now on (_build_filter) instead of filtering by the old ACL
+                for r in rows:
+                    coll.payload[r]["allowed_users"] = allowed_users
+                coll.acl_stale = True
+                coll.wrote()
+                return
+            sids = np.fromiter((coll.scope_id(coll.payload[r]["folder_path"], coll.payload[r]["index_folder"], acl) for r in rows),
+                               dtype=np.uint32, count=len(rows))
+            index.set_scope(np.asarray(rows, dtype=np.uint64) + np.uint64(getattr(index, "row_base", 0)), sids)
             for r in rows:
                 coll.payload[r]["allowed_users"] = allowed_users
-            if rows:
-                coll.wrote()
+            coll.wrote()
 
     def store_chunks(
         self,
@@ -554,7 +655,9 @@ class VectorStoreService:
         created = np.full(n, engine.TS_MISSING, dtype=np.int64)
         modified = np.full(n, engine.TS_MISSING, dtype=np.int64)
         coll = self._coll
+        acls = []
         for idx, (text, embedding, metadata) in enumerate(chunks):
+            acls.append(_acl_of(metadata.allowed_users))
             ids.append(str(uuid.uuid4()))
             payload = {
                 "text": text,
@@ -598,7 +701,7 @@ class VectorStoreService:
                     nnz = len(ix)
             indptr[idx + 1] = indptr[idx] + nnz
         with coll.lock:
-            scope = np.fromiter((coll.scope_id(p["folder_path"], p["index_folder"]) for p in payloads),
+            scope = np.fromiter((coll.scope_id(p["folder_path"], p["index_folder"], a) for p, a in zip(payloads, acls)),
                                 dtype=np.uint32, count=n)
             tcat = np.concatenate(terms) if terms else np.zeros(0, np.uint32)
             vcat = np.concatenate(vals) if vals else np.zeros(0, np.float32)
@@ -661,14 +764,25 @@ class VectorStoreService:
         date_end: int | None = None,
         date_field: str | None = None,
         scope_key=None,
+        visible_to: list[str] | None = None,
     ) -> engine.Filter | None:
         """Evaluate the folder clauses over the scope dictionary and return the device filter.
 
         must folder_path == folder_filter; must folder_path IN include_folders (exact strings, the
         caller already expanded prefixes); must_not folder_path == e; must_not index_folder == f;
         must ts in [gte, lte] on source_created_at if date_field == "created" else source_modified_at.
-        Returns None when no clause applies (reference :525-530)."""
+        Returns None when no clause applies (reference :525-530).
+
+        Additive: ``visible_to`` (a list of principals: the user's e-mail and group ids) keeps the rows whose
+        ``allowed_users`` is absent or None, or shares an entry with it; ``allowed_users == []`` is visible to nobody.
+        None adds no clause.  The clause is computed per call (the folder bits stay cached by ``scope_key``) and is
+        left out when it passes every scope."""
         coll = self._coll
+        if visible_to is not None:
+            visible_to = _principals(visible_to, "visible_to")
+            if coll.acl_stale:
+                raise RuntimeError(f"collection '{coll.name}': an ACL changed on an index that cannot rewrite scope ids "
+                                   "(no set_scope), so visible_to cannot be enforced")
         bits = None
         cached = None
         if scope_key is not None:
@@ -687,7 +801,8 @@ class VectorStoreService:
             with coll.lock:
                 n_scopes = len(coll.scope_list)
                 bits = np.zeros(max(1, (n_scopes + 31) // 32), dtype=np.uint32)
-                for sid, (fp, ifp) in enumerate(coll.scope_list):
+                for sid, key in enumerate(coll.scope_list):
+                    fp, ifp = key[0], key[1]
                     ok = ((not folder_filter or fp == folder_filter) and (inc is None or fp in inc)
                           and fp not in exc and ifp not in dis)
                     if ok:
@@ -696,6 +811,17 @@ class VectorStoreService:
                     if len(coll.bits_cache) >= 256:
                         coll.bits_cache.pop(next(iter(coll.bits_cache)))
                     coll.bits_cache[scope_key] = (coll.scope_version, bits)
+        if visible_to is not None:
+            with coll.lock:
+                acl = coll.acl_bits(visible_to)
+            if acl is not None:
+                if bits is None:
+                    bits = acl
+                else:                                     # a cached fold may predate scopes added since: they read as 0
+                    n = min(len(bits), len(acl))
+                    both = np.zeros(max(len(bits), len(acl)), np.uint32)
+                    both[:n] = bits[:n] & acl[:n]
+                    bits = both
         ts_field, lo, hi = engine.TS_NONE, engine.TS_MIN, engine.TS_MAX
         if date_start is not None or date_end is not None:
             field_map = {"created": engine.TS_CREATED, "modified": engine.TS_MODIFIED}
@@ -740,6 +866,34 @@ class VectorStoreService:
         Additive: ``scope_key`` (any hashable, e.g. ``(user_id, project_id, settings_version)``) lets the
         folded folder bitset be cached across calls.  Concurrent callers are coalesced into one device
         batch (``_Coalescer``)."""
+        return self._search(query_embedding, limit, folder_filter, include_folders, exclude_folders, exclude_index_folders,
+                            sparse_query, sparse_weight, date_start, date_end, date_field, scope_key, None)
+
+    def search_visible(
+        self,
+        query_embedding: list[float],
+        limit: int = 10,
+        folder_filter: str | None = None,
+        include_folders: list[str] | None = None,
+        exclude_folders: list[str] | None = None,
+        exclude_index_folders: list[str] | None = None,
+        sparse_query: tuple[list[int], list[float]] | None = None,
+        sparse_weight: float = 0.1,
+        date_start: int | None = None,
+        date_end: int | None = None,
+        date_field: str | None = None,
+        scope_key=None,
+        *,
+        visible_to: list[str] | None,
+    ) -> list[StoredChunk]:
+        """Additive: ``search`` restricted to the chunks the caller may see.  ``visible_to`` lists the caller's
+        principals (the user's e-mail plus the group ids the caller resolved); a chunk is returned only if its
+        ``allowed_users`` is absent or None, or shares an entry with ``visible_to`` (see ``_build_filter``)."""
+        return self._search(query_embedding, limit, folder_filter, include_folders, exclude_folders, exclude_index_folders,
+                            sparse_query, sparse_weight, date_start, date_end, date_field, scope_key, visible_to)
+
+    def _search(self, query_embedding, limit, folder_filter, include_folders, exclude_folders, exclude_index_folders,
+                sparse_query, sparse_weight, date_start, date_end, date_field, scope_key, visible_to):
         self.client
         coll = self._coll
         if _is_device_tensor(query_embedding):
@@ -749,10 +903,10 @@ class VectorStoreService:
             return self.search_batch(query_embedding[None, :], limit=limit, folder_filter=folder_filter, include_folders=include_folders,
                                      exclude_folders=exclude_folders, exclude_index_folders=exclude_index_folders,
                                      sparse_queries=[sparse_query], sparse_weight=sparse_weight, date_start=date_start,
-                                     date_end=date_end, date_field=date_field)[0]
+                                     date_end=date_end, date_field=date_field, visible_to=visible_to)[0]
         search_filter = self._build_filter(
             folder_filter, include_folders, exclude_folders, exclude_index_folders,
-            date_start=date_start, date_end=date_end, date_field=date_field, scope_key=scope_key)
+            date_start=date_start, date_end=date_end, date_field=date_field, scope_key=scope_key, visible_to=visible_to)
         q = np.asarray(query_embedding, dtype=np.float32)
         if q.ndim != 1 or q.shape[0] != self.dimension:
             raise ValueError(f"Vector dimension error: expected {self.dimension}, got {q.shape[-1] if q.ndim else 0}")
@@ -799,25 +953,29 @@ class VectorStoreService:
         date_field: str | None = None,
         fusion: str | None = None,
         filters: list[dict | None] | None = None,
+        visible_to: list[str] | None = None,
     ) -> list[list[StoredChunk]]:
         """Additive: ``search`` for B queries in one device pass.
 
         By default the B queries share one filter, built from the folder and date arguments.  ``filters`` gives each
         query its own instead: a list of B entries, each None (unfiltered) or a dict of ``_build_filter`` keyword
         arguments (``folder_filter``, ``include_folders``, ``exclude_folders``, ``exclude_index_folders``,
-        ``date_start``, ``date_end``, ``date_field``, ``scope_key``).  Queries whose filters have equal content share
-        one device mask.  Giving ``filters`` together with any of the shared filter arguments is a ValueError."""
+        ``date_start``, ``date_end``, ``date_field``, ``scope_key``, ``visible_to``).  Queries whose filters have equal
+        content share one device mask.  Giving ``filters`` together with any of the shared filter arguments
+        (``visible_to`` included) is a ValueError.  ``visible_to`` restricts the results to the chunks those principals
+        may see, as in ``search_visible``."""
         index = self.client
         coll = self._coll
         B = len(query_embeddings)
         if filters is None:
             search_filter = self._build_filter(
                 folder_filter, include_folders, exclude_folders, exclude_index_folders,
-                date_start=date_start, date_end=date_end, date_field=date_field)
+                date_start=date_start, date_end=date_end, date_field=date_field, visible_to=visible_to)
             flts = [search_filter] if search_filter is not None else None
             filter_of = np.zeros(B, np.int32) if search_filter is not None else None
         else:
-            shared = (folder_filter, include_folders, exclude_folders, exclude_index_folders, date_start, date_end, date_field)
+            shared = (folder_filter, include_folders, exclude_folders, exclude_index_folders, date_start, date_end, date_field,
+                      visible_to)
             if any(a is not None for a in shared):
                 raise ValueError("give either per-query filters or the shared filter arguments, not both")
             if len(filters) != B:
